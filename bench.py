@@ -13,9 +13,10 @@ The same JSON line also carries, at every N:
   train_ln    BASELINE configs[4]: the +LN +AdamW +cosine variant, data parallel;
   metrics_1rank / metrics_match_1rank (N > 1): rank 0 re-evaluates the whole workload alone, outside every timed region.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision tf32|fp32] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision tf32|fp32] [--impl reference] [--dump-outputs DIR]
 
-Prints ONE JSON line on rank 0.  `--impl reference` times the CPU restatement of the reference's
+Every timed loop (the headline evaluate, its end-to-end variant, the MIND-large and training side measurements) times
+exactly K steps.  Prints ONE JSON line on rank 0.  `--impl reference` times the CPU restatement of the reference's
 path (oracle/torch_port.py, PyTorch-CPU on all host cores) on a bounded sample of the same workload.
 """
 import argparse
@@ -214,6 +215,38 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES_PER_ARRAY = 12 << 20
+
+
+def dump_outputs(out_dir, means, det, n_news):
+    """--dump-outputs: what the last timed evaluate step returned (the metric means) and computed on the way (per-impression
+    metrics, candidate scores, user vectors, news vectors) as float .npy files.  An array larger than DUMP_BYTES_PER_ARRAY
+    is cut to a fixed sample of its rows (np.random.default_rng(0), sorted), so equal arguments give equal rows.
+    per_impression holds the impressions whose metrics are defined: one with a single label class has no AUC (NaN in the
+    reference, left out of its nanmean), and it is left out here too, so every value written is finite."""
+    import torch
+
+    def sample(a):
+        rows = DUMP_BYTES_PER_ARRAY // (a[0].numel() * a.element_size())
+        if a.shape[0] > rows:
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))
+            a = a[torch.from_numpy(idx).to(a.device)]
+        return a.cpu().numpy()
+
+    per = det["per_impression"]
+    per = per[~torch.isnan(per).any(dim=1)]
+    arrays = dict(metrics=np.asarray(means, dtype=np.float64), per_impression=sample(per),
+                  scores=sample(det["scores"]), user_vectors=sample(det["user_vectors"]),
+                  news_vectors=sample(det["table"][:n_news]))
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if not np.isfinite(a).all():
+            raise RuntimeError(f"--dump-outputs: {name} of the last timed step is not finite")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(world, precision, workload="small-per-gpu"):
     n_news, n_imp = workload_sizes(world, workload)
     name = ("NRMS evaluate pipeline, MIND-large-shaped in total, sharded over the GPUs (BASELINE configs[3])"
@@ -227,7 +260,7 @@ def workload_config(world, precision, workload="small-per-gpu"):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--precision", default="tf32", choices=["tf32", "fp32"])
@@ -237,7 +270,13 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the train-step side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-large", action="store_true", help="skip the MIND-large side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed evaluate step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 evaluate pass (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -281,7 +320,7 @@ def main():
     # ---------------------------------------------------------------------------------------------------
     # one evaluate workload: resident loop (`value`), end-to-end loop (`e2e`), 1-rank cross-check
     # ---------------------------------------------------------------------------------------------------
-    def run_eval(workload, steps, warmup, sample_clocks):
+    def run_eval(workload, steps, warmup, sample_clocks, dump_dir=None):
         news, imp = make_data(world, workload)
         host = EvalHost(news, imp["hist_rows"], imp["cand_offsets"], imp["cand_rows"], imp["labels"])
         inputs = EvalInputs.from_host(host, dev)
@@ -289,7 +328,7 @@ def main():
         stage = {}
         h2d = [host.nbytes()]
 
-        def timed_eval(resident, record_stages=False):
+        def timed_eval(resident, record_stages=False, details=False):
             marks = []
 
             def mark(name):
@@ -302,7 +341,8 @@ def main():
             e0.record()
             inp = resident if resident is not None else EvalInputs.from_host(host, dev)
             h2d[0] = inp.h2d_bytes
-            means = evaluate_tensors(model, inp, mark=mark if record_stages else None)   # ends with the D2H of 8 doubles
+            # ends with the D2H of 8 doubles
+            out = evaluate_tensors(model, inp, mark=mark if record_stages else None, return_details=details)
             e1.record()
             torch.cuda.synchronize()
             if record_stages:
@@ -312,7 +352,7 @@ def main():
                 # 8-double all-reduce, where a rank waits for the slowest one, and the read-back of the means)
                 stage.setdefault("pre", []).append(e0.elapsed_time(marks[0][1]))
                 stage.setdefault("allreduce_readback", []).append(marks[-1][1].elapsed_time(e1))
-            return e0.elapsed_time(e1), means
+            return e0.elapsed_time(e1), out
 
         # the attention launches are bracketed with CUDA events in BOTH loops (same instrumentation; the events are
         # created and pooled during the warm-up)
@@ -327,10 +367,17 @@ def main():
         lib.nrms_set_option(b"time_k1", 1)
         l0 = lib.nrms_launch_count()
         times, means = [], None
-        for _ in range(steps):
-            ms, means = timed_eval(inputs, record_stages=True)
+        for i in range(steps):
+            # the last step also returns the arrays it computed on the way; in tensor mode that costs one fp32 copy of the
+            # news table, so it is asked for only when they are dumped
+            ms, means = timed_eval(inputs, record_stages=True, details=dump_dir is not None and i == steps - 1)
             times.append(ms)
         launches = int(lib.nrms_launch_count() - l0)
+        if dump_dir is not None:
+            means, det = means
+            if rank == 0:
+                dump_outputs(dump_dir, means, det, host.n_news)
+            del det
         kstat = {k: tuple(lib.nrms_get_stat(f"{k}_{w}".encode()) for w in ("ms", "launches", "sequences"))
                  for k in ("k1", "k1n", "k1g", "k1gn")}
         lib.nrms_set_option(b"time_k1", 1)      # clears the records, stays on
@@ -372,10 +419,10 @@ def main():
         torch.cuda.empty_cache()
         return res
 
-    head = run_eval(args.workload, args.steps, args.warmup, sample_clocks=True)
+    head = run_eval(args.workload, args.steps, args.warmup, sample_clocks=True, dump_dir=args.dump_outputs)
     large = None
     if args.workload != "mind-large" and not args.no_large:
-        large = run_eval("mind-large", max(3, min(args.steps, 5)), 3, sample_clocks=False)
+        large = run_eval("mind-large", args.steps, 3, sample_clocks=False)
 
     # ---------------------------------------------------------------------------------------------------
     # rooflines of the headline workload, from SURVEY 8(d)'s algorithmic bytes / flops
@@ -460,7 +507,7 @@ def main():
         missing = {k: v for k, v in m.state_dict().items() if k not in sdl}     # LayerNorm affine of the variant
         m.load_state_dict({**{k: torch.from_numpy(v) for k, v in sdl.items()}, **missing})
         m.to(dev).train().set_precision(args.precision)
-        n_train = max(5, args.steps)
+        n_train = args.steps
         ts = TrainStep(m, lr=1e-4, adamw=adamw, weight_decay=0.01 if adamw else 0.0,
                        cosine_total_steps=(n_train + 3) if cosine else None)
         cand, clicked = synthetic.make_train_batch(128, news_small, k_neg=4, seed=1234 + rank)

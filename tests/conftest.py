@@ -7,6 +7,9 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+if GOLDEN not in sys.path:
+    sys.path.insert(0, GOLDEN)
 
 
 def pytest_configure(config):
@@ -15,9 +18,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    path = os.path.join(ROOT, "tests", "golden", "nrms_golden.npz")
-    z = np.load(path)
-    return {k: z[k] for k in z.files}
+    from compact import expand_nrms
+    return expand_nrms(np.load(os.path.join(GOLDEN, "nrms_golden.npz")))
 
 
 @pytest.fixture(scope="session")

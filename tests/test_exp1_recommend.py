@@ -16,6 +16,7 @@ from conftest import ROOT, rel_l2_rows
 from oracle import nrms_oracle as O
 
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+from compact import expand_exp1, pinned  # noqa: E402
 from exp1_weights import make_state  # noqa: E402
 
 ATTRS = ['category', 'subcategory', 'title']
@@ -24,8 +25,7 @@ ATTRS_A = ['category', 'subcategory', 'title', 'abstract']
 
 @pytest.fixture(scope="module")
 def g1():
-    z = np.load(os.path.join(ROOT, "tests", "golden", "exp1_golden.npz"))
-    return {k: z[k] for k in z.files}
+    return expand_exp1(np.load(os.path.join(ROOT, "tests", "golden", "exp1_golden.npz")))
 
 
 def _cfg(attrs):
@@ -162,8 +162,8 @@ def test_exp1_train_step_gradients_vs_reference(g1, dev):
     for k, p in m.named_parameters():
         ref = g1["grad/" + k]
         got = p.grad.detach().cpu().numpy()
-        got = got[:ref.shape[0]] if got.ndim == 2 else got
-        scale = max(float(np.abs(ref).max()), float(g1["gradnorm/" + k]) / np.sqrt(max(p.numel(), 1)), 1e-12)
+        got = pinned(got, 48)                      # make_golden_exp1.py stores the first 48 rows of a matrix
+        scale = max(float(g1["absmax/grad/" + k]), float(g1["gradnorm/" + k]) / np.sqrt(max(p.numel(), 1)), 1e-12)
         err = float(np.abs(got - ref).max())
         assert err <= 2e-4 * scale + 1e-9, (k, err, scale)
         full_norm = float(torch.linalg.vector_norm(p.grad.double()))

@@ -10,7 +10,8 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import rel_l2_rows
+from conftest import GOLDEN, rel_l2_rows
+from compact import expand_masked, pinned
 from oracle import nrms_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -275,14 +276,14 @@ def test_train_step_fp32_matches_reference(dev, golden, golden_sd):
     assert abs(losses[1] - float(golden["train/loss2"])) < 2e-5
     for k, g in grads.items():
         ref = golden["train/grad/" + k]
-        got = g if "embedding" in k else (g[:48] if g.ndim == 2 else g)
-        scale = np.abs(ref).max() + 1e-12
+        got = pinned(g, None if "embedding" in k else 48)
+        scale = golden["absmax/train/grad/" + k] + 1e-12
         assert np.abs(got - ref).max() < 2e-4 * scale + 1e-8, (k, np.abs(got - ref).max(), scale)
     assert not grads[O.EMB_KEY][0].any()
     sd = {k: v.detach().cpu().numpy() for k, v in m.state_dict().items()}
     for k, v in sd.items():
         ref = golden["train/adam2/" + k]
-        got = v[:48] if v.ndim == 2 else v
+        got = pinned(v, 48)
         gs = float(np.abs(golden["train/grad/" + k]).mean())
         d = np.abs(got.astype(np.float64) - ref)
         assert d.max() <= 2.5e-4, k                      # never more than ~2 lr per step off
@@ -298,8 +299,8 @@ def test_train_step_tensor_mode_gradients(dev, golden, golden_sd):
     assert abs(losses[0] - float(golden["train/loss"])) < 2e-3
     for k, g in grads.items():
         ref = golden["train/grad/" + k]
-        got = g if "embedding" in k else (g[:48] if g.ndim == 2 else g)
-        scale = np.abs(ref).max() + 1e-12
+        got = pinned(g, None if "embedding" in k else 48)
+        scale = golden["absmax/train/grad/" + k] + 1e-12
         assert np.abs(got - ref).max() < 3e-3 * scale + 1e-8, (k, np.abs(got - ref).max(), scale)
     assert not grads[O.EMB_KEY][0].any()
 
@@ -329,7 +330,7 @@ def test_adam_kernel_elementwise(dev, golden, golden_sd):
     for k in golden_sd:
         if "embedding" in k:
             continue
-        p0 = golden_sd[k][:48] if golden_sd[k].ndim == 2 else golden_sd[k]
+        p0 = pinned(golden_sd[k], 48)
         g = golden["train/grad/" + k]
         for tag, kw in (("adam1", {}), ("adamw1", dict(weight_decay=0.01, decoupled=True))):
             p = t(p0.reshape(-1).copy(), dev)
@@ -630,7 +631,7 @@ def test_mhsa_length_mask(dev, precision):
     reference module (tests/golden/mhsa_masked_golden.npz) for both compiled sequence lengths."""
     import os
     from newsrecommendationsystem_b200.model.general.attention.multihead_self import MultiHeadSelfAttention
-    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "mhsa_masked_golden.npz"))
+    g = expand_masked(np.load(os.path.join(GOLDEN, "mhsa_masked_golden.npz")))
     att = MultiHeadSelfAttention(300, 15)
     att.load_state_dict({f"W_{n.upper()}.{k}": torch.from_numpy(g[f"{'W' if k == 'weight' else 'b'}{n}"])
                          for n in "qkv" for k in ("weight", "bias")})
@@ -640,11 +641,19 @@ def test_mhsa_length_mask(dev, precision):
         with torch.no_grad():
             c = att(t(g[f"S{S}/x"], dev), length=torch.from_numpy(g[f"S{S}/length"]))
             c0 = att(t(g[f"S{S}/x"], dev))
-        ref = g[f"S{S}/ctx"].reshape(-1, 300)
-        got = c.cpu().numpy().reshape(-1, 300)
-        keep = np.linalg.norm(ref, axis=1) > 0                 # the rows of the length-0 sequence are exactly zero
-        assert not got[~keep].any()
-        assert rel_l2_rows(got[keep], ref[keep]) < (2e-5 if precision == "fp32" else 1e-3)
+        tol = 2e-5 if precision == "fp32" else 1e-3
+        full = c.cpu().numpy()
+        assert not full[g[f"S{S}/length"] == 0].any()          # the rows of the length-0 sequence are exactly zero
+        ref = g[f"S{S}/ctx"].reshape(-1, 300)                  # the reference at the positions the fixture keeps
+        got = full[:, g[f"S{S}/pos"]].reshape(-1, 300)
+        keep = np.linalg.norm(ref, axis=1) > 0
+        assert rel_l2_rows(got[keep], ref[keep]) < tol
+        # every position against the oracle (pinned to the reference in test_oracle_golden.py)
+        ora, _ = O.mhsa_forward(g[f"S{S}/x"], {k: g[k] for k in ("Wq", "bq", "Wk", "bk", "Wv", "bv")}, 15,
+                                length=g[f"S{S}/length"])
+        ora = ora.reshape(-1, 300)
+        keep = np.linalg.norm(ora, axis=1) > 0
+        assert rel_l2_rows(full.reshape(-1, 300)[keep], ora[keep]) < tol
         assert torch.equal(c[0], c0[0]) and torch.equal(c[5], c0[5])     # length >= S: the mask is a no-op
 
 

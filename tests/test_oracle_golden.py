@@ -4,13 +4,15 @@ import numpy as np
 import pytest
 
 from oracle import nrms_oracle as O
-from conftest import rel_l2_rows
+from conftest import GOLDEN, rel_l2_rows
+from compact import expand_masked, pinned
 
-ROWS = 48
+ROWS = 48   # make_golden.py stores the first ROWS rows of a matrix (all of the word embedding's gradient)
 
 
 def clip(a):
-    return a[:ROWS] if a.ndim == 2 else a
+    """The entries of a parameter-shaped array that the fixture keeps of the reference's."""
+    return pinned(a, ROWS)
 
 
 def test_gather_bit_exact(golden, golden_sd):
@@ -52,8 +54,8 @@ def test_train_grads(golden, step1):
     grads = step1[2]
     for k, g in grads.items():
         ref = golden["train/grad/" + k]
-        got = g if "embedding" in k else clip(g)
-        scale = np.abs(ref).max() + 1e-12
+        got = pinned(g) if "embedding" in k else clip(g)
+        scale = golden["absmax/train/grad/" + k] + 1e-12
         # W_K.bias grads are analytically ~0 (row-softmax shift invariance): pure roundoff
         assert np.abs(got - ref).max() < 5e-5 * scale + 1e-8, k
     assert not grads[O.EMB_KEY][0].any()   # padding_idx row has zero grad
@@ -238,12 +240,12 @@ def test_mhsa_length_mask_matches_reference():
     """The `length` branch (multihead_self.py:60-68) of the oracle vs vectors generated by the live reference module
     (tests/golden/make_golden_masked.py): full length, one key, zero keys, length past the end."""
     import os
-    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "mhsa_masked_golden.npz"))
+    g = expand_masked(np.load(os.path.join(GOLDEN, "mhsa_masked_golden.npz")))
     p = {f"W{n}": g[f"W{n}"] for n in "qkv"}
     p.update({f"b{n}": g[f"b{n}"] for n in "qkv"})
     for S in (20, 50):
         out, _ = O.mhsa_forward(g[f"S{S}/x"], p, 15, length=g[f"S{S}/length"])
-        np.testing.assert_allclose(out, g[f"S{S}/ctx"], rtol=2e-5, atol=2e-6)
+        np.testing.assert_allclose(out[:, g[f"S{S}/pos"]], g[f"S{S}/ctx"], rtol=2e-5, atol=2e-6)
         out0, _ = O.mhsa_forward(g[f"S{S}/x"], p, 15)
         assert not out[2].any()                                  # length 0: 0 / (0 + 1e-8)
         np.testing.assert_array_equal(out[0], out0[0])           # length == S: the mask is a no-op
