@@ -241,6 +241,32 @@ int nrms_recommend_user(const float* table, int64_t n_rows, const int32_t* hist_
                         float* user_vec, float* scores, int32_t* order, void* workspace, size_t workspace_bytes,
                         void* stream);
 
+/* ---- top-k news of the whole table per user ------------------------------------------
+ * The ranking of src/recommend.py:338-340 (np.argsort(-y) over the candidates the caller passes) generalised to every
+ * row of the news table: for each user u, top_rows[u, 0..k) are the k rows of [0, n_news) with the highest score
+ * table[row] . user_vec[u], and top_scores[u, j] is that score.
+ *   - Order: score descending, equal scores by row ascending (the rule of nrms_recommend_user), so the result is unique
+ *     and does not depend on the launch configuration.  -0 and +0 are equal scores.  A NaN score ranks below every number
+ *     and is never returned.  When fewer than k rows remain, the tail is row -1, score -inf.  1 <= k <= 256.
+ *   - mode NRMS_MODE_TF32: `table` is the fp16 copy in nrms_pack_rows_f16's layout (rows of 320 halfs); user_vec is rounded
+ *     to fp16 and the dot products run on the tensor cores (tcgen05 kind::f16, fp32 accumulation).
+ *     mode NRMS_MODE_FP32: `table` is fp32 [>= n_news, 300]; CUDA-core fp32 dot products.
+ *     Only rows [0, n_news) are candidates: rows past it (evaluate's PADDED_NEWS replicas, the closing zero row of the fp16
+ *     copy) are never read as candidates.
+ *   - user_vec fp32 [n_users, 300].  exclude_rows int32 [n_users, n_exclude] (n_exclude <= 64) or NULL: those rows are
+ *     never returned for that user -- the intended input is the history rows [n_users, 50].  Entries outside [0, n_news)
+ *     are ignored (the pads), duplicates are harmless.
+ *   - Outputs top_scores fp32 [n_users, k], top_rows int32 [n_users, k].
+ *   - Asynchronous, no host sync, no allocation.  The workspace (nrms_topk_workspace_bytes; 0 for arguments the call
+ *     rejects) grows with n_users * (k + n_exclude) and the number of news splits, never with n_users * n_news.
+ *   - Arguments are checked before any CUDA call: k out of range or n_exclude > 64 -> NRMS_E_UNSUPPORTED; null or
+ *     misaligned pointers (table / user_vec 16 bytes, workspace 256 bytes) -> NRMS_E_INVALID. */
+size_t nrms_topk_workspace_bytes(int64_t n_users, int64_t n_news, int k, int n_exclude, int mode);
+int nrms_topk_news(const void* table, int64_t n_news, const float* user_vec, int64_t n_users,
+                   const int32_t* exclude_rows, int n_exclude, int k,
+                   float* top_scores, int32_t* top_rows,
+                   void* workspace, size_t workspace_bytes, int mode, void* stream);
+
 /* ---- click predictor --------------------------------------------------------------- */
 /* scores[b,c] = cand[b,c,:] . user[b,:]     cand [B,C,X], user [B,X] */
 int nrms_score_fwd(const float* cand, const float* user, int64_t B, int C, int X,

@@ -64,6 +64,8 @@ SIGNATURES = {
     "nrms_copy_rows_strided": (_i32, [_vp, _i64, _vp, _i64, _i64, _i32, _vp]),
     "nrms_recommend_workspace_bytes": (_sz, []),
     "nrms_recommend_user": (_i32, [_vp, _i64, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "nrms_topk_workspace_bytes": (_sz, [_i64, _i64, _i32, _i32, _i32]),
+    "nrms_topk_news": (_i32, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_score_fwd": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _vp]),
     "nrms_score_bwd": (_i32, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     "nrms_score_csr": (_i32, [_vp, _vp, _vp, _vp, _i64, _vp, _vp]),

@@ -642,6 +642,50 @@ def recommend_user(table, hist_rows, cand_rows, wqkv, bqkv, wa, ba, qa, rank=Tru
 
 
 @torch.no_grad()
+def topk_news(table, n_news, user_vec, k, exclude_rows=None, mode=_lib.MODE_TF32):
+    """The k rows of table[:n_news] with the highest dot product with each user vector (nrms_topk_news): returns
+    (scores fp32 [U, k], rows int32 [U, k]) on the device, ordered by score descending and equal scores by row ascending;
+    tail entries (fewer than k rows left) are row -1, score -inf.  No score matrix is materialised and nothing syncs.
+    mode MODE_TF32: `table` is the fp16 [>= n_news, 320] copy of `pack_rows_f16` (tensor cores, user vectors rounded to
+    fp16); MODE_FP32: `table` is fp32 [>= n_news, 300].  exclude_rows: int [U, <= 64] rows never returned for that user
+    (history rows; values outside [0, n_news) such as pads are ignored), on the host or the device."""
+    n_news = int(n_news)
+    if mode == _lib.MODE_TF32:
+        if table.dtype != torch.float16 or table.dim() != 2 or table.shape[1] != 320:
+            raise RuntimeError("topk_news in tensor mode takes the fp16 [n, 320] table of pack_rows_f16, got "
+                               f"{table.dtype} {tuple(table.shape)}")
+    elif mode == _lib.MODE_FP32:
+        if table.dtype != torch.float32 or table.dim() != 2 or table.shape[1] != D:
+            raise RuntimeError(f"topk_news in FP32 mode takes an fp32 [n, {D}] table, got {table.dtype} {tuple(table.shape)}")
+    else:
+        raise ValueError(f"unknown mode {mode!r}")
+    if not 0 < n_news <= table.shape[0]:
+        raise RuntimeError(f"n_news = {n_news} must be in [1, {table.shape[0]}] (rows of the table)")
+    _require_cuda(table, user_vec)
+    lib = _lib.load()
+    dev = table.device
+    table = table.contiguous()
+    u = _f32c(user_vec)
+    if u.dim() != 2 or u.shape[1] != D:
+        raise RuntimeError(f"user_vec must be [U, {D}], got {tuple(u.shape)}")
+    U = u.shape[0]
+    ex, n_ex = None, 0
+    if exclude_rows is not None:
+        ex = torch.as_tensor(exclude_rows).to(device=dev, dtype=torch.int32).contiguous()
+        if ex.dim() != 2 or ex.shape[0] != U:
+            raise RuntimeError(f"exclude_rows must be [U = {U}, n_exclude], got {tuple(ex.shape)}")
+        n_ex = ex.shape[1]
+        if n_ex == 0:
+            ex = None
+    scores = torch.empty((U, k), dtype=torch.float32, device=dev)
+    rows = torch.empty((U, k), dtype=torch.int32, device=dev)
+    ws = _bytes(lib.nrms_topk_workspace_bytes(U, n_news, int(k), n_ex, mode), dev)
+    check(lib.nrms_topk_news(ptr(table), n_news, ptr(u), U, ptr(ex), n_ex, int(k), ptr(scores), ptr(rows), ptr(ws),
+                             ws.numel(), mode, stream_ptr(dev)), "nrms_topk_news")
+    return scores, rows
+
+
+@torch.no_grad()
 def additive_forward(c, wa, ba, qa, mode=_lib.MODE_TF32):
     """Standalone AdditiveAttention.forward, inference only."""
     lib = _lib.load()

@@ -136,6 +136,45 @@ class Recommender:
                                             stream_ptr(dev)), "nrms_recommend_user")
         return st["order"][:n_c], st["scores"][:n_c], st["user"]
 
+    @torch.no_grad()
+    def top_k_rows(self, hist_rows, k, exclude_clicked=True):
+        """The k best news of the whole table for each user, not only for candidates the caller already has.
+        hist_rows: int32 [U, 50] in `history_rows` form (pads = the table's last row), host or device.  Returns (rows int32
+        [U, k], scores fp32 [U, k], user_vec fp32 [U, 300]) on the device, no sync: rows by descending score (equal scores
+        by ascending row), the clicked rows left out when exclude_clicked; tail entries are row -1, score -inf.
+        Arithmetic follows the user encoder's precision: tensor mode scores against an fp16 copy of the table, packed on
+        the first call and kept."""
+        from . import _lib
+        from .config import resolve_mode
+        ue = self.model.user_encoder
+        dev = self.table.device
+        hist = torch.as_tensor(hist_rows).to(device=dev, dtype=torch.int32).contiguous()
+        if hist.dim() != 2 or hist.shape[1] != self.n_hist:
+            raise RuntimeError(f"hist_rows must be [U, {self.n_hist}], got {tuple(hist.shape)}")
+        user_vec = ue.forward_indexed(self.table, hist)
+        mode = resolve_mode(ue.config, ue.precision)
+        if mode == _lib.MODE_TF32:
+            if getattr(self, "_table16", None) is None:
+                self._table16 = ops.pack_rows_f16(self.table)
+            table = self._table16
+        else:
+            table = self.table
+        scores, rows = ops.topk_news(table, self.pad_row, user_vec, k, exclude_rows=hist if exclude_clicked else None,
+                                     mode=mode)
+        return rows, scores, user_vec
+
+    def top_k(self, clicked_news, k, exclude_clicked=True):
+        """Id form of `top_k_rows` for one user: clicked_news = list of news ids -> (news ids by descending score,
+        y = (score + 1) / 2 in that order), the pair and convention of `recommend` (src/recommend.py:338-340) over the
+        whole table.  Fewer than k ids come back when fewer news remain."""
+        hist = torch.tensor([self.history_rows(clicked_news)], dtype=torch.int32)
+        rows, scores, _ = self.top_k_rows(hist, k, exclude_clicked)
+        rows = rows[0].cpu().numpy()
+        scores = scores[0].cpu().numpy()
+        keep = rows >= 0
+        y = (scores[keep].astype(np.float64) + 1.0) / 2.0
+        return np.array(self.ids, dtype=object)[rows[keep]].astype(str), y
+
     def recommend(self, clicked_news, impressions):
         """clicked_news: list of news ids; impressions: list of candidate ids, optionally 'id-label' strings
         (src/recommend.py:301-332) -> (candidate ids sorted by descending score, y = (score + 1) / 2 sorted), the pair
