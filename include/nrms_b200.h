@@ -231,8 +231,9 @@ int nrms_copy_rows_strided(const float* src, int64_t src_stride, float* dst, int
 
 /* ---- single-user latency path (SURVEY 8 f4; src/recommend.py:245-341) ---------------------
  * One user, two cluster launches: user_vec [300] = UserEncoder(table[hist_rows[0..50)]), scores[c] = table[cand_rows[c]] .
- * user_vec, order = candidate positions by descending score (equal scores in ascending position: np.argsort(-y) of
- * recommend.py:339 on a stable sort).  table fp32 [n_rows, 300] (the news2vector cache, PADDED_NEWS = a zero row);
+ * user_vec, order = candidate positions by descending score (equal scores in ascending position, -0 == +0; NaN scores
+ * after every number, -inf included, in ascending position: np.argsort(-y) of recommend.py:339 on a stable sort).
+ * table fp32 [n_rows, 300] (the news2vector cache, PADDED_NEWS = a zero row);
  * hist_rows int32 [50] and cand_rows int32 [C] are DEVICE arrays with values in [0, n_rows) (an out-of-range value
  * reads row n_rows - 1).  order may be NULL (scores only); with order, C <= 4096.  FP32 arithmetic. */
 size_t nrms_recommend_workspace_bytes(void);

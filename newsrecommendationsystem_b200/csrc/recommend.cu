@@ -57,6 +57,13 @@ struct SmemA {
 #define LAT_PRINT(name, n)
 #endif
 
+// Ranking key of a score: unsigned order = score order, -0 == +0, and NaN (key 0) below every number, -inf included.
+__device__ __forceinline__ uint32_t rank_key(float s) {
+  if (s != s) return 0u;
+  const uint32_t u = __float_as_uint(s == 0.f ? 0.f : s);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem));
@@ -215,7 +222,7 @@ pool_score_kernel(const float* __restrict__ table, int64_t n_rows, const int32_t
                   int32_t* __restrict__ order) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   SmemB& sm = *reinterpret_cast<SmemB*>(smem_raw);
-  float* sc = reinterpret_cast<float*>(smem_raw + sizeof(SmemB));     // [C rounded up to 4]: every candidate's score
+  uint32_t* sc = reinterpret_cast<uint32_t*>(smem_raw + sizeof(SmemB));   // [C rounded up to 4]: every rank_key(score)
   cg::cluster_group cluster = cg::this_cluster();
   const int r = (int)cluster.block_rank();
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -224,7 +231,7 @@ pool_score_kernel(const float* __restrict__ table, int64_t n_rows, const int32_t
   LAT_T(0);
 
   for (int f = tid; f < S * DV4; f += THREADS) cp_async16(&sm.ctx[0][0] + 4 * f, ctx_g + 4 * f);
-  if (order != nullptr && tid < 4) sc[((C + 3) & ~3) - 1 - tid] = -INFINITY;    // pad entries never sort before anything
+  if (order != nullptr && tid < 4) sc[((C + 3) & ~3) - 1 - tid] = 0u;   // pad entries (j >= C) never sort before anything
   // warp = history rows warp, warp + 8, ..; lane = additive unit (25 of 32 lanes).  The loads of a batch of rows are all
   // issued before the first is used, and the row sums come from shuffles (shared-memory float atomics on one address
   // per row serialise: 13k of the first version's 16k cycles).
@@ -316,7 +323,7 @@ pool_score_kernel(const float* __restrict__ table, int64_t n_rows, const int32_t
       const int l = lane + 32 * k;
       u[k] = (l < DV4) ? *reinterpret_cast<const float4*>(&sm.user[4 * l]) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    float* sc_remote = (order != nullptr && lane < CL) ? cluster.map_shared_rank(sc, lane) : nullptr;
+    uint32_t* sc_remote = (order != nullptr && lane < CL) ? cluster.map_shared_rank(sc, lane) : nullptr;
     constexpr int INF = 4;
     for (int c0 = r * 8 + warp; c0 < C; c0 += INF * CL * 8) {
       float4 a[INF][3];
@@ -344,7 +351,7 @@ pool_score_kernel(const float* __restrict__ table, int64_t n_rows, const int32_t
         s0 = warp_sum(s0);
         if (c < C) {
           if (lane == 0) scores[c] = s0;
-          if (sc_remote != nullptr) sc_remote[c] = s0;
+          if (sc_remote != nullptr) sc_remote[c] = rank_key(s0);
         }
       }
     }
@@ -354,15 +361,16 @@ pool_score_kernel(const float* __restrict__ table, int64_t n_rows, const int32_t
   cluster.sync();
   LAT_T(5);
 
-  // rank by counting: candidate i goes to position #{j : s_j > s_i or (s_j == s_i and j < i)} -- descending score, equal
-  // scores in ascending candidate position (np.argsort(-y) of recommend.py:339 on a stable sort).  CTA r ranks the
-  // candidates i = r (mod 8); every comparison reads shared memory as a warp broadcast.
+  // rank by counting: candidate i goes to position #{j : k_j > k_i or (k_j == k_i and j < i)} over the keys k = rank_key(s)
+  // -- descending score, equal scores in ascending candidate position, NaN last and in candidate order (np.argsort(-y) of
+  // recommend.py:339 on a stable sort).  CTA r ranks the candidates i = r (mod 8); every comparison reads shared memory
+  // as a warp broadcast.
   const int C4 = (C + 3) & ~3;
   for (int i = r + CL * tid; i < C; i += CL * THREADS) {
-    const float si = sc[i];
+    const uint32_t si = sc[i];
     int before = 0;
     for (int j = 0; j < C4; j += 4) {
-      const float4 sj = *reinterpret_cast<const float4*>(sc + j);
+      const uint4 sj = *reinterpret_cast<const uint4*>(sc + j);
       before += (sj.x > si || (sj.x == si && j < i)) ? 1 : 0;
       before += (sj.y > si || (sj.y == si && j + 1 < i)) ? 1 : 0;
       before += (sj.z > si || (sj.z == si && j + 2 < i)) ? 1 : 0;

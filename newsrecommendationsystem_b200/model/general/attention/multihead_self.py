@@ -31,7 +31,9 @@ class MultiHeadSelfAttention(nn.Module):
         """([W_Q;W_K;W_V] [3D,D], [b_Q;b_K;b_V] [3D]) -- autograd splits the gradients back.
 
         Without grad mode (inference: evaluate encodes thousands of batches with fixed parameters) the concatenation is
-        cached and reused until a parameter is written (tensor version counters) or moved."""
+        cached and reused until a parameter is written (tensor version counters) or moved.  Every writer of the
+        parameters must bump their version: torch's in-place ops do, and so does FusedAdam.step, whose kernel writes
+        through raw pointers."""
         ps = (self.W_Q.weight, self.W_K.weight, self.W_V.weight, self.W_Q.bias, self.W_K.bias, self.W_V.bias)
         if torch.is_grad_enabled():
             return torch.cat(ps[:3], dim=0), torch.cat(ps[3:], dim=0)

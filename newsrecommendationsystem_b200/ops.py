@@ -15,9 +15,10 @@ from . import _lib
 from ._lib import check, ptr, stream_ptr
 
 D, H, QD = 300, 15, 200
-# True (set by optim.FusedAdam): the news encoder's backward accumulates the embedding gradient directly into the
-# parameter's existing .grad buffer instead of returning a fresh 85 MB tensor for autograd to add.
-EMB_GRAD_IN_PLACE = False
+# An embedding parameter marked `_nrms_grad_sink` (optim.FusedAdam marks the parameters it owns) has a .grad that is a
+# live view of the optimizer's flat gradient: the news encoder's backward accumulates the embedding gradient directly
+# into it instead of returning a fresh 85 MB tensor for autograd to add.  Every other embedding gets its gradient
+# through autograd, so torch.autograd.grad and backward(inputs=...) see it.
 
 
 def _require_cuda(*tensors):
@@ -73,7 +74,7 @@ class _NewsEncoderFn(torch.autograd.Function):
             if needs_grad:
                 ctx.save_for_backward(tokens, wqkv_c, wa_c, qa_c, stash, *([lnw_c] if ln else []))
                 ctx.meta = (n, L, emb_c.shape[0], float(dropout_p), int(seed), int(offset), mode, ln)
-                ctx.emb_param = emb if (EMB_GRAD_IN_PLACE and emb.is_leaf) else None
+                ctx.emb_param = emb if (emb.is_leaf and getattr(emb, "_nrms_grad_sink", False)) else None
                 ctx.rows = rows
             return out
         ctx.rows = None
@@ -95,7 +96,7 @@ class _NewsEncoderFn(torch.autograd.Function):
         if needs_grad:
             ctx.save_for_backward(tokens, wqkv_c, wa_c, qa_c, stash, *([lnw_c] if ln else []))
             ctx.meta = (n, L, emb_c.shape[0], float(dropout_p), int(seed), int(offset), mode, ln)
-            ctx.emb_param = emb if (EMB_GRAD_IN_PLACE and emb.is_leaf) else None
+            ctx.emb_param = emb if (emb.is_leaf and getattr(emb, "_nrms_grad_sink", False)) else None
         return out
 
     @staticmethod

@@ -5,7 +5,8 @@ betas=(0.9,0.999), eps=1e-8).  On construction the parameters are re-pointed int
 device buffer and their `.grad` into one flat gradient buffer, so that
   * the update is a single libnrms_b200 launch streaming 4 reads + 3 writes per element, and
   * data-parallel training needs exactly one NCCL all-reduce per step (`allreduce_grads`).
-Parameter names/shapes (state_dict) are untouched; `load_state_dict` copies in place.
+Parameter names/shapes (state_dict) are untouched; `load_state_dict` copies in place.  `step()` bumps every parameter's
+version counter, as an in-place torch op would.
 """
 from __future__ import annotations
 
@@ -42,9 +43,9 @@ class FusedAdam(torch.optim.Optimizer):
                 view.copy_(p.data)
                 p.data = view
                 p.grad = self.flat_grad[o:o + p.numel()].view_as(p)
+                p._nrms_grad_sink = True   # its .grad is a live view of flat_grad: the news encoder may scatter into it
         self._params, self._offsets = ps, offs
         self.step_count = 0
-        ops.EMB_GRAD_IN_PLACE = True       # .grad of every parameter is a live view of flat_grad from here on
         # data parallel: every replica starts from rank 0's parameters (the gradient all-reduce keeps them identical from
         # then on; replicas built from different seeds would otherwise diverge silently)
         import torch.distributed as dist
@@ -81,6 +82,9 @@ class FusedAdam(torch.optim.Optimizer):
         ops.adam_step_(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_count,
                        lr=g["lr"], betas=g["betas"], eps=g["eps"], weight_decay=g["weight_decay"],
                        decoupled=g["decoupled"], grad_scale=grad_scale)
+        # the kernel writes through raw pointers, which autograd does not see: bump every parameter's version counter so
+        # caches keyed on it (MultiHeadSelfAttention.packed, Recommender) rebuild and saved-tensor checks hold
+        torch.autograd.graph.increment_version(self._params)
         return loss
 
 

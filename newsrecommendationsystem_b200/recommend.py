@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 import csv
+import ctypes as C
 import os
 
 from . import ops
@@ -102,38 +103,44 @@ class Recommender:
                   "idx_host": torch.empty(self.n_hist + 4096, dtype=torch.int32).pin_memory(),
                   "idx_dev": torch.empty(self.n_hist + 4096, dtype=torch.int32, device=dev),
                   "scores": torch.empty(4096, dtype=torch.float32, device=dev),
-                  "order": torch.empty(4096, dtype=torch.int32, device=dev)}
+                  "order": torch.empty(4096, dtype=torch.int32, device=dev),
+                  "copied": torch.cuda.Event()}        # recorded after each idx_host -> idx_dev copy
             self._st = st
         return st
 
     @torch.no_grad()
     def recommend_rows(self, hist_rows, cand_rows):
-        """Row-index form: returns (order int32 [C], scores fp32 [C], user_vec fp32 [300]) on the device, no sync.
+        """Row-index form: returns (order int32 [C], scores fp32 [C], user_vec fp32 [300]) on the device.
         Up to 4,096 candidates go through preallocated buffers (one pinned H2D copy of 50 + C indices, two launches);
-        the returned tensors are views that the next call overwrites."""
-        from ._lib import check, ptr, stream_ptr
+        the returned tensors are views that the next call overwrites.  The host waits only when the previous call's
+        index copy has not run yet, before it rewrites the pinned staging buffer; otherwise nothing syncs.
+        Order: score descending, equal scores by ascending candidate position, NaN scores last (np.argsort(-y) on a
+        stable sort), on both sides of the 4,096-candidate limit."""
+        from ._lib import check, ptr
         n_c = len(cand_rows)
+        dev = self.table.device
         if n_c > 4096:
-            dev = self.table.device
             ue = self.model.user_encoder
             a = ue.additive_attention
             user, scores, _ = ops.recommend_user(self.table, torch.as_tensor(hist_rows, dtype=torch.int32).to(dev),
                                                  torch.as_tensor(cand_rows, dtype=torch.int32).to(dev),
                                                  *ue.multihead_self_attention.packed(), a.linear.weight, a.linear.bias,
                                                  a.attention_query_vector, rank=False)
-            return torch.argsort(scores, descending=True, stable=True).int(), scores, user
+            return torch.argsort(-scores, stable=True).int(), scores, user     # ascending sort puts NaN last
         st = self._state()
+        st["copied"].synchronize()                 # the previous call's copy may still read idx_host
         h = st["idx_host"]
         h[:self.n_hist] = torch.as_tensor(hist_rows, dtype=torch.int32)
         h[self.n_hist:self.n_hist + n_c] = torch.as_tensor(cand_rows, dtype=torch.int32)
         d = st["idx_dev"]
         d[:self.n_hist + n_c].copy_(h[:self.n_hist + n_c], non_blocking=True)
+        stream = torch.cuda.current_stream(dev)
+        st["copied"].record(stream)
         w = st["w"]
-        dev = self.table.device
         check(st["lib"].nrms_recommend_user(ptr(self.table), self.table.shape[0], ptr(d), ptr(d[self.n_hist:]), n_c,
                                             ptr(w[0]), ptr(w[1]), ptr(w[2]), ptr(w[3]), ptr(w[4]), ptr(st["user"]),
                                             ptr(st["scores"]), ptr(st["order"]), ptr(st["ws"]), st["ws"].numel(),
-                                            stream_ptr(dev)), "nrms_recommend_user")
+                                            C.c_void_p(stream.cuda_stream)), "nrms_recommend_user")
         return st["order"][:n_c], st["scores"][:n_c], st["user"]
 
     @torch.no_grad()
