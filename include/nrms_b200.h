@@ -77,8 +77,9 @@ int64_t nrms_launch_count(void);
  *  context rows never leave the SM; measured slower than K1g + K2, see DESIGN.md).
  * "attn_safe_softmax" (default -1): -1 = the attention kernels choose between 2^s and the row-shifted form
  *  2^(s - max) / (Z + 1e-8 * 2^-max) from a bound on the scores, 0 / 1 force one form (tests).
- * "train_attn_mma" (default 1): tensor-mode training attention over titles on mma.sync TF32 tiles (attn_mma.cu); 0 = the
- *  CUDA-core kernels of the FP32 mode.
+ * "train_attn_mma" (default 1): tensor-mode training attention of the news encoder, over titles (L = 20) and 50-token
+ *  texts (L = 50), on mma.sync TF32 tiles (attn_mma.cu); 0 = the CUDA-core kernels of the FP32 mode.  The user
+ *  encoder's S = 50 training attention stays on the CUDA-core kernel either way.
  * "k1f_debug": component-removal timing masks of K1f (garbage results; profiles/k1f_probe.py). */
 int nrms_set_option(const char* key, int value);
 /* "time_k1" = 1 brackets every fused K1 launch with CUDA events on the launching stream (clears the previous
@@ -102,7 +103,8 @@ size_t nrms_encoder_bwd_workspace_bytes(int64_t n_seq, int S, int mode);
 /* News encoder forward: tokens int64 [n_titles, L] -> out fp32 [n_titles, 300].
  * emb: [num_words, 300].  stash: NULL for inference, else nrms_encoder_stash_bytes bytes.
  * dropout_p in [0,1): 0 = eval mode.  (seed, offset) key the in-kernel Philox stream.
- * L = 20 (title, config.num_words_title); inference (stash == NULL) also accepts L = 50 (a 50-token text). */
+ * L = 20 (title, config.num_words_title) or 50 (a 50-token text such as Exp1's abstract), for training (stash != NULL)
+ * and inference alike; any other L returns NRMS_E_UNSUPPORTED before any CUDA call. */
 int nrms_news_encoder_fwd(const int64_t* tokens, int64_t n_titles, int L,
                           const float* emb, int64_t num_words,
                           const float* wqkv, const float* bqkv,
@@ -121,7 +123,8 @@ int nrms_news_encoder_i32_fwd(const int32_t* tokens, int64_t n_titles, int L,
                               const float* wa, const float* ba, const float* qa,
                               float* out, void* workspace, size_t workspace_bytes, void* stream);
 
-/* News encoder backward.  d_out [n_titles,300].  Gradients are ACCUMULATED (+=) into
+/* News encoder backward (L = 20 or 50, as the forward that wrote the stash).  d_out [n_titles,300].  Gradients are
+ * ACCUMULATED (+=) into
  * d_emb [num_words,300] (row 0 = padding_idx is never touched), d_wqkv [900,300],
  * d_bqkv [900], d_wa [200,300], d_ba [200], d_qa [200]. */
 int nrms_news_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_titles, int L,
@@ -192,8 +195,8 @@ int nrms_additive_bwd(const float* d_out, const float* c, int64_t n_seq, int S, 
  * The reference DataLoader ships 1+K+50 token tensors per step (src/dataset.py:17-85, src/train.py:118-124); here the
  * pre-tokenised news table int64 [n_news, L] lives on the device and a minibatch is news-row indices: title t of the call
  * is row news_rows[t] (int64, in [0, n_news)) of token_table, gathered inside the embedding gather / gradient scatter
- * kernels.  Training form only (stash required); ln_* NULL = plain NRMS, else the config-5 variant.  Stash / workspace
- * sizes and the gradient contract are those of nrms_news_encoder_fwd / _bwd. */
+ * kernels.  Training form only (stash required); ln_* NULL = plain NRMS, else the config-5 variant.  L = 20 or 50.
+ * Stash / workspace sizes and the gradient contract are those of nrms_news_encoder_fwd / _bwd. */
 int nrms_news_encoder_rows_fwd(const int64_t* token_table, int64_t n_news, const int64_t* news_rows, int64_t n_titles,
                                int L, const float* emb, int64_t num_words, const float* wqkv, const float* bqkv,
                                const float* ln_gamma, const float* ln_beta, const float* wa, const float* ba,

@@ -433,6 +433,337 @@ attn_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, 
 
 }  // namespace amma
 
+// ---- 50-token texts (the abstract encoder of model/Exp1) ------------------------------------------------------------
+// Same contractions and semantics as the title kernels above, but their layout does not carry over: per (text, head) the
+// scores are 50 x 50, so a whole score fragment per warp would not fit the registers, and dS / attn (50 x 50) no longer
+// fit the dead K / V tiles the title backward parks them in.
+//
+// Layout.  One warp per (text, head); tiles Q, K, V (and G = dO in the backward) of [56 rows][28 floats]: keys pad to 7
+// n8 tiles (rows 50..55 stay zero), queries to 4 m16 tiles (rows 56..63 are not stored: their fragment loads read zero),
+// the head dimension to 3 k8 steps (columns 20..27 stay zero).  The tiles are read-only once staged.
+//   forward:  per 16-query tile, S = Q K^T (28 accumulators), attn, O = attn V (12 accumulators), dropout-2 mask drawn
+//             in registers (one Philox evaluation per lane and 8-column block, halves exchanged between lane pairs)
+//   backward, pass 1, per 16-query tile:  S = Q K^T, attn, dP = G V^T, dS, dQ = dS K; 1 / (sum + eps) and
+//             delta = sum_j attn dP of every query row are kept in shared memory (2 x 64 floats per head)
+//   backward, pass 2, per 16-key tile:    S^T = K Q^T, attn^T = exp(S^T / sqrt 20) / (sum + eps) of the query column,
+//             dP^T = V G^T, dS^T = attn^T (dP^T - delta) / sqrt 20, dK = dS^T Q (dS split hi + lo, as in the title
+//             kernel: the K-bias gradient is a sum that cancels), dV = attn^T G
+// So the scores and exponentials are computed twice (seven 64 x 56 x 24 contractions instead of five) rather than parking
+// two 50 x 50 matrices per head in shared memory.  Heads per CTA: 3 in the forward (56 KB, 4 CTAs per SM), 1 in the
+// backward (25.6 KB, 8 CTAs per SM); the warps never wait for each other, so a CTA of one warp loses nothing.
+namespace amma50 {
+
+constexpr int S = 50;            // tokens per text
+constexpr int RT = 56;           // tile rows (7 x 8)
+constexpr int ST = 28;           // tile row pitch in floats (conflict-free fragment loads, see amma)
+constexpr int TILE = RT * ST;
+constexpr int MT = 4;            // 16-row tiles over the queries (64 >= 50)
+constexpr int NT = 7;            // 8-column tiles over the keys (56 >= 50)
+constexpr int HC_FWD = 3, HC_BWD = 1;
+constexpr int ZS = 64;           // floats per per-row vector (1 / (sum + eps), delta) of the backward
+
+typedef float Row[NT][4];        // accumulators of 16 rows x 56 columns
+typedef float Out[3][4];         // accumulators of 16 rows x 24 columns (the head dimension)
+
+template <typename F>
+__device__ __forceinline__ void zero(F& c) {
+  float* f = &c[0][0];
+#pragma unroll
+  for (int i = 0; i < (int)(sizeof(F) / sizeof(float)); ++i) f[i] = 0.f;
+}
+
+// c[i][j] += sum_d A[m0 + i][d] B[j][d]     (16 rows of tile A from row m0, the 56 rows of tile B)
+__device__ __forceinline__ void gemm_nt(Row& c, const float* A, int m0, const float* B, int g, int t) {
+  const int r0 = m0 + g, r1 = r0 + 8;
+#pragma unroll
+  for (int ks = 0; ks < 3; ++ks) {
+    const uint32_t a0 = amma::ld(A + r0 * ST + ks * 8 + t), a2 = amma::ld(A + r0 * ST + ks * 8 + t + 4);
+    const uint32_t a1 = r1 < RT ? amma::ld(A + r1 * ST + ks * 8 + t) : 0u;
+    const uint32_t a3 = r1 < RT ? amma::ld(A + r1 * ST + ks * 8 + t + 4) : 0u;
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt) {
+      const uint32_t b0 = amma::ld(B + (nt * 8 + g) * ST + ks * 8 + t), b1 = amma::ld(B + (nt * 8 + g) * ST + ks * 8 + t + 4);
+      amma::mma_tf32(c[nt], a0, a1, a2, a3, b0, b1);
+    }
+  }
+}
+
+// c[i][d] += sum_j P[i][j] B[j][d]          (P: accumulators used in place as the A operand, see amma::gemm_frag_n)
+// SPLIT: P is taken as tf32(P) + tf32(P - tf32(P)), two products per step
+template <bool SPLIT>
+__device__ __forceinline__ void gemm_frag_n(Out& c, const Row& p, const float* B, int g, int t) {
+#pragma unroll
+  for (int ks = 0; ks < NT; ++ks) {
+    float hi[4], lo[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      hi[e] = amma::tf32_round(p[ks][e]);
+      lo[e] = SPLIT ? amma::tf32_round(p[ks][e] - hi[e]) : 0.f;
+    }
+#pragma unroll
+    for (int nt = 0; nt < 3; ++nt) {
+      const uint32_t b0 = amma::ld(B + (ks * 8 + 2 * t) * ST + nt * 8 + g), b1 = amma::ld(B + (ks * 8 + 2 * t + 1) * ST + nt * 8 + g);
+      amma::mma_tf32(c[nt], __float_as_uint(hi[0]), __float_as_uint(hi[2]), __float_as_uint(hi[1]), __float_as_uint(hi[3]), b0, b1);
+      if (SPLIT)
+        amma::mma_tf32(c[nt], __float_as_uint(lo[0]), __float_as_uint(lo[2]), __float_as_uint(lo[1]), __float_as_uint(lo[3]), b0, b1);
+    }
+  }
+}
+
+constexpr float SCALE_LOG2E = 1.4426950408889634f / amma::SQRT_DH;     // exp(s / sqrt 20) = 2^(s * log2(e) / sqrt 20)
+constexpr float INV_SQRT_DH = 1.f / amma::SQRT_DH;
+
+// raw scores -> attention weights in place (key columns >= 50 -> 0); inv[half] = 1 / (row sum + 1e-8) of row g + 8 half
+__device__ __forceinline__ void softmax_rows(Row& c, int t, float (&inv)[2]) {
+#pragma unroll
+  for (int half = 0; half < 2; ++half) {
+    float sum = 0.f;
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        const int col = nt * 8 + 2 * t + e;
+        const float v = col < S ? amma::ex2(c[nt][half * 2 + e] * SCALE_LOG2E) : 0.f;
+        c[nt][half * 2 + e] = v;
+        sum += v;
+      }
+    sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+    sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+    inv[half] = 1.f / (sum + amma::ATTN_EPS);
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+      for (int e = 0; e < 2; ++e) c[nt][half * 2 + e] *= inv[half];
+  }
+}
+
+// rows m0 .. m0 + 15 (those < 50) of an Out fragment to global rows of pitch ld_ (two floats per store)
+__device__ __forceinline__ void store_rows(float* dst, int64_t ld_, const Out& c, int m0, int g, int t) {
+#pragma unroll
+  for (int nt = 0; nt < 3; ++nt)
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+      const int row = m0 + g + 8 * half, col = nt * 8 + 2 * t;
+      if (row < S && col < DH)
+        *reinterpret_cast<float2*>(dst + row * ld_ + col) = make_float2(c[nt][half * 2], c[nt][half * 2 + 1]);
+    }
+}
+
+// the same rows written transposed, dstT[col * ldt + row] (the K-major operand of the dWqkv contraction).  A column of a
+// 16-row tile is 64 contiguous bytes of dstT, and each store instruction of the warp fills four 32-byte sectors (eight
+// consecutive rows of four columns), so the scalar stores waste no bandwidth.
+__device__ __forceinline__ void store_cols(float* dstT, int64_t ldt, const Out& c, int m0, int g, int t) {
+#pragma unroll
+  for (int nt = 0; nt < 3; ++nt)
+#pragma unroll
+    for (int half = 0; half < 2; ++half)
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        const int row = m0 + g + 8 * half, col = nt * 8 + 2 * t + e;
+        if (row < S && col < DH) dstT[(int64_t)col * ldt + row] = c[nt][half * 2 + e];
+      }
+}
+
+// warp-private staging as amma::warp_fetch: tile w <- columns [w*300 + col0, +20) of the text's 50 qkv rows for w < 3,
+// of its d_ctx rows (times the dropout-2 mask) for w == 3; 250 sixteen-byte pieces per tile, rounded to TF32 in place
+template <int NTILES>
+__device__ __forceinline__ void fetch(float* tiles, const float* __restrict__ qkv_head, const float* __restrict__ g_head,
+                                      int lane, int64_t row0, int col0, float p, float scale, uint64_t seed, uint64_t offset) {
+  constexpr int PIECES = S * (DH / 4);
+  constexpr int PT = (PIECES + 31) / 32;
+#pragma unroll
+  for (int w = 0; w < NTILES; ++w)
+#pragma unroll
+    for (int k = 0; k < PT; ++k) {
+      const int f = lane + 32 * k, j = f / (DH / 4), d4 = f % (DH / 4);
+      if (f < PIECES) {
+        const float* src = (w < 3) ? qkv_head + (int64_t)j * D3 + w * D + d4 * 4 : g_head + (int64_t)j * D + d4 * 4;
+        amma::cp_async16(tiles + w * TILE + j * ST + d4 * 4, src);
+      }
+    }
+  amma::cp_async_wait_all();
+#pragma unroll
+  for (int w = 0; w < NTILES; ++w)
+#pragma unroll
+    for (int k = 0; k < PT; ++k) {
+      const int f = lane + 32 * k, j = f / (DH / 4), d4 = f % (DH / 4);
+      if (f < PIECES) {
+        float4* q = reinterpret_cast<float4*>(tiles + w * TILE + j * ST + d4 * 4);
+        float4 x = *q;
+        if (w == 3 && p > 0.f) {
+          const float4 m = dropout_mask4((uint64_t)(row0 + j) * D + col0 + d4 * 4, amma::DROPOUT_STREAM_CTX, p, scale, seed, offset);
+          x.x *= m.x; x.y *= m.y; x.z *= m.z; x.w *= m.w;
+        }
+        *q = make_float4(amma::tf32_round(x.x), amma::tf32_round(x.y), amma::tf32_round(x.z), amma::tf32_round(x.w));
+      }
+    }
+  __syncwarp();
+}
+
+__global__ void __launch_bounds__(HC_FWD * 32)
+attn50_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ ctx, int64_t n_seq, float p, float scale, uint64_t seed,
+                  uint64_t offset) {
+  extern __shared__ __align__(16) float smem[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
+  for (int f = tid; f < HC_FWD * 3 * TILE; f += blockDim.x) smem[f] = 0.f;
+  __syncthreads();
+  float* Q = smem + warp * 3 * TILE;
+  const float* K = Q + TILE;
+  const float* V = K + TILE;
+  const int colbase = blockIdx.y * (HC_FWD * DH) + warp * DH;
+  for (int64_t seq = blockIdx.x; seq < n_seq; seq += gridDim.x) {
+    __syncwarp();             // every lane is done with the previous text's tiles
+    fetch<3>(Q, qkv + seq * S * D3 + colbase, nullptr, lane, seq * S, colbase, 0.f, 1.f, 0, 0);
+#pragma unroll 1
+    for (int mt = 0; mt < MT; ++mt) {
+      Row a;
+      zero(a);
+      gemm_nt(a, Q, mt * 16, K, g, t);
+      float inv[2];
+      softmax_rows(a, t, inv);
+      Out o;
+      zero(o);
+      gemm_frag_n<false>(o, a, V, g, t);
+      if (p > 0.f) {
+        // dropout-2 mask of element (seq*50 + row) * 300 + col: a Philox evaluation yields an aligned group of four
+        // columns, and a lane pair (t, t^1) holds two columns of one group in two rows.  The even lane draws row g's
+        // group, the odd lane row g + 8's, and each hands its partner the half it needs.
+#pragma unroll
+        for (int nt = 0; nt < 3; ++nt) {
+          const int odd = t & 1;
+          const float4 m = dropout_mask4((uint64_t)(seq * S + mt * 16 + g + 8 * odd) * D + colbase + nt * 8 + (t >> 1) * 4,
+                                         amma::DROPOUT_STREAM_CTX, p, scale, seed, offset);
+          const float r0 = __shfl_xor_sync(0xffffffffu, odd ? m.x : m.z, 1);
+          const float r1 = __shfl_xor_sync(0xffffffffu, odd ? m.y : m.w, 1);
+          o[nt][0] *= odd ? r0 : m.x;
+          o[nt][1] *= odd ? r1 : m.y;
+          o[nt][2] *= odd ? m.z : r0;
+          o[nt][3] *= odd ? m.w : r1;
+        }
+      }
+      store_rows(ctx + seq * S * D + colbase, D, o, mt * 16, g, t);
+    }
+  }
+}
+
+__global__ void __launch_bounds__(HC_BWD * 32)
+attn50_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, float* __restrict__ d_qkv,
+                  float* __restrict__ d_qkv_t, int64_t ldt, int64_t n_seq, float p, float scale, uint64_t seed,
+                  uint64_t offset) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int PER_WARP = 4 * TILE + 2 * ZS;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
+  for (int f = tid; f < HC_BWD * PER_WARP; f += blockDim.x) smem[f] = 0.f;
+  __syncthreads();
+  float* Q = smem + warp * PER_WARP;
+  const float* K = Q + TILE;
+  const float* V = K + TILE;
+  const float* G = V + TILE;
+  float* zinv = Q + 4 * TILE;
+  float* delta = zinv + ZS;
+  const int colbase = blockIdx.y * (HC_BWD * DH) + warp * DH;
+  for (int64_t seq = blockIdx.x; seq < n_seq; seq += gridDim.x) {
+    __syncwarp();             // every lane is done with the previous text's tiles and row vectors
+    fetch<4>(Q, qkv + seq * S * D3 + colbase, d_ctx + seq * S * D + colbase, lane, seq * S, colbase, p, scale, seed, offset);
+    float* out = d_qkv + seq * S * D3 + colbase;
+    float* out_t = d_qkv_t ? d_qkv_t + (int64_t)colbase * ldt + seq * S : nullptr;     // [900, ldt]: row = column of dQKV
+    // ---- pass 1: query tiles -> dQ, row vectors ----
+#pragma unroll 1
+    for (int mt = 0; mt < MT; ++mt) {
+      Row a, dp;
+      zero(a);
+      gemm_nt(a, Q, mt * 16, K, g, t);
+      float inv[2];
+      softmax_rows(a, t, inv);                // a = attn
+      zero(dp);
+      gemm_nt(dp, G, mt * 16, V, g, t);       // dp = dO V^T
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        float dl = 0.f;
+#pragma unroll
+        for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) dl = fmaf(a[nt][half * 2 + e], dp[nt][half * 2 + e], dl);
+        dl += __shfl_xor_sync(0xffffffffu, dl, 1);
+        dl += __shfl_xor_sync(0xffffffffu, dl, 2);
+#pragma unroll
+        for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) dp[nt][half * 2 + e] = a[nt][half * 2 + e] * (dp[nt][half * 2 + e] - dl) * INV_SQRT_DH;
+        const int row = mt * 16 + g + 8 * half;
+        if (t == 0 && row < S) {
+          zinv[row] = inv[half];
+          delta[row] = dl;
+        }
+      }
+      Out r;
+      zero(r);
+      gemm_frag_n<false>(r, dp, K, g, t);     // dQ = dS K
+      store_rows(out, D3, r, mt * 16, g, t);
+      if (out_t) store_cols(out_t, ldt, r, mt * 16, g, t);
+    }
+    __syncwarp();             // the row vectors are visible to every lane
+    // ---- pass 2: key tiles -> dK, dV ----
+#pragma unroll 1
+    for (int kt = 0; kt < MT; ++kt) {
+      Row a, dp;
+      zero(a);
+      gemm_nt(a, K, kt * 16, Q, g, t);        // S^T: rows = keys, columns = queries
+      zero(dp);
+      gemm_nt(dp, V, kt * 16, G, g, t);       // dP^T = V dO^T
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int col = nt * 8 + 2 * t + e;
+          const float z = col < S ? zinv[col] : 0.f, dl = col < S ? delta[col] : 0.f;
+#pragma unroll
+          for (int half = 0; half < 2; ++half) {
+            const float at = col < S ? amma::ex2(a[nt][half * 2 + e] * SCALE_LOG2E) * z : 0.f;
+            a[nt][half * 2 + e] = at;                                                     // attn^T
+            dp[nt][half * 2 + e] = at * (dp[nt][half * 2 + e] - dl) * INV_SQRT_DH;        // dS^T
+          }
+        }
+      Out r;
+      zero(r);
+      gemm_frag_n<true>(r, dp, Q, g, t);      // dK = (dS_hi + dS_lo)^T Q
+      store_rows(out + D, D3, r, kt * 16, g, t);
+      if (out_t) store_cols(out_t + (int64_t)D * ldt, ldt, r, kt * 16, g, t);
+      zero(r);
+      gemm_frag_n<false>(r, a, G, g, t);      // dV = attn^T dO
+      store_rows(out + 2 * D, D3, r, kt * 16, g, t);
+      if (out_t) store_cols(out_t + (int64_t)2 * D * ldt, ldt, r, kt * 16, g, t);
+    }
+  }
+}
+
+}  // namespace amma50
+
+int attn_mma50_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st) {
+  const size_t smem = (size_t)amma50::HC_FWD * 3 * amma50::TILE * sizeof(float);
+  static bool configured[64] = {false};
+  if (cudaError_t e = set_max_dynamic_smem(amma50::attn50_fwd_kernel, (int)smem, configured)) return cuda_fail(e, "attn_mma50_fwd attr");
+  int64_t gx = n_seq < (int64_t)num_sms() * 8 ? n_seq : (int64_t)num_sms() * 8;
+  const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
+  amma50::attn50_fwd_kernel<<<dim3((unsigned)gx, H / amma50::HC_FWD), amma50::HC_FWD * 32, smem, st>>>(qkv, ctx, n_seq, p, scale,
+                                                                                                   seed, offset);
+  NRMS_LAUNCH_CHECK("attn_mma50_fwd");
+  return NRMS_OK;
+}
+
+int attn_mma50_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
+                   uint64_t seed, uint64_t offset, cudaStream_t st) {
+  const size_t smem = (size_t)amma50::HC_BWD * (4 * amma50::TILE + 2 * amma50::ZS) * sizeof(float);
+  static bool configured[64] = {false};
+  if (cudaError_t e = set_max_dynamic_smem(amma50::attn50_bwd_kernel, (int)smem, configured)) return cuda_fail(e, "attn_mma50_bwd attr");
+  int64_t gx = n_seq < (int64_t)num_sms() * 8 ? n_seq : (int64_t)num_sms() * 8;
+  const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
+  amma50::attn50_bwd_kernel<<<dim3((unsigned)gx, H / amma50::HC_BWD), amma50::HC_BWD * 32, smem, st>>>(
+      qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, scale, seed, offset);
+  NRMS_LAUNCH_CHECK("attn_mma50_bwd");
+  return NRMS_OK;
+}
+
 int attn_mma_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st) {
   const size_t smem = amma::NBUF * (size_t)amma::HC * 3 * amma::TILE * sizeof(float);
   static bool configured[64] = {false};

@@ -42,7 +42,8 @@ static Stash carve_stash(void* base, int64_t rows, bool ln = false) {
   return s;
 }
 
-static bool g_train_attn_mma = true;   // nrms_set_option("train_attn_mma"): tensor-mode title attention on mma.sync tiles
+static bool g_train_attn_mma = true;   // nrms_set_option("train_attn_mma"): tensor-mode news-encoder training attention
+                                       // (titles and 50-token texts) on mma.sync tiles
 constexpr int64_t INFER_CHUNK_ROWS = 2048 * 20;  // rows processed per pass in inference (reference batch 2048 titles)
 constexpr int REDUCE_BLOCKS = 296;
 
@@ -146,11 +147,13 @@ static cudaError_t launch_additive_bwd(const float* d_out, const float* cin, con
   return cudaGetLastError();
 }
 
-// Forward over `n_seq` sequences whose input rows X are already materialised in st.x.
+// Forward over `n_seq` sequences whose input rows X are already materialised in st.x.  text_train: the news encoder's
+// training form -- in tensor mode its 50-token texts take the mma.sync attention; every other S = 50 caller (the user
+// encoder, inference) keeps the CUDA-core kernel.
 static int encoder_core_fwd(const Stash& s, int64_t n_seq, int S, const float* wqkv, const float* bqkv,
                             const float* wa, const float* ba, const float* qa, float* out, float p2,
                             uint64_t seed, uint64_t offset, int64_t row_base, int mode, cudaStream_t st,
-                            const LnArgs* ln = nullptr) {
+                            const LnArgs* ln = nullptr, bool text_train = false) {
   const int64_t rows = n_seq * S;
   int rc = gemm_nt_bias(s.x, D, wqkv, D, bqkv, s.qkv, D3, rows, D3, D, mode, st);
   if (rc) return rc;
@@ -160,6 +163,9 @@ static int encoder_core_fwd(const Stash& s, int64_t n_seq, int S, const float* w
   if (S == 20 && mode == NRMS_MODE_TF32 && g_train_attn_mma) {
     // tensor mode, titles: exp-softmax attention on mma.sync TF32 tiles (attn_mma.cu)
     if (int rc2 = attn_mma_fwd(s.qkv, s.c, n_seq, p2, seed, off2, st)) return rc2;
+    e = cudaSuccess;
+  } else if (S == 50 && text_train && mode == NRMS_MODE_TF32 && g_train_attn_mma) {
+    if (int rc2 = attn_mma50_fwd(s.qkv, s.c, n_seq, p2, seed, off2, st)) return rc2;
     e = cudaSuccess;
   } else if (S == 20) e = launch_attention_fwd<20, 15>(s.qkv, s.c, n_seq, p2, seed, off2, st);
   else e = launch_attention_fwd<50, 5>(s.qkv, s.c, n_seq, p2, seed, off2, st);
@@ -222,11 +228,12 @@ static int additive_block_bwd(const float* d_out, const float* cin, const float*
   return NRMS_OK;
 }
 
-// Backward over the whole stash.  d_x (rows x 300) receives dL/dX.
+// Backward over the whole stash.  d_x (rows x 300) receives dL/dX.  text_train: as in encoder_core_fwd.
 static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, int64_t n_seq, int S,
                             const float* wqkv, const float* wa, const float* qa, float* d_x, float* d_wqkv,
                             float* d_bqkv, float* d_wa, float* d_ba, float* d_qa, float p2, uint64_t seed,
-                            uint64_t offset, int mode, cudaStream_t st, const LnArgs* ln = nullptr) {
+                            uint64_t offset, int mode, cudaStream_t st, const LnArgs* ln = nullptr,
+                            bool text_train = false) {
   // FP32 mode: every contraction on the CUDA cores (reference-exact up to summation order).  Tensor mode: the four
   // GEMMs run on tcgen05 (TF32 operands rounded by the TMA unit, fp32 accumulation) through the K-major NT kernel:
   //   dC  += dU   Wa        = NT(dU   [rows,200], Wa^T   [300,200])
@@ -263,6 +270,10 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
   if (S == 20 && tc && g_train_attn_mma) {
     // the kernel also leaves dQKV^T in t1 (the K-major operand of the dWqkv contraction below)
     if (int rc2 = attn_mma_bwd(s.qkv, w.d_c, w.d_qkv, w.t1, w.ldr, n_seq, p2, seed, offset, st)) return rc2;
+    dqkv_t_written = true;
+    e = cudaSuccess;
+  } else if (S == 50 && text_train && tc && g_train_attn_mma) {
+    if (int rc2 = attn_mma50_bwd(s.qkv, w.d_c, w.d_qkv, w.t1, w.ldr, n_seq, p2, seed, offset, st)) return rc2;
     dqkv_t_written = true;
     e = cudaSuccess;
   } else if (S == 20) e = launch_attention_bwd<20, NRMS_ATTN_BWD_HC20>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
@@ -351,10 +362,6 @@ static int news_encoder_fwd_impl(const int64_t* tokens, int64_t n_titles, int L,
   if (int rc = check_common(L, mode)) return rc;
   NRMS_CHECK_ARG(news_rows == nullptr || stash != nullptr, NRMS_E_UNSUPPORTED,
                  "the index-only form (token table + news rows) is the training form: pass a stash");
-  // training (a stash is requested) is compiled for the title length; inference also takes 50-token texts (the
-  // abstract encoder of the reference's Exp1 model is this same block, src/model/Exp1/news_encoder.py:10-34)
-  NRMS_CHECK_ARG(L == 20 || (L == 50 && stash == nullptr), NRMS_E_UNSUPPORTED,
-                 "news encoder compiled for title length 20 (inference: 20 or 50), got %d", L);
   NRMS_CHECK_ARG(n_titles >= 0 && num_words > 0, NRMS_E_INVALID, "bad sizes");
   if (n_titles == 0) return NRMS_OK;
   NRMS_CHECK_ARG(tokens && emb && wqkv && bqkv && wa && ba && qa && out, NRMS_E_INVALID, "null pointer");
@@ -372,7 +379,7 @@ static int news_encoder_fwd_impl(const int64_t* tokens, int64_t n_titles, int L,
     gather_embedding_kernel<<<(unsigned)gb, 256, 0, st>>>(tokens, rows, emb, s.x, dropout_p, scale, seed, offset,
                                                           news_rows, L);
     NRMS_LAUNCH_CHECK("gather_embedding");
-    return encoder_core_fwd(s, n_titles, L, wqkv, bqkv, wa, ba, qa, out, dropout_p, seed, offset, 0, mode, st, ln);
+    return encoder_core_fwd(s, n_titles, L, wqkv, bqkv, wa, ba, qa, out, dropout_p, seed, offset, 0, mode, st, ln, true);
   }
   // inference
   if (mode == NRMS_MODE_TF32 && dropout_p == 0.f && tc_fused_workspace_bytes(n_titles, L, num_words) != (size_t)-1) {
@@ -441,7 +448,6 @@ static int news_encoder_bwd_impl(const float* d_out, const int64_t* tokens, int6
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (int rc = check_ln(ln, true)) return rc;
   if (int rc = check_common(L, mode)) return rc;
-  NRMS_CHECK_ARG(L == 20, NRMS_E_UNSUPPORTED, "news encoder compiled for title length 20, got %d", L);
   if (n_titles == 0) return NRMS_OK;
   NRMS_CHECK_ARG(n_titles > 0 && num_words > 0, NRMS_E_INVALID, "bad sizes");
   NRMS_CHECK_ARG(d_out && tokens && wqkv && wa && qa && stash && d_emb && d_wqkv && d_bqkv && d_wa && d_ba && d_qa,
@@ -454,7 +460,7 @@ static int news_encoder_bwd_impl(const float* d_out, const int64_t* tokens, int6
   Stash s = carve_stash(const_cast<void*>(stash), rows, ln != nullptr);
   BwdWs w = carve_bwd(workspace, rows, true, mode);
   int rc = encoder_core_bwd(s, w, d_out, n_titles, L, wqkv, wa, qa, w.d_x, d_wqkv, d_bqkv, d_wa, d_ba, d_qa,
-                            dropout_p, seed, offset, mode, st, ln);
+                            dropout_p, seed, offset, mode, st, ln, true);
   if (rc) return rc;
   const float scale = dropout_p > 0.f ? 1.f / (1.f - dropout_p) : 1.f;
   int64_t gb = (rows + 7) / 8;

@@ -38,6 +38,17 @@ class Exp1(torch.nn.Module):
         user_vector = self.user_encoder(vec[:, n_cand:])
         return self.click_predictor(vec[:, :n_cand], user_vector)
 
+    def forward_rows(self, news_table, cand_rows, hist_rows):
+        """Index-only minibatch: news_table {attribute: device column} with N + 1 rows (title [N+1, 20], abstract
+        [N+1, 50], category / subcategory [N+1]; row N is the pad, as NewsTable.token_table_with_pad builds it),
+        cand_rows [B, 1+K] and hist_rows [B, N_clicked] news-row indices -> logits [B, 1+K]."""
+        B, n_cand = cand_rows.shape
+        dev = next(iter(news_table.values())).device
+        rows = torch.cat([cand_rows.to(dev, non_blocking=True), hist_rows.to(dev, non_blocking=True)], dim=1)
+        vec = self.news_encoder.forward_rows(news_table, rows.reshape(-1).long()).view(B, rows.shape[1], -1)
+        user_vector = self.user_encoder(vec[:, n_cand:])
+        return self.click_predictor(vec[:, :n_cand], user_vector)
+
     def get_news_vector(self, news):
         """news: {"title": B x L, "category": B, ...} -> B x word_embedding_dim"""
         return self.news_encoder(news)

@@ -13,8 +13,15 @@ from ..general.attention.multihead_self import MultiHeadSelfAttention
 from ..general.attention.additive import AdditiveAttention
 
 
+# Philox keys of the text encoders' dropout streams.  Both encoders start at offset 0 each step, so with one key element
+# i of a title and element i of an abstract would drop together; the abstract gets its own key (the title keeps the
+# key it always had, so title-only models draw the same masks as before).
+DROPOUT_SEEDS = {"title": 0x5EED, "abstract": 0xAB57AC7}
+
+
 class TextEncoder(nn.Module):
-    def __init__(self, word_embedding, word_embedding_dim, num_attention_heads, query_vector_dim, dropout_probability):
+    def __init__(self, word_embedding, word_embedding_dim, num_attention_heads, query_vector_dim, dropout_probability,
+                 dropout_seed=0x5EED):
         super().__init__()
         self.word_embedding = word_embedding
         self.dropout_probability = dropout_probability
@@ -22,15 +29,17 @@ class TextEncoder(nn.Module):
         self.additive_attention = AdditiveAttention(query_vector_dim, word_embedding_dim)
         self.precision = None
         self._dropout_calls = 0
-        self.dropout_seed = 0x5EED
+        self.dropout_seed = dropout_seed
 
     def _seed(self):
         import torch.distributed as dist
         rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
         return (int(self.dropout_seed) + 0x9E3779B97F4A7C15 * rank) & 0xFFFFFFFFFFFFFFFF
 
-    def forward(self, text):
-        """text: integer [n, num_words_text] (20 = title; 50 = abstract, inference only) -> fp32 [n, 300]."""
+    def forward(self, text, news_rows=None):
+        """text: integer [n, num_words_text] (20 = title, 50 = abstract; training and inference) -> fp32 [n, 300].
+        With news_rows (int64 [m] on the device) `text` is the device-resident token column [N + 1, L] of the news table
+        and the call encodes its rows news_rows, read through the indices inside the gather / scatter kernels."""
         dev = self.word_embedding.weight.device
         if not text.is_cuda and text.numel():
             lo, hi = int(text.min()), int(text.max())
@@ -42,11 +51,12 @@ class TextEncoder(nn.Module):
         offset = 0
         if p > 0.0:
             offset = self._dropout_calls
-            self._dropout_calls += (text.numel() * ops.D) // 4 + 1
+            n_tok = text.numel() if news_rows is None else news_rows.numel() * text.shape[1]
+            self._dropout_calls += (n_tok * ops.D) // 4 + 1
         a = self.additive_attention
         return ops.news_encoder(text, self.word_embedding.weight, wqkv, bqkv, a.linear.weight, a.linear.bias,
                                 a.attention_query_vector, dropout_p=p, seed=self._seed(), offset=offset,
-                                mode=resolve_mode(None, self.precision))
+                                mode=resolve_mode(None, self.precision), news_rows=news_rows)
 
 
 class ElementEncoder(nn.Module):
@@ -84,7 +94,7 @@ class NewsEncoder(nn.Module):
         text_names = sorted(set(config.dataset_attributes['news']) & {'title', 'abstract'})
         self.text_encoders = nn.ModuleDict({
             name: TextEncoder(word_embedding, config.word_embedding_dim, config.num_attention_heads,
-                              config.query_vector_dim, config.dropout_probability)
+                              config.query_vector_dim, config.dropout_probability, DROPOUT_SEEDS[name])
             for name in text_names
         })
         category_embedding = nn.Embedding(config.num_categories, config.category_embedding_dim, padding_idx=0)
@@ -117,6 +127,16 @@ class NewsEncoder(nn.Module):
         -> B x word_embedding_dim"""
         all_vectors = [encoder(news[name]) for name, encoder in self.text_encoders.items()] + \
                       [encoder(news[name]) for name, encoder in self.element_encoders.items()]
+        return self._pool(all_vectors)
+
+    def forward_rows(self, news_table, rows):
+        """news_table: {attribute: device column with N + 1 rows}, rows: int64 [m] on the device -> m x 300.  The text
+        columns are read through the indices inside the gather / scatter kernels; the element ids are gathered first."""
+        all_vectors = [encoder(news_table[name], news_rows=rows) for name, encoder in self.text_encoders.items()] + \
+                      [encoder(news_table[name][rows]) for name, encoder in self.element_encoders.items()]
+        return self._pool(all_vectors)
+
+    def _pool(self, all_vectors):
         if len(all_vectors) == 1:
             return all_vectors[0]
         return self.final_attention(ops.stack_vectors(all_vectors))

@@ -48,11 +48,13 @@ class TrainStep:
         kernels (nrms_news_encoder_rows_fwd/bwd): no gathered token tensor is materialised."""
         if self.cosine_total_steps:
             self.optimizer.param_groups[0]["lr"] = cosine_lr(self.base_lr, self.steps, self.cosine_total_steps)
+        # a model with several news attributes (Exp1) takes a dict of device columns with one row per news
+        n_rows = next(iter(token_table.values())).shape[0] if isinstance(token_table, dict) else token_table.shape[0]
         if not cand_rows.is_cuda and cand_rows.numel():
             lo = min(int(cand_rows.min()), int(hist_rows.min()))
             hi = max(int(cand_rows.max()), int(hist_rows.max()))
-            if lo < 0 or hi >= token_table.shape[0]:
-                raise IndexError(f"news rows must lie in [0, {token_table.shape[0]}), got [{lo}, {hi}]")
+            if lo < 0 or hi >= n_rows:
+                raise IndexError(f"news rows must lie in [0, {n_rows}), got [{lo}, {hi}]")
         logits = self.model.forward_rows(token_table, cand_rows, hist_rows)
         loss = ops.cross_entropy_label0(logits)
         self.optimizer.zero_grad()
@@ -63,6 +65,18 @@ class TrainStep:
         return loss.detach()
 
     def step(self, candidate_news, clicked_news):
-        """Reference minibatch format: lists of {"title": LongTensor[B, L]} (src/train.py:202-203)."""
+        """Reference minibatch format: lists of {"title": LongTensor[B, L]} (src/train.py:202-203), or of every
+        attribute the model reads ({"title", "abstract", "category", ...}) for a model without forward_tokens (Exp1)."""
+        if not hasattr(self.model, "forward_tokens"):
+            if self.cosine_total_steps:
+                self.optimizer.param_groups[0]["lr"] = cosine_lr(self.base_lr, self.steps, self.cosine_total_steps)
+            logits = self.model(candidate_news, clicked_news)
+            loss = ops.cross_entropy_label0(logits)
+            self.optimizer.zero_grad()
+            loss.backward()
+            scale = self.optimizer.allreduce_grads()
+            self.optimizer.step(grad_scale=scale)
+            self.steps += 1
+            return loss.detach()
         titles = torch.stack([x["title"] for x in candidate_news] + [x["title"] for x in clicked_news], dim=1)
         return self.step_tokens(titles, len(candidate_news))
