@@ -17,6 +17,7 @@
  *   nrms_rank_metrics           calculate_single_user_metric + nanmean  src/evaluate.py:24-42,160-168,270-272
  *   nrms_news_encoder_rows_fwd/bwd  NewsEncoder over an index-only minibatch    src/dataset.py:17-85, src/train.py:118-124
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
+ *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
  *   nrms_element_encoder_fwd/bwd, nrms_add_position_fwd/bwd, nrms_additive_fwd/bwd at 2..4 candidates
  *                               model/Exp1                                  src/model/Exp1/news_encoder.py:37-111,
  *                                                                           src/model/Exp1/user_encoder.py:15-31
@@ -167,7 +168,7 @@ int nrms_user_encoder_bwd(const float* d_out, int64_t n_users, int S,
                           void* workspace, size_t workspace_bytes,
                           int mode, void* stream);
 
-/* Standalone L0 blocks (inference only; inside the encoders they are fused):
+/* Standalone L0 blocks (inside the encoders they are fused; both have a backward below):
  *   nrms_mhsa_fwd      MultiHeadSelfAttention.forward(Q) with K=V=Q, length=None   multihead_self.py:46-76
  *                      x [n_seq,S,300] -> ctx [n_seq,S,300]; workspace >= n_seq*S*900*4 bytes
  *   nrms_additive_fwd  AdditiveAttention.forward                                   additive.py:27-53
@@ -181,6 +182,17 @@ int nrms_mhsa_masked_fwd(const float* x, const int32_t* lengths, int64_t n_seq, 
                          const float* bqkv, float* ctx, void* workspace, size_t workspace_bytes, int mode, void* stream);
 int nrms_additive_fwd(const float* c, int64_t n_seq, int S, const float* wa, const float* ba, const float* qa,
                       float* out, void* workspace, size_t workspace_bytes, int mode, void* stream);
+
+/* MultiHeadSelfAttention backward for the standalone block (K=V=Q), with or without the `length` mask.
+ * fwd_workspace = the workspace nrms_mhsa_fwd / nrms_mhsa_masked_fwd filled (QKV [n_seq*S, 900] at its start), lengths
+ * the same int32 [n_seq] the forward took (NULL = no mask).  Masked keys get exactly zero dK / dV; length <= 0 leaves the
+ * whole sequence out.  d_x [n_seq,S,300] is OVERWRITTEN (NULL: not computed); d_wqkv [900,300] and d_bqkv [900] are
+ * accumulated into.  Tensor mode runs the attention on mma.sync TF32 tiles (nrms_set_option("train_attn_mma", 0): the
+ * CUDA-core kernels of FP32 mode) and the weight and input contractions on tcgen05. */
+size_t nrms_mhsa_bwd_workspace_bytes(int64_t n_seq, int S, int mode);
+int nrms_mhsa_bwd(const float* d_ctx, const float* x, const int32_t* lengths, int64_t n_seq, int S, const float* wqkv,
+                  const void* fwd_workspace, float* d_x, float* d_wqkv, float* d_bqkv, void* workspace,
+                  size_t workspace_bytes, int mode, void* stream);
 
 /* AdditiveAttention backward for the standalone block.  nrms_additive_fwd accepts S = 20, 50 and 2..4 (the final attention
  * over the 2..4 element vectors of model/Exp1, src/model/Exp1/news_encoder.py:104-110; that form always runs on the CUDA

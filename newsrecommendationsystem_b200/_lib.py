@@ -48,6 +48,8 @@ SIGNATURES = {
                                         _vp, _vp, _sz, _i32, _vp]),
     "nrms_mhsa_fwd": (_i32, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_mhsa_masked_fwd": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
+    "nrms_mhsa_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "nrms_mhsa_bwd": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_additive_fwd": (_i32, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_additive_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "nrms_additive_bwd": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),

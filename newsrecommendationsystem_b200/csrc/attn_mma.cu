@@ -22,6 +22,11 @@
 //             dK = dS^T Q and dV = attn^T G read dS / attn back TRANSPOSED from shared memory: they are parked in the V
 //             and K tiles, which are dead by then (their padding stays zero: only the 20x20 block is written).
 // Global loads: warp-private 16-byte async copies, no block-wide barrier in the title loop (see warp_fetch).
+//
+// Key mask (the backward's MASKED instantiation, for the standalone block's `length`, multihead_self.py:60-68): the
+// exponentials of key columns >= length are 0 where they are formed, so the row sums, attn, dS and delta see nothing
+// of them, and the dK / dV rows of masked keys come out exactly zero with no special case (dS hi + lo included: both
+// halves are 0).  Query rows past the length are computed like the others.
 #include "common.cuh"
 #include "tc_api.cuh"
 
@@ -36,6 +41,12 @@ constexpr int HC = 5;            // heads per CTA (one warp each)
 constexpr int THREADS = HC * 32;
 constexpr float SQRT_DH = 4.47213595499957939f;
 constexpr float ATTN_EPS = 1e-8f;
+
+// keys of sequence `seq` that the `length` mask keeps: min(max(length, 0), s) (encoder_kernels.cuh, attention_fwd_kernel)
+__device__ __forceinline__ int key_limit(const int32_t* __restrict__ lengths, int64_t seq, int s) {
+  const int l = lengths[seq];
+  return l < 0 ? 0 : (l < s ? l : s);
+}
 constexpr uint32_t DROPOUT_STREAM_CTX = 2;     // encoder_kernels.cuh
 constexpr int NBUF = 1;          // one set of tiles per warp (a second set, filled under the compute, halved the resident warps: slower)
 
@@ -142,14 +153,14 @@ __device__ __forceinline__ void gemm_tn(Frag& c, const float* T, const float* B,
   }
 }
 
-// raw scores -> attention weights in place: exp(s / sqrt 20) for key columns < 20, 0 for the padding columns,
-// divided by (row sum + 1e-8)  (multihead_self.py:16-20: no max subtraction)
+// raw scores -> attention weights in place: exp(s / sqrt 20) for key columns < jmax (20, or the clamped length of the
+// masked backward), 0 for the others, divided by (row sum + 1e-8)  (multihead_self.py:16-20: no max subtraction)
 __device__ __forceinline__ float ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-__device__ __forceinline__ void softmax_rows(Frag& c, int t) {
+__device__ __forceinline__ void softmax_rows(Frag& c, int t, int jmax = S) {
   constexpr float SCALE_LOG2E = 1.4426950408889634f / SQRT_DH;     // exp(s / sqrt 20) = 2^(s * log2(e) / sqrt 20)
 #pragma unroll
   for (int mt = 0; mt < 2; ++mt)
@@ -161,7 +172,7 @@ __device__ __forceinline__ void softmax_rows(Frag& c, int t) {
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
           const int col = nt * 8 + 2 * t + e;
-          const float v = col < S ? ex2(c[mt][nt][half * 2 + e] * SCALE_LOG2E) : 0.f;
+          const float v = col < jmax ? ex2(c[mt][nt][half * 2 + e] * SCALE_LOG2E) : 0.f;
           c[mt][nt][half * 2 + e] = v;
           sum += v;
         }
@@ -334,9 +345,12 @@ attn_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ ctx, int64_t 
   }
 }
 
+// MASKED: keys at positions >= lengths[seq] are left out (see the header); otherwise `lengths` is not read
+template <bool MASKED>
 __global__ void __launch_bounds__(THREADS)
 attn_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, float* __restrict__ d_qkv,
-                float* __restrict__ d_qkv_t, int64_t ldt, int64_t n_seq, float p, float scale, uint64_t seed, uint64_t offset) {
+                float* __restrict__ d_qkv_t, int64_t ldt, int64_t n_seq, float p, float scale, uint64_t seed, uint64_t offset,
+                const int32_t* __restrict__ lengths) {
   extern __shared__ __align__(16) float smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
   const int hc = blockIdx.y;
@@ -362,7 +376,7 @@ attn_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, 
     zero(a);
     gemm_nt(a, Q, K, g, t);
     AT(4);
-    softmax_rows(a, t);                       // a = attn
+    softmax_rows(a, t, MASKED ? key_limit(lengths, seq, S) : S);       // a = attn (masked key columns 0)
     AT(5);
     zero(dp);
     gemm_nt(dp, G, V, g, t);                  // dp = dO V^T
@@ -451,6 +465,8 @@ attn_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, 
 // So the scores and exponentials are computed twice (seven 64 x 56 x 24 contractions instead of five) rather than parking
 // two 50 x 50 matrices per head in shared memory.  Heads per CTA: 3 in the forward (56 KB, 4 CTAs per SM), 1 in the
 // backward (25.6 KB, 8 CTAs per SM); the warps never wait for each other, so a CTA of one warp loses nothing.
+// The backward's MASKED instantiation zeroes the exponentials of masked keys in both passes: key columns in pass 1,
+// key rows of the transposed tile in pass 2 (see the key mask of the title kernels).
 namespace amma50 {
 
 constexpr int S = 50;            // tokens per text
@@ -513,8 +529,9 @@ __device__ __forceinline__ void gemm_frag_n(Out& c, const Row& p, const float* B
 constexpr float SCALE_LOG2E = 1.4426950408889634f / amma::SQRT_DH;     // exp(s / sqrt 20) = 2^(s * log2(e) / sqrt 20)
 constexpr float INV_SQRT_DH = 1.f / amma::SQRT_DH;
 
-// raw scores -> attention weights in place (key columns >= 50 -> 0); inv[half] = 1 / (row sum + 1e-8) of row g + 8 half
-__device__ __forceinline__ void softmax_rows(Row& c, int t, float (&inv)[2]) {
+// raw scores -> attention weights in place (key columns >= jmax -> 0; jmax = 50 or the clamped length);
+// inv[half] = 1 / (row sum + 1e-8) of row g + 8 half
+__device__ __forceinline__ void softmax_rows(Row& c, int t, float (&inv)[2], int jmax = S) {
 #pragma unroll
   for (int half = 0; half < 2; ++half) {
     float sum = 0.f;
@@ -523,7 +540,7 @@ __device__ __forceinline__ void softmax_rows(Row& c, int t, float (&inv)[2]) {
 #pragma unroll
       for (int e = 0; e < 2; ++e) {
         const int col = nt * 8 + 2 * t + e;
-        const float v = col < S ? amma::ex2(c[nt][half * 2 + e] * SCALE_LOG2E) : 0.f;
+        const float v = col < jmax ? amma::ex2(c[nt][half * 2 + e] * SCALE_LOG2E) : 0.f;
         c[nt][half * 2 + e] = v;
         sum += v;
       }
@@ -646,10 +663,11 @@ attn50_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ ctx, int64_
   }
 }
 
+template <bool MASKED>
 __global__ void __launch_bounds__(HC_BWD * 32)
 attn50_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, float* __restrict__ d_qkv,
                   float* __restrict__ d_qkv_t, int64_t ldt, int64_t n_seq, float p, float scale, uint64_t seed,
-                  uint64_t offset) {
+                  uint64_t offset, const int32_t* __restrict__ lengths) {
   extern __shared__ __align__(16) float smem[];
   constexpr int PER_WARP = 4 * TILE + 2 * ZS;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
@@ -667,6 +685,7 @@ attn50_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx
     fetch<4>(Q, qkv + seq * S * D3 + colbase, d_ctx + seq * S * D + colbase, lane, seq * S, colbase, p, scale, seed, offset);
     float* out = d_qkv + seq * S * D3 + colbase;
     float* out_t = d_qkv_t ? d_qkv_t + (int64_t)colbase * ldt + seq * S : nullptr;     // [900, ldt]: row = column of dQKV
+    const int jmax = MASKED ? amma::key_limit(lengths, seq, S) : S;
     // ---- pass 1: query tiles -> dQ, row vectors ----
 #pragma unroll 1
     for (int mt = 0; mt < MT; ++mt) {
@@ -674,7 +693,7 @@ attn50_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx
       zero(a);
       gemm_nt(a, Q, mt * 16, K, g, t);
       float inv[2];
-      softmax_rows(a, t, inv);                // a = attn
+      softmax_rows(a, t, inv, jmax);          // a = attn
       zero(dp);
       gemm_nt(dp, G, mt * 16, V, g, t);       // dp = dO V^T
 #pragma unroll
@@ -719,7 +738,8 @@ attn50_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx
           const float z = col < S ? zinv[col] : 0.f, dl = col < S ? delta[col] : 0.f;
 #pragma unroll
           for (int half = 0; half < 2; ++half) {
-            const float at = col < S ? amma::ex2(a[nt][half * 2 + e] * SCALE_LOG2E) * z : 0.f;
+            const bool keep = col < S && (!MASKED || kt * 16 + g + 8 * half < jmax);        // query column, key row
+            const float at = keep ? amma::ex2(a[nt][half * 2 + e] * SCALE_LOG2E) * z : 0.f;
             a[nt][half * 2 + e] = at;                                                     // attn^T
             dp[nt][half * 2 + e] = at * (dp[nt][half * 2 + e] - dl) * INV_SQRT_DH;        // dS^T
           }
@@ -751,17 +771,26 @@ int attn_mma50_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_
   return NRMS_OK;
 }
 
-int attn_mma50_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
-                   uint64_t seed, uint64_t offset, cudaStream_t st) {
+template <bool MASKED>
+static int attn_mma50_bwd_launch(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt,
+                                 int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st,
+                                 const int32_t* lengths) {
   const size_t smem = (size_t)amma50::HC_BWD * (4 * amma50::TILE + 2 * amma50::ZS) * sizeof(float);
   static bool configured[64] = {false};
-  if (cudaError_t e = set_max_dynamic_smem(amma50::attn50_bwd_kernel, (int)smem, configured)) return cuda_fail(e, "attn_mma50_bwd attr");
+  if (cudaError_t e = set_max_dynamic_smem(amma50::attn50_bwd_kernel<MASKED>, (int)smem, configured))
+    return cuda_fail(e, "attn_mma50_bwd attr");
   int64_t gx = n_seq < (int64_t)num_sms() * 8 ? n_seq : (int64_t)num_sms() * 8;
   const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
-  amma50::attn50_bwd_kernel<<<dim3((unsigned)gx, H / amma50::HC_BWD), amma50::HC_BWD * 32, smem, st>>>(
-      qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, scale, seed, offset);
+  amma50::attn50_bwd_kernel<MASKED><<<dim3((unsigned)gx, H / amma50::HC_BWD), amma50::HC_BWD * 32, smem, st>>>(
+      qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, scale, seed, offset, lengths);
   NRMS_LAUNCH_CHECK("attn_mma50_bwd");
   return NRMS_OK;
+}
+
+int attn_mma50_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
+                   uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths) {
+  return lengths ? attn_mma50_bwd_launch<true>(qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, seed, offset, st, lengths)
+                 : attn_mma50_bwd_launch<false>(qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, seed, offset, st, nullptr);
 }
 
 int attn_mma_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st) {
@@ -775,17 +804,25 @@ int attn_mma_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t 
   return NRMS_OK;
 }
 
-int attn_mma_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
-                 uint64_t seed, uint64_t offset, cudaStream_t st) {
+template <bool MASKED>
+static int attn_mma_bwd_launch(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq,
+                               float p, uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths) {
   const size_t smem = amma::NBUF * (size_t)amma::HC * 4 * amma::TILE * sizeof(float);
   static bool configured[64] = {false};
-  if (cudaError_t e = set_max_dynamic_smem(amma::attn_bwd_kernel, (int)smem, configured)) return cuda_fail(e, "attn_mma_bwd attr");
+  if (cudaError_t e = set_max_dynamic_smem(amma::attn_bwd_kernel<MASKED>, (int)smem, configured))
+    return cuda_fail(e, "attn_mma_bwd attr");
   int64_t gx = n_seq < (int64_t)num_sms() * 8 ? n_seq : (int64_t)num_sms() * 8;
   const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
-  amma::attn_bwd_kernel<<<dim3((unsigned)gx, H / amma::HC), amma::THREADS, smem, st>>>(qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, scale,
-                                                                                       seed, offset);
+  amma::attn_bwd_kernel<MASKED><<<dim3((unsigned)gx, H / amma::HC), amma::THREADS, smem, st>>>(
+      qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, scale, seed, offset, lengths);
   NRMS_LAUNCH_CHECK("attn_mma_bwd");
   return NRMS_OK;
+}
+
+int attn_mma_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
+                 uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths) {
+  return lengths ? attn_mma_bwd_launch<true>(qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, seed, offset, st, lengths)
+                 : attn_mma_bwd_launch<false>(qkv, d_ctx, d_qkv, d_qkv_t, ldt, n_seq, p, seed, offset, st, nullptr);
 }
 
 }  // namespace nrms

@@ -94,17 +94,17 @@ static cudaError_t launch_attention_fwd(const float* qkv, float* ctx, int64_t n_
   return cudaGetLastError();
 }
 
-template <int S, int HC>
+template <int S, int HC, bool MASKED = false>
 static cudaError_t launch_attention_bwd(const float* qkv, const float* d_ctx, float* d_qkv, int64_t n_seq, float p,
-                                        uint64_t seed, uint64_t offset, cudaStream_t st) {
+                                        uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths = nullptr) {
   constexpr int threads = ((S * HC + 31) / 32) * 32;
   const size_t smem = (4 * S * HC * DH + 2 * HC * S * (S + 1)) * sizeof(float);
   static bool configured[64] = {false};
-  if (cudaError_t e = set_max_dynamic_smem(attention_bwd_kernel<S, HC>, (int)smem, configured)) return e;
+  if (cudaError_t e = set_max_dynamic_smem(attention_bwd_kernel<S, HC, MASKED>, (int)smem, configured)) return e;
   int64_t gx = n_seq < (int64_t)num_sms() * 4 ? n_seq : (int64_t)num_sms() * 4;
   dim3 grid((unsigned)gx, H / HC);
   const float scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
-  attention_bwd_kernel<S, HC><<<grid, threads, smem, st>>>(qkv, d_ctx, d_qkv, n_seq, p, scale, seed, offset);
+  attention_bwd_kernel<S, HC, MASKED><<<grid, threads, smem, st>>>(qkv, d_ctx, d_qkv, n_seq, p, scale, seed, offset, lengths);
   count_launch();
   return cudaGetLastError();
 }
@@ -228,6 +228,46 @@ static int additive_block_bwd(const float* d_out, const float* cin, const float*
   return NRMS_OK;
 }
 
+// Backward of the q|k|v projection QKV = X Wqkv^T + bqkv from dQKV [rows,900], shared by the encoders and the
+// standalone self-attention block: d_bqkv += colsum(dQKV), d_wqkv += dQKV^T X, d_x = dQKV Wqkv (skipped when d_x is
+// null).  Tensor mode takes the transposed operands from t1 / t2 / wt (t1 = dQKV^T already when dqkv_t_written).
+struct QkvBwdWs {
+  float *d_qkv, *partial, *t1, *t2, *wt;
+  int64_t ldr;
+};
+static int qkv_proj_bwd(const QkvBwdWs& w, const float* x, const float* wqkv, int64_t rows, float* d_x, float* d_wqkv,
+                        float* d_bqkv, bool tc, bool dqkv_t_written, cudaStream_t st) {
+  int cb = (int)(rows < REDUCE_BLOCKS ? rows : REDUCE_BLOCKS);
+  int splits = (int)((rows + 4095) / 4096);
+  if (splits > 64) splits = 64;
+  // d_bqkv = colsum(dQKV)
+  colsum_partial_kernel<<<cb, 256, 0, st>>>(w.d_qkv, rows, D3, w.partial);
+  NRMS_LAUNCH_CHECK("colsum_dqkv");
+  launch_partial_reduce_accum(w.partial, cb, D3, D3, d_bqkv, st);
+  NRMS_LAUNCH_CHECK("dbqkv_reduce");
+  if (tc) {
+    // d_wqkv[900,300] += dQKV^T X
+    if (!dqkv_t_written)
+      if (int rc = transpose_f32(w.d_qkv, D3, w.t1, w.ldr, rows, D3, st)) return rc;
+    if (int rc = transpose_f32(x, D, w.t2, w.ldr, rows, D, st)) return rc;
+    if (int rc = tc_gemm_nt_ex(w.t1, w.ldr, w.t2, w.ldr, nullptr, d_wqkv, D, D3, D, (int)rows,
+                               tc_gemm_auto_splits(D3, D, (int)rows), TC_EPI_ATOMIC, st)) return rc;
+    if (!d_x) return NRMS_OK;
+    // d_x = dQKV * Wqkv
+    if (int rc = transpose_f32(wqkv, D, w.wt, D3, D3, D, st)) return rc;
+    if (int rc = tc_gemm_nt_ex(w.d_qkv, D3, w.wt, D3, nullptr, d_x, D, rows, D, D3, 1, TC_EPI_STORE, st)) return rc;
+  } else {
+    // d_wqkv[900,300] += dQKV^T X
+    cudaError_t e = sgemm_launch<1, 1, EPI_ATOMIC>(w.d_qkv, D3, x, D, nullptr, d_wqkv, D, D3, D, rows, splits, st);
+    if (e != cudaSuccess) return cuda_fail(e, "sgemm dWqkv");
+    if (!d_x) return NRMS_OK;
+    // d_x = dQKV * Wqkv   ([rows,900] x [900,300])
+    e = sgemm_launch<0, 1, EPI_STORE>(w.d_qkv, D3, wqkv, D, nullptr, d_x, D, rows, D, D3, 1, st);
+    if (e != cudaSuccess) return cuda_fail(e, "sgemm dX");
+  }
+  return NRMS_OK;
+}
+
 // Backward over the whole stash.  d_x (rows x 300) receives dL/dX.  text_train: as in encoder_core_fwd.
 static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, int64_t n_seq, int S,
                             const float* wqkv, const float* wa, const float* qa, float* d_x, float* d_wqkv,
@@ -249,9 +289,6 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
     const AddBwdWs aw{w.d_u, w.partial, w.t1, w.t2, w.wt, w.ldr};
     if (int rc = additive_block_bwd(d_out, cin, s.t, s.w, wa, qa, w.d_c, aw, n_seq, S, d_wa, d_ba, d_qa, tc, st)) return rc;
   }
-  int cb = (int)(rows < REDUCE_BLOCKS ? rows : REDUCE_BLOCKS);
-  int splits = (int)((rows + 4095) / 4096);
-  if (splits > 64) splits = 64;
   cudaError_t e;
   if (ln) {   // d_c holds dL/dCN: through the LayerNorm, in place; d_gamma / d_beta via per-block partial sums
     int lb = (int)((rows + 7) / 8 < REDUCE_BLOCKS ? (rows + 7) / 8 : REDUCE_BLOCKS);
@@ -279,30 +316,8 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
   } else if (S == 20) e = launch_attention_bwd<20, NRMS_ATTN_BWD_HC20>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
   else e = launch_attention_bwd<50, 5>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
   if (e != cudaSuccess) return cuda_fail(e, "attention_bwd");
-  // d_bqkv = colsum(dQKV)
-  colsum_partial_kernel<<<cb, 256, 0, st>>>(w.d_qkv, rows, D3, w.partial);
-  NRMS_LAUNCH_CHECK("colsum_dqkv");
-  launch_partial_reduce_accum(w.partial, cb, D3, D3, d_bqkv, st);
-  NRMS_LAUNCH_CHECK("dbqkv_reduce");
-  if (tc) {
-    // d_wqkv[900,300] += dQKV^T X
-    if (!dqkv_t_written)
-      if (int rc = transpose_f32(w.d_qkv, D3, w.t1, w.ldr, rows, D3, st)) return rc;
-    if (int rc = transpose_f32(s.x, D, w.t2, w.ldr, rows, D, st)) return rc;
-    if (int rc = tc_gemm_nt_ex(w.t1, w.ldr, w.t2, w.ldr, nullptr, d_wqkv, D, D3, D, (int)rows,
-                               tc_gemm_auto_splits(D3, D, (int)rows), TC_EPI_ATOMIC, st)) return rc;
-    // d_x = dQKV * Wqkv
-    if (int rc = transpose_f32(wqkv, D, w.wt, D3, D3, D, st)) return rc;
-    if (int rc = tc_gemm_nt_ex(w.d_qkv, D3, w.wt, D3, nullptr, d_x, D, rows, D, D3, 1, TC_EPI_STORE, st)) return rc;
-  } else {
-    // d_wqkv[900,300] += dQKV^T X
-    e = sgemm_launch<1, 1, EPI_ATOMIC>(w.d_qkv, D3, s.x, D, nullptr, d_wqkv, D, D3, D, rows, splits, st);
-    if (e != cudaSuccess) return cuda_fail(e, "sgemm dWqkv");
-    // d_x = dQKV * Wqkv   ([rows,900] x [900,300])
-    e = sgemm_launch<0, 1, EPI_STORE>(w.d_qkv, D3, wqkv, D, nullptr, d_x, D, rows, D, D3, 1, st);
-    if (e != cudaSuccess) return cuda_fail(e, "sgemm dX");
-  }
-  return NRMS_OK;
+  const QkvBwdWs qw{w.d_qkv, w.partial, w.t1, w.t2, w.wt, w.ldr};
+  return qkv_proj_bwd(qw, s.x, wqkv, rows, d_x, d_wqkv, d_bqkv, tc, dqkv_t_written, st);
 }
 
 static int check_common(int S, int mode) {
@@ -638,7 +653,7 @@ int nrms_user_encoder_ln_bwd(const float* d_out, int64_t n_users, int S, const f
                                workspace_bytes, mode, stream, &ln);
 }
 
-// ---- standalone L0 blocks (inference): MultiHeadSelfAttention.forward / AdditiveAttention.forward ----
+// ---- standalone L0 blocks: MultiHeadSelfAttention.forward / AdditiveAttention.forward and their backwards ----
 static int mhsa_fwd_impl(const float* x, const int32_t* lengths, int64_t n_seq, int S, const float* wqkv,
                          const float* bqkv, float* ctx, void* workspace, size_t workspace_bytes, int mode, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -669,6 +684,74 @@ int nrms_mhsa_masked_fwd(const float* x, const int32_t* lengths, int64_t n_seq, 
                          const float* bqkv, float* ctx, void* workspace, size_t workspace_bytes, int mode, void* stream) {
   NRMS_CHECK_ARG(lengths != nullptr || n_seq == 0, NRMS_E_INVALID, "null lengths");
   return mhsa_fwd_impl(x, lengths, n_seq, S, wqkv, bqkv, ctx, workspace, workspace_bytes, mode, stream);
+}
+
+// workspace of nrms_mhsa_bwd: dQKV [rows,900] | partial sums [296,900]; tensor mode adds t1 [900,ldr] (dQKV^T) |
+// t2 [300,ldr] (X^T) | wt [300,900] (Wqkv^T), ldr = rows rounded up to 4
+static QkvBwdWs carve_mhsa_bwd(void* base, int64_t rows, int mode, size_t* bytes) {
+  QkvBwdWs w{};
+  char* p = reinterpret_cast<char*>(base);
+  size_t off = 0;
+  auto take = [&](size_t nfloat) {
+    float* r = reinterpret_cast<float*>(p + off);
+    off += align_up(nfloat * sizeof(float), 256);
+    return r;
+  };
+  w.d_qkv = take((size_t)rows * D3);
+  w.partial = take((size_t)REDUCE_BLOCKS * D3);
+  w.ldr = (rows + 3) / 4 * 4;
+  if (mode == NRMS_MODE_TF32) {
+    w.t1 = take((size_t)w.ldr * D3);
+    w.t2 = take((size_t)w.ldr * D);
+    w.wt = take((size_t)D3 * D);
+  }
+  *bytes = off;
+  return w;
+}
+
+size_t nrms_mhsa_bwd_workspace_bytes(int64_t n_seq, int S, int mode) {
+  if (n_seq <= 0 || S <= 0) return 0;
+  size_t bytes = 0;
+  carve_mhsa_bwd(nullptr, n_seq * S, mode, &bytes);
+  return bytes;
+}
+
+int nrms_mhsa_bwd(const float* d_ctx, const float* x, const int32_t* lengths, int64_t n_seq, int S, const float* wqkv,
+                  const void* fwd_workspace, float* d_x, float* d_wqkv, float* d_bqkv, void* workspace,
+                  size_t workspace_bytes, int mode, void* stream) {
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (int rc = check_common(S, mode)) return rc;
+  NRMS_CHECK_ARG(n_seq >= 0, NRMS_E_INVALID, "bad sizes");
+  if (n_seq == 0) return NRMS_OK;
+  NRMS_CHECK_ARG(d_ctx && x && wqkv && fwd_workspace && d_wqkv && d_bqkv, NRMS_E_INVALID, "null pointer");
+  NRMS_CHECK_ARG(aligned16(d_ctx) && aligned16(x) && aligned16(wqkv) && aligned16(fwd_workspace) && aligned16(d_wqkv) &&
+                     (!d_x || aligned16(d_x)) && (reinterpret_cast<uintptr_t>(lengths) & 3) == 0,
+                 NRMS_E_INVALID, "pointers must be 16-byte aligned (lengths: 4-byte)");
+  const int64_t rows = n_seq * S;
+  size_t need = 0;
+  QkvBwdWs w = carve_mhsa_bwd(workspace, rows, mode, &need);
+  NRMS_CHECK_ARG(workspace && aligned16(workspace) && workspace_bytes >= need, NRMS_E_WORKSPACE,
+                 "workspace too small: need %zu bytes", need);
+  const bool tc = (mode == NRMS_MODE_TF32);
+  const float* qkv = reinterpret_cast<const float*>(fwd_workspace);     // what nrms_mhsa_(masked_)fwd left there
+  bool dqkv_t_written = false;
+  if (tc && g_train_attn_mma) {
+    // mma.sync tiles, as the encoders' training attention; the kernel also leaves dQKV^T in t1
+    const int rc = S == 20 ? attn_mma_bwd(qkv, d_ctx, w.d_qkv, w.t1, w.ldr, n_seq, 0.f, 0, 0, st, lengths)
+                           : attn_mma50_bwd(qkv, d_ctx, w.d_qkv, w.t1, w.ldr, n_seq, 0.f, 0, 0, st, lengths);
+    if (rc) return rc;
+    dqkv_t_written = true;
+  } else {
+    cudaError_t e;
+    if (S == 20)
+      e = lengths ? launch_attention_bwd<20, NRMS_ATTN_BWD_HC20, true>(qkv, d_ctx, w.d_qkv, n_seq, 0.f, 0, 0, st, lengths)
+                  : launch_attention_bwd<20, NRMS_ATTN_BWD_HC20>(qkv, d_ctx, w.d_qkv, n_seq, 0.f, 0, 0, st);
+    else
+      e = lengths ? launch_attention_bwd<50, 5, true>(qkv, d_ctx, w.d_qkv, n_seq, 0.f, 0, 0, st, lengths)
+                  : launch_attention_bwd<50, 5>(qkv, d_ctx, w.d_qkv, n_seq, 0.f, 0, 0, st);
+    if (e != cudaSuccess) return cuda_fail(e, "attention_bwd");
+  }
+  return qkv_proj_bwd(w, x, wqkv, rows, d_x, d_wqkv, d_bqkv, tc, dqkv_t_written, st);
 }
 
 int nrms_additive_fwd(const float* c, int64_t n_seq, int S, const float* wa, const float* ba, const float* qa,

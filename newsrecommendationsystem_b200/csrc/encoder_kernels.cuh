@@ -177,11 +177,14 @@ attention_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ ctx, int
 //   attn = e/(Z+eps)  =>  ds_ij = attn_ij (dattn_ij - sum_k attn_ik dattn_ik) / sqrt(d)
 // P/DS rows have a pitch of S+1 words: phase 1 (threads = consecutive i, same j) and phase 2 (threads = consecutive j)
 // are both bank-conflict free.
+// MASKED (the standalone block's `length`): phase 1 runs over the keys j < jmax of the forward kernel and writes attn = 0
+// and ds = 0 for the others, so phase 2 gives exactly zero dK / dV rows for masked keys.  Unmasked, `lengths` is unread.
 // ----------------------------------------------------------------------------------------
-template <int S, int HC>
+template <int S, int HC, bool MASKED = false>
 __global__ void __launch_bounds__(((S * HC + 31) / 32) * 32)
 attention_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx, float* __restrict__ d_qkv,
-                     int64_t n_seq, float p, float scale, uint64_t seed, uint64_t offset) {
+                     int64_t n_seq, float p, float scale, uint64_t seed, uint64_t offset,
+                     const int32_t* __restrict__ lengths = nullptr) {
   constexpr int W = HC * DH;
   constexpr int W4 = W / 4;
   constexpr int SP = S + 1;
@@ -229,8 +232,10 @@ attention_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_
 #pragma unroll
       for (int d = 0; d < DH; ++d) { a[d] = Qs[i * W + hl * DH + d]; b[d] = Gs[i * W + hl * DH + d]; r[d] = 0.f; }
       float Z = 0.f, num = 0.f;
+      int jmax = S;
+      if (MASKED) { const int l = lengths[seq]; jmax = l < 0 ? 0 : (l < S ? l : S); }
 #pragma unroll 4
-      for (int j = 0; j < S; ++j) {
+      for (int j = 0; j < jmax; ++j) {
         const float4* kp = reinterpret_cast<const float4*>(Ks + j * W + hl * DH);
         const float4* vp = reinterpret_cast<const float4*>(Vs + j * W + hl * DH);
         float sp[DH / 4], dp[DH / 4];      // five independent 4-term chains per dot product, in the forward's order
@@ -251,7 +256,7 @@ attention_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_
       const float zinv = 1.f / (Z + ATTN_EPS);
       const float delta = num * zinv;
 #pragma unroll 4
-      for (int j = 0; j < S; ++j) {
+      for (int j = 0; j < jmax; ++j) {
         const float4* kp = reinterpret_cast<const float4*>(Ks + j * W + hl * DH);
         const float at = prow[j] * zinv;
         const float ds = at * (drow[j] - delta) * INV_SQRT_DH;
@@ -264,6 +269,8 @@ attention_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ d_
           r[4 * c + 2] = fmaf(ds, k.z, r[4 * c + 2]); r[4 * c + 3] = fmaf(ds, k.w, r[4 * c + 3]);
         }
       }
+      if (MASKED)
+        for (int j = jmax; j < S; ++j) prow[j] = drow[j] = 0.f;
       float4* op = reinterpret_cast<float4*>(d_qkv + (seq * S + i) * D3 + hc * W + hl * DH);
 #pragma unroll
       for (int c = 0; c < DH / 4; ++c) op[c] = make_float4(r[4 * c], r[4 * c + 1], r[4 * c + 2], r[4 * c + 3]);

@@ -43,12 +43,13 @@ int tc_gemm_nt_f16(const void* A16, int64_t lda, const void* B16, int64_t ldb, v
 // recomputes the probabilities from the stashed q|k|v rows); qkv [n_seq*20, 900], ctx / d_ctx [n_seq*20, 300]
 int attn_mma_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st);
 // d_qkv_t (nullable): the same gradients also written transposed, [900, ldt] (the dWqkv contraction's K-major operand)
+// lengths (nullable, int32 [n_seq]): the key mask of the standalone block -- keys at positions >= lengths[seq] are left out
 int attn_mma_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
-                 uint64_t seed, uint64_t offset, cudaStream_t st);
+                 uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths = nullptr);
 // the same two passes over 50-token texts (abstracts): qkv [n_seq*50, 900], ctx / d_ctx [n_seq*50, 300]
 int attn_mma50_fwd(const float* qkv, float* ctx, int64_t n_seq, float p, uint64_t seed, uint64_t offset, cudaStream_t st);
 int attn_mma50_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_qkv_t, int64_t ldt, int64_t n_seq, float p,
-                   uint64_t seed, uint64_t offset, cudaStream_t st);
+                   uint64_t seed, uint64_t offset, cudaStream_t st, const int32_t* lengths = nullptr);
 // K1f (k1f_attn_pool.cu): table attention + additive pooling in one kernel (the context rows stay on the SM)
 int k1f_qk_bound(const void* table16, int64_t n_rows, float* bound, cudaStream_t st);
 int k1f_run(int S, int idx_kind, const void* table16, int64_t n_table_rows, const void* rows, int64_t n_seq,

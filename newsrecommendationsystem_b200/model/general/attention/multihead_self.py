@@ -1,9 +1,10 @@
-"""MultiHeadSelfAttention parameter container + standalone forward.
+"""MultiHeadSelfAttention parameter container + standalone forward and backward.
 
 Mirror of reference src/model/general/attention/multihead_self.py:26-76: three nn.Linear
 (W_Q, W_K, W_V; xavier_uniform weights, :41-44), no output projection.  Inside NewsEncoder /
 UserEncoder the projections, the exp-softmax attention and the pooling run inside
 libnrms_b200; this class owns the parameters so state_dict keys match the reference.
+Called on its own it trains too, with or without the `length` mask (nrms_mhsa_bwd).
 """
 import torch
 import torch.nn as nn
@@ -46,17 +47,16 @@ class MultiHeadSelfAttention(nn.Module):
         return cache[1], cache[2]
 
     def forward(self, Q, K=None, V=None, length=None):
-        """Standalone use (inference).  Inside NewsEncoder / UserEncoder this block is fused into the encoder
-        kernels; NRMS never passes K, V or length (src/model/NRMS/news_encoder.py:41, user_encoder.py:23).  The
-        `length` mask branch (reference :60-68: keys at positions >= length[b] are multiplied out of the exp-softmax)
-        is compiled for the self-attention form; cross-attention (K or V different from Q) fails loudly."""
+        """Standalone use, in grad mode or not.  Inside NewsEncoder / UserEncoder this block is fused into the
+        encoder kernels; NRMS never passes K, V or length (src/model/NRMS/news_encoder.py:41, user_encoder.py:23).
+        The `length` mask branch (reference :60-68: keys at positions >= length[b] are multiplied out of the
+        exp-softmax; `length` is a host or device integer tensor, one entry per sequence, and gets no gradient) is
+        compiled for the self-attention form; cross-attention (K or V different from Q) fails loudly.  Gradients
+        reach Q and the six parameters through torch.cat in packed()."""
         if (K is not None and K is not Q) or (V is not None and V is not Q):
             raise NotImplementedError("libnrms_b200 compiles MultiHeadSelfAttention for K = V = Q (self-attention)")
-        if torch.is_grad_enabled() and (Q.requires_grad or self.W_Q.weight.requires_grad):
-            raise NotImplementedError("standalone MultiHeadSelfAttention.forward is inference-only; training goes "
-                                      "through NewsEncoder / UserEncoder (use torch.no_grad() here)")
         from .... import ops
         from ....config import resolve_mode
         wqkv, bqkv = self.packed()
-        return ops.mhsa_forward(Q.to(self.W_Q.weight.device), wqkv, bqkv,
-                                mode=resolve_mode(None, getattr(self, "precision", None)), length=length)
+        return ops.mhsa(Q.to(self.W_Q.weight.device), wqkv, bqkv,
+                        mode=resolve_mode(None, getattr(self, "precision", None)), length=length)

@@ -441,9 +441,8 @@ def gemm_nt(a, b, bias=None, mode=_lib.MODE_TF32):
     return c
 
 
-@torch.no_grad()
-def mhsa_forward(x, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
-    """Standalone MultiHeadSelfAttention.forward(Q, length=length) (K=V=Q), inference only."""
+def _mhsa_fwd(x, wqkv, bqkv, mode, length):
+    """nrms_mhsa_fwd / nrms_mhsa_masked_fwd -> (ctx, x_c, w_c, len_c, ws); ws holds q|k|v [n*S, 900] afterwards."""
     lib = _lib.load()
     _require_cuda(x, wqkv, bqkv)
     n, S, d = x.shape
@@ -458,10 +457,52 @@ def mhsa_forward(x, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
         len_c = length.to(device=x.device, dtype=torch.int32).contiguous().view(-1)
         check(lib.nrms_mhsa_masked_fwd(ptr(x_c), ptr(len_c), n, S, ptr(w_c), ptr(b_c), ptr(ctx), ptr(ws), ws.numel(),
                                        mode, stream_ptr(x.device)), "nrms_mhsa_masked_fwd")
-        return ctx
+        return ctx, x_c, w_c, len_c, ws
     check(lib.nrms_mhsa_fwd(ptr(x_c), n, S, ptr(w_c), ptr(b_c), ptr(ctx), ptr(ws), ws.numel(), mode,
                             stream_ptr(x.device)), "nrms_mhsa_fwd")
-    return ctx
+    return ctx, x_c, w_c, None, ws
+
+
+@torch.no_grad()
+def mhsa_forward(x, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
+    """Standalone MultiHeadSelfAttention.forward(Q, length=length) (K=V=Q) without autograd."""
+    return _mhsa_fwd(x, wqkv, bqkv, mode, length)[0]
+
+
+class _MHSAFn(torch.autograd.Function):
+    """Standalone MultiHeadSelfAttention.forward(Q, length=length) (reference multihead_self.py:15-23,46-76, K=V=Q) with
+    its backward.  The forward is nrms_mhsa_(masked_)fwd, so grad and no-grad forwards give the same bits; its
+    workspace (q|k|v) is what the backward reads."""
+
+    @staticmethod
+    def forward(ctx, x, wqkv, bqkv, mode, length, track_grad):
+        out, x_c, w_c, len_c, ws = _mhsa_fwd(x, wqkv, bqkv, mode, length)
+        if track_grad and any(ctx.needs_input_grad):
+            ctx.save_for_backward(x_c, w_c, len_c, ws)
+            ctx.meta = (mode,)
+        return out
+
+    @staticmethod
+    def backward(ctx, d_ctx):
+        lib = _lib.load()
+        x, wqkv, lengths, fws = ctx.saved_tensors
+        (mode,) = ctx.meta
+        n, S, _ = x.shape
+        dev = d_ctx.device
+        d_ctx = d_ctx.contiguous().float()
+        d_x = torch.empty_like(x) if ctx.needs_input_grad[0] else None
+        d_w = torch.zeros((3 * D, D), dtype=torch.float32, device=dev)
+        d_b = torch.zeros((3 * D,), dtype=torch.float32, device=dev)
+        ws = _bytes(lib.nrms_mhsa_bwd_workspace_bytes(n, S, mode), dev)
+        check(lib.nrms_mhsa_bwd(ptr(d_ctx), ptr(x), ptr(lengths), n, S, ptr(wqkv), ptr(fws), ptr(d_x), ptr(d_w), ptr(d_b),
+                                ptr(ws), ws.numel(), mode, stream_ptr(dev)), "nrms_mhsa_bwd")
+        return (d_x, d_w if ctx.needs_input_grad[1] else None, d_b if ctx.needs_input_grad[2] else None,
+                None, None, None)
+
+
+def mhsa(x, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
+    """MultiHeadSelfAttention.forward(Q, length=length), autograd-connected (forward and backward in libnrms_b200)."""
+    return _MHSAFn.apply(x, wqkv, bqkv, mode, length, torch.is_grad_enabled())
 
 
 class _AdditiveFn(torch.autograd.Function):
