@@ -18,6 +18,7 @@
  *   nrms_news_encoder_rows_fwd/bwd  NewsEncoder over an index-only minibatch    src/dataset.py:17-85, src/train.py:118-124
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
  *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
+ *   nrms_mha_fwd/bwd            MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries / keys  (same lines)
  *   nrms_element_encoder_fwd/bwd, nrms_add_position_fwd/bwd, nrms_additive_fwd/bwd at 2..4 candidates
  *                               model/Exp1                                  src/model/Exp1/news_encoder.py:37-111,
  *                                                                           src/model/Exp1/user_encoder.py:15-31
@@ -193,6 +194,31 @@ size_t nrms_mhsa_bwd_workspace_bytes(int64_t n_seq, int S, int mode);
 int nrms_mhsa_bwd(const float* d_ctx, const float* x, const int32_t* lengths, int64_t n_seq, int S, const float* wqkv,
                   const void* fwd_workspace, float* d_x, float* d_wqkv, float* d_bqkv, void* workspace,
                   size_t workspace_bytes, int mode, void* stream);
+
+/* MultiHeadSelfAttention.forward(Q, K, V, length) at any 1 <= Sq, Sk <= 64: cross-attention (K and / or V other inputs
+ * than Q) and self-attention at lengths other than 20 and 50.  xq [n_seq,Sq,300], xk and xv [n_seq,Sk,300]; pass the
+ * same pointer for the same input (K = Q, K = V, ...): each input is projected onto the rows of wqkv it needs, once
+ * when its roles' rows are adjacent (Q = V with K another input takes two 300-row projections).  Distinct inputs must
+ * be distinct pointers: two pointers that are equal are one input.  ctx [n_seq,Sq,300].  lengths (int32 [n_seq], NULL = no mask) is the reference's `length`: with Sq == Sk the
+ * keys j < length[b] are kept; with Sq == 1 < Sk the reference's [B,H,1,1] mask broadcasts, so all keys are kept iff
+ * length[b] >= 1; any other Sq != Sk with lengths -> NRMS_E_UNSUPPORTED.  length <= 0 gives a zero context.
+ * Tensor mode: projections on tcgen05, attention on mma.sync TF32 tiles; FP32 mode: CUDA cores throughout.
+ * The forward workspace keeps the projections; it is what nrms_mha_bwd reads (the same inputs, shapes and lengths).
+ * Backward: d_xq / d_xk / d_xv are OVERWRITTEN (NULL: not computed).  When two inputs are the same pointer their gradient
+ * pointers must be equal or NULL, and that buffer receives the sum; gradients of distinct inputs must be distinct
+ * buffers, and none may be an input (NRMS_E_INVALID).  d_wqkv [900,300] and d_bqkv [900] are accumulated into.
+ * Masked keys get exactly zero dK / dV rows.  Arguments are checked before any CUDA call: Sq or Sk outside 1..64 ->
+ * NRMS_E_UNSUPPORTED, null or misaligned pointers (the workspace included) -> NRMS_E_INVALID, a null or short
+ * workspace -> NRMS_E_WORKSPACE. */
+size_t nrms_mha_fwd_workspace_bytes(int64_t n_seq, int Sq, int Sk);
+int nrms_mha_fwd(const float* xq, const float* xk, const float* xv, int64_t n_seq, int Sq, int Sk, const int32_t* lengths,
+                 const float* wqkv, const float* bqkv, float* ctx, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream);
+size_t nrms_mha_bwd_workspace_bytes(int64_t n_seq, int Sq, int Sk, int mode);
+int nrms_mha_bwd(const float* d_ctx, const float* xq, const float* xk, const float* xv, int64_t n_seq, int Sq, int Sk,
+                 const int32_t* lengths, const float* wqkv, const void* fwd_workspace, float* d_xq, float* d_xk,
+                 float* d_xv, float* d_wqkv, float* d_bqkv, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream);
 
 /* AdditiveAttention backward for the standalone block.  nrms_additive_fwd accepts S = 20, 50 and 2..4 (the final attention
  * over the 2..4 element vectors of model/Exp1, src/model/Exp1/news_encoder.py:104-110; that form always runs on the CUDA

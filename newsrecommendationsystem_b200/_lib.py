@@ -50,6 +50,11 @@ SIGNATURES = {
     "nrms_mhsa_masked_fwd": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_mhsa_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "nrms_mhsa_bwd": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
+    "nrms_mha_fwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "nrms_mha_fwd": (_i32, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
+    "nrms_mha_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32]),
+    "nrms_mha_bwd": (_i32, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32,
+                            _vp]),
     "nrms_additive_fwd": (_i32, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "nrms_additive_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "nrms_additive_bwd": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),

@@ -229,40 +229,46 @@ static int additive_block_bwd(const float* d_out, const float* cin, const float*
 }
 
 // Backward of the q|k|v projection QKV = X Wqkv^T + bqkv from dQKV [rows,900], shared by the encoders and the
-// standalone self-attention block: d_bqkv += colsum(dQKV), d_wqkv += dQKV^T X, d_x = dQKV Wqkv (skipped when d_x is
+// standalone attention block: d_bqkv += colsum(dQKV), d_wqkv += dQKV^T X, d_x = dQKV Wqkv (skipped when d_x is
 // null).  Tensor mode takes the transposed operands from t1 / t2 / wt (t1 = dQKV^T already when dqkv_t_written).
+// ncols < 900: the projection onto a contiguous slice of rows of Wqkv (wqkv, d_wqkv and d_bqkv point at the slice, dQKV
+// is [rows, ncols]) -- the standalone block projects each input onto the rows it needs (nrms_mha_bwd).  accum_dx: d_x +=
+// instead of d_x = (the second projection of an input the block projects twice).
 struct QkvBwdWs {
   float *d_qkv, *partial, *t1, *t2, *wt;
   int64_t ldr;
 };
 static int qkv_proj_bwd(const QkvBwdWs& w, const float* x, const float* wqkv, int64_t rows, float* d_x, float* d_wqkv,
-                        float* d_bqkv, bool tc, bool dqkv_t_written, cudaStream_t st) {
+                        float* d_bqkv, bool tc, bool dqkv_t_written, cudaStream_t st, int ncols = D3,
+                        bool accum_dx = false) {
   int cb = (int)(rows < REDUCE_BLOCKS ? rows : REDUCE_BLOCKS);
   int splits = (int)((rows + 4095) / 4096);
   if (splits > 64) splits = 64;
   // d_bqkv = colsum(dQKV)
-  colsum_partial_kernel<<<cb, 256, 0, st>>>(w.d_qkv, rows, D3, w.partial);
+  colsum_partial_kernel<<<cb, 256, 0, st>>>(w.d_qkv, rows, ncols, w.partial);
   NRMS_LAUNCH_CHECK("colsum_dqkv");
-  launch_partial_reduce_accum(w.partial, cb, D3, D3, d_bqkv, st);
+  launch_partial_reduce_accum(w.partial, cb, ncols, ncols, d_bqkv, st);
   NRMS_LAUNCH_CHECK("dbqkv_reduce");
   if (tc) {
     // d_wqkv[900,300] += dQKV^T X
     if (!dqkv_t_written)
-      if (int rc = transpose_f32(w.d_qkv, D3, w.t1, w.ldr, rows, D3, st)) return rc;
+      if (int rc = transpose_f32(w.d_qkv, ncols, w.t1, w.ldr, rows, ncols, st)) return rc;
     if (int rc = transpose_f32(x, D, w.t2, w.ldr, rows, D, st)) return rc;
-    if (int rc = tc_gemm_nt_ex(w.t1, w.ldr, w.t2, w.ldr, nullptr, d_wqkv, D, D3, D, (int)rows,
-                               tc_gemm_auto_splits(D3, D, (int)rows), TC_EPI_ATOMIC, st)) return rc;
+    if (int rc = tc_gemm_nt_ex(w.t1, w.ldr, w.t2, w.ldr, nullptr, d_wqkv, D, ncols, D, (int)rows,
+                               tc_gemm_auto_splits(ncols, D, (int)rows), TC_EPI_ATOMIC, st)) return rc;
     if (!d_x) return NRMS_OK;
     // d_x = dQKV * Wqkv
-    if (int rc = transpose_f32(wqkv, D, w.wt, D3, D3, D, st)) return rc;
-    if (int rc = tc_gemm_nt_ex(w.d_qkv, D3, w.wt, D3, nullptr, d_x, D, rows, D, D3, 1, TC_EPI_STORE, st)) return rc;
+    if (int rc = transpose_f32(wqkv, D, w.wt, ncols, ncols, D, st)) return rc;
+    if (int rc = tc_gemm_nt_ex(w.d_qkv, ncols, w.wt, ncols, nullptr, d_x, D, rows, D, ncols, 1,
+                               accum_dx ? TC_EPI_ACCUM : TC_EPI_STORE, st)) return rc;
   } else {
     // d_wqkv[900,300] += dQKV^T X
-    cudaError_t e = sgemm_launch<1, 1, EPI_ATOMIC>(w.d_qkv, D3, x, D, nullptr, d_wqkv, D, D3, D, rows, splits, st);
+    cudaError_t e = sgemm_launch<1, 1, EPI_ATOMIC>(w.d_qkv, ncols, x, D, nullptr, d_wqkv, D, ncols, D, rows, splits, st);
     if (e != cudaSuccess) return cuda_fail(e, "sgemm dWqkv");
     if (!d_x) return NRMS_OK;
     // d_x = dQKV * Wqkv   ([rows,900] x [900,300])
-    e = sgemm_launch<0, 1, EPI_STORE>(w.d_qkv, D3, wqkv, D, nullptr, d_x, D, rows, D, D3, 1, st);
+    e = accum_dx ? sgemm_launch<0, 1, EPI_ACCUM>(w.d_qkv, ncols, wqkv, D, nullptr, d_x, D, rows, D, ncols, 1, st)
+                 : sgemm_launch<0, 1, EPI_STORE>(w.d_qkv, ncols, wqkv, D, nullptr, d_x, D, rows, D, ncols, 1, st);
     if (e != cudaSuccess) return cuda_fail(e, "sgemm dX");
   }
   return NRMS_OK;
@@ -752,6 +758,190 @@ int nrms_mhsa_bwd(const float* d_ctx, const float* x, const int32_t* lengths, in
     if (e != cudaSuccess) return cuda_fail(e, "attention_bwd");
   }
   return qkv_proj_bwd(w, x, wqkv, rows, d_x, d_wqkv, d_bqkv, tc, dqkv_t_written, st);
+}
+
+// ---- MultiHeadSelfAttention.forward(Q, K, V, length) at 1 <= Sq, Sk <= 64 (nrms_mha_*) ----
+// Each input is projected onto the contiguous rows of Wqkv it needs, into its own buffer; an input passed in two roles
+// whose weight rows are adjacent is projected once:
+//   Q's input -> A [n*Sq, 300 c]: c = 3 when it is also K's and V's (self-attention, one 900-column GEMM), 2 when it is
+//                also K's (q|k), else 1
+//   K's input, when not Q's -> Bk [n*Sk, 600] (k|v) when it is also V's, else [n*Sk, 300]
+//   V's input, when not K's -> Bv [n*Sk, 300] (when it is Q's but K's is another input, W_Q and W_V are not adjacent in
+//                Wqkv: Q's input gets a second 300-column projection here, and its gradient is the sum of both)
+// The forward workspace holds A | Bk | Bv at their largest (900, 300 and 300 columns; a [n*Sk, 600] Bk runs on into Bv's
+// slot), and the backward's dA | dBk | dBv have the same layout, so the attention backward writes dq / dk / dv with the
+// pitches of q / k / v and every projection backward reads one contiguous [rows, 300 c] matrix.
+struct MhaPlan {
+  int n_proj;                // projections (one per input, two for Q's input when it is V's but not K's)
+  const float* x[3];
+  int64_t rows[3];
+  int c0[3], nc[3];          // rows [300 c0, 300 (c0 + nc)) of Wqkv
+  float* buf[3];             // projection (or its gradient), [rows, 300 nc]
+  MhaOperands op;
+  size_t bytes;
+};
+static MhaPlan mha_plan(const float* xq, const float* xk, const float* xv, int64_t n_seq, int sq, int sk, void* base) {
+  MhaPlan p{};
+  char* b = reinterpret_cast<char*>(base);
+  const size_t a_bytes = align_up((size_t)n_seq * sq * D3 * sizeof(float), 256);
+  const size_t k_bytes = align_up((size_t)n_seq * sk * D * sizeof(float), 256);
+  float* A = reinterpret_cast<float*>(b);
+  float* Bk = reinterpret_cast<float*>(b + a_bytes);
+  float* Bv = reinterpret_cast<float*>(b + a_bytes + k_bytes);
+  p.bytes = a_bytes + 2 * k_bytes;
+  const bool qk = xq == xk, qv = xq == xv, kv = xk == xv;
+  auto add = [&](const float* x, int64_t rows, int c0, int nc, float* buf) {
+    const int i = p.n_proj++;
+    p.x[i] = x; p.rows[i] = rows; p.c0[i] = c0; p.nc[i] = nc; p.buf[i] = buf;
+  };
+  const int na = (qk && qv) ? 3 : (qk ? 2 : 1);
+  add(xq, n_seq * sq, 0, na, A);
+  p.op.q = A; p.op.ldq = (int64_t)D * na;
+  if (qk) {
+    p.op.k = A + D; p.op.ldk = p.op.ldq;
+  } else {
+    add(xk, n_seq * sk, 1, kv ? 2 : 1, Bk);
+    p.op.k = Bk; p.op.ldk = kv ? 2 * D : D;
+  }
+  if (qk && qv) {
+    p.op.v = A + 2 * D; p.op.ldv = p.op.ldq;
+  } else if (kv) {
+    p.op.v = Bk + D; p.op.ldv = 2 * D;
+  } else {
+    add(xv, n_seq * sk, 2, 1, Bv);
+    p.op.v = Bv; p.op.ldv = D;
+  }
+  return p;
+}
+
+// the checks both directions share, in order: mode, shapes, sizes (n_seq == 0 -> done), null / misaligned pointers,
+// inputs passed twice with different row counts
+static int mha_check(const float* xq, const float* xk, const float* xv, int64_t n_seq, int sq, int sk,
+                     const int32_t* lengths, const float* wqkv, int mode, bool* done) {
+  *done = false;
+  NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
+  NRMS_CHECK_ARG(sq >= 1 && sq <= 64 && sk >= 1 && sk <= 64, NRMS_E_UNSUPPORTED,
+                 "query / key counts %d / %d unsupported (compiled: 1..64)", sq, sk);
+  NRMS_CHECK_ARG(lengths == nullptr || sq == sk || sq == 1, NRMS_E_UNSUPPORTED,
+                 "a length mask needs as many queries as keys, or one query (%d queries, %d keys)", sq, sk);
+  NRMS_CHECK_ARG(n_seq >= 0, NRMS_E_INVALID, "bad sizes");
+  if (n_seq == 0) {
+    *done = true;
+    return NRMS_OK;
+  }
+  NRMS_CHECK_ARG(xq && xk && xv && wqkv, NRMS_E_INVALID, "null pointer");
+  NRMS_CHECK_ARG(aligned16(xq) && aligned16(xk) && aligned16(xv) && aligned16(wqkv) &&
+                     (reinterpret_cast<uintptr_t>(lengths) & 3) == 0,
+                 NRMS_E_INVALID, "pointers must be 16-byte aligned (lengths: 4-byte)");
+  NRMS_CHECK_ARG((xq != xk && xq != xv) || sq == sk, NRMS_E_INVALID,
+                 "the query input is also the key or value input: Sq (%d) must equal Sk (%d)", sq, sk);
+  return NRMS_OK;
+}
+
+size_t nrms_mha_fwd_workspace_bytes(int64_t n_seq, int Sq, int Sk) {
+  if (n_seq <= 0 || Sq <= 0 || Sk <= 0) return 0;
+  return mha_plan(nullptr, nullptr, nullptr, n_seq, Sq, Sk, nullptr).bytes;
+}
+
+int nrms_mha_fwd(const float* xq, const float* xk, const float* xv, int64_t n_seq, int Sq, int Sk, const int32_t* lengths,
+                 const float* wqkv, const float* bqkv, float* ctx, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream) {
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  bool done;
+  if (int rc = mha_check(xq, xk, xv, n_seq, Sq, Sk, lengths, wqkv, mode, &done)) return rc;
+  if (done) return NRMS_OK;
+  NRMS_CHECK_ARG(bqkv && ctx, NRMS_E_INVALID, "null pointer");
+  NRMS_CHECK_ARG(aligned16(bqkv) && aligned16(ctx), NRMS_E_INVALID, "pointers must be 16-byte aligned");
+  NRMS_CHECK_ARG(ctx != xq && ctx != xk && ctx != xv, NRMS_E_INVALID, "ctx must not alias an input");
+  NRMS_CHECK_ARG(aligned16(workspace), NRMS_E_INVALID, "workspace must be 16-byte aligned");
+  const MhaPlan p = mha_plan(xq, xk, xv, n_seq, Sq, Sk, workspace);
+  NRMS_CHECK_ARG(workspace && workspace_bytes >= p.bytes, NRMS_E_WORKSPACE,
+                 "workspace too small: need %zu bytes", p.bytes);
+  for (int i = 0; i < p.n_proj; ++i) {
+    const int64_t w0 = (int64_t)p.c0[i] * D;
+    if (int rc = gemm_nt_bias(p.x[i], D, wqkv + w0 * D, D, bqkv + w0, p.buf[i], (int64_t)D * p.nc[i], p.rows[i], D * p.nc[i],
+                              D, mode, st)) return rc;
+  }
+  return mha_attn_fwd(p.op, ctx, n_seq, Sq, Sk, lengths, mode, st);
+}
+
+// workspace of nrms_mha_bwd: dA | dBk | dBv (mha_plan) | partial sums [296,900]; tensor mode adds t1 [900,ldr] |
+// t2 [300,ldr] | wt [300,900], ldr = n_seq * max(Sq, Sk) rounded up to 4 (shared by the inputs, one after the other)
+static size_t carve_mha_bwd(void* base, int64_t n_seq, int sq, int sk, int mode, QkvBwdWs* w) {
+  const MhaPlan dp = mha_plan(nullptr, nullptr, nullptr, n_seq, sq, sk, nullptr);
+  char* p = reinterpret_cast<char*>(base);
+  size_t off = dp.bytes;
+  auto take = [&](size_t nfloat) {
+    float* r = reinterpret_cast<float*>(p + off);
+    off += align_up(nfloat * sizeof(float), 256);
+    return r;
+  };
+  QkvBwdWs ws{};
+  ws.partial = take((size_t)REDUCE_BLOCKS * D3);
+  ws.ldr = (n_seq * (sq > sk ? sq : sk) + 3) / 4 * 4;
+  if (mode == NRMS_MODE_TF32) {
+    ws.t1 = take((size_t)ws.ldr * D3);
+    ws.t2 = take((size_t)ws.ldr * D);
+    ws.wt = take((size_t)D3 * D);
+  }
+  if (w) *w = ws;
+  return off;
+}
+
+size_t nrms_mha_bwd_workspace_bytes(int64_t n_seq, int Sq, int Sk, int mode) {
+  if (n_seq <= 0 || Sq <= 0 || Sk <= 0) return 0;
+  return carve_mha_bwd(nullptr, n_seq, Sq, Sk, mode, nullptr);
+}
+
+int nrms_mha_bwd(const float* d_ctx, const float* xq, const float* xk, const float* xv, int64_t n_seq, int Sq, int Sk,
+                 const int32_t* lengths, const float* wqkv, const void* fwd_workspace, float* d_xq, float* d_xk,
+                 float* d_xv, float* d_wqkv, float* d_bqkv, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream) {
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  bool done;
+  if (int rc = mha_check(xq, xk, xv, n_seq, Sq, Sk, lengths, wqkv, mode, &done)) return rc;
+  if (done) return NRMS_OK;
+  NRMS_CHECK_ARG(d_ctx && fwd_workspace && d_wqkv && d_bqkv, NRMS_E_INVALID, "null pointer");
+  NRMS_CHECK_ARG(aligned16(d_ctx) && aligned16(fwd_workspace) && aligned16(d_wqkv) && aligned16(d_bqkv) &&
+                     (!d_xq || aligned16(d_xq)) && (!d_xk || aligned16(d_xk)) && (!d_xv || aligned16(d_xv)) &&
+                     aligned16(workspace),
+                 NRMS_E_INVALID, "pointers must be 16-byte aligned");
+  // aliasing: an input passed twice has one gradient buffer (or NULL for the alias), which receives the sum; gradients
+  // of distinct inputs are distinct buffers, and no gradient buffer is an input
+  const float* xs[3] = {xq, xk, xv};
+  float* ds[3] = {d_xq, d_xk, d_xv};
+  for (int a = 0; a < 3; ++a) {
+    for (int b = a + 1; b < 3; ++b) {
+      if (xs[a] == xs[b])
+        NRMS_CHECK_ARG(!ds[a] || !ds[b] || ds[a] == ds[b], NRMS_E_INVALID,
+                       "an input passed twice takes one gradient buffer (the other NULL or the same)");
+      else
+        NRMS_CHECK_ARG(!ds[a] || !ds[b] || ds[a] != ds[b], NRMS_E_INVALID, "distinct inputs need distinct gradient buffers");
+    }
+    NRMS_CHECK_ARG(!ds[a] || (ds[a] != xq && ds[a] != xk && ds[a] != xv && ds[a] != d_ctx), NRMS_E_INVALID,
+                   "a gradient buffer must not alias an input");
+  }
+  QkvBwdWs w;
+  const size_t need = carve_mha_bwd(workspace, n_seq, Sq, Sk, mode, &w);
+  NRMS_CHECK_ARG(workspace && workspace_bytes >= need, NRMS_E_WORKSPACE, "workspace too small: need %zu bytes", need);
+  const MhaPlan p = mha_plan(xq, xk, xv, n_seq, Sq, Sk, const_cast<void*>(fwd_workspace));   // the forward's projections
+  const MhaPlan dp = mha_plan(xq, xk, xv, n_seq, Sq, Sk, workspace);                          // their gradients
+  if (int rc = mha_attn_bwd(p.op, d_ctx, const_cast<float*>(dp.op.q), const_cast<float*>(dp.op.k), const_cast<float*>(dp.op.v),
+                            n_seq, Sq, Sk, lengths, mode, st)) return rc;
+  const bool tc = (mode == NRMS_MODE_TF32);
+  for (int i = 0; i < p.n_proj; ++i) {
+    float* dx = nullptr;          // the one gradient buffer of this input, if any of its roles has one
+    for (int r = 2; r >= 0; --r)
+      if (xs[r] == p.x[i] && ds[r]) dx = ds[r];
+    bool accum = false;           // a second projection of the same input adds to the first one's dX
+    for (int j = 0; j < i; ++j) accum = accum || p.x[j] == p.x[i];
+    const int64_t w0 = (int64_t)p.c0[i] * D;
+    QkvBwdWs wi = w;
+    wi.d_qkv = dp.buf[i];
+    if (int rc = qkv_proj_bwd(wi, p.x[i], wqkv + w0 * D, p.rows[i], dx, d_wqkv + w0 * D, d_bqkv + w0, tc, false, st,
+                              D * p.nc[i], accum)) return rc;
+  }
+  return NRMS_OK;
 }
 
 int nrms_additive_fwd(const float* c, int64_t n_seq, int S, const float* wa, const float* ba, const float* qa,

@@ -4,7 +4,8 @@ Mirror of reference src/model/general/attention/multihead_self.py:26-76: three n
 (W_Q, W_K, W_V; xavier_uniform weights, :41-44), no output projection.  Inside NewsEncoder /
 UserEncoder the projections, the exp-softmax attention and the pooling run inside
 libnrms_b200; this class owns the parameters so state_dict keys match the reference.
-Called on its own it trains too, with or without the `length` mask (nrms_mhsa_bwd).
+Called on its own it trains too, with or without the `length` mask: self-attention at 20 and 50 tokens through
+nrms_mhsa_*, and cross-attention or any other 1..64 queries and keys through nrms_mha_*.
 """
 import torch
 import torch.nn as nn
@@ -49,14 +50,28 @@ class MultiHeadSelfAttention(nn.Module):
     def forward(self, Q, K=None, V=None, length=None):
         """Standalone use, in grad mode or not.  Inside NewsEncoder / UserEncoder this block is fused into the
         encoder kernels; NRMS never passes K, V or length (src/model/NRMS/news_encoder.py:41, user_encoder.py:23).
+        K = None means K = Q and V = None means V = Q, as in the reference.
+          - Self-attention (K and V None or `is Q`) at 20 or 50 tokens: nrms_mhsa_* (ops.mhsa).
+          - Everything else with 1..64 queries Sq and 1..64 keys Sk, K and V of the same length: nrms_mha_* (ops.mha),
+            cross-attention included.  An input used in two roles (`K is V`, ...) is projected once.
+          - Other shapes raise NotImplementedError.
         The `length` mask branch (reference :60-68: keys at positions >= length[b] are multiplied out of the
         exp-softmax; `length` is a host or device integer tensor, one entry per sequence, and gets no gradient) is
-        compiled for the self-attention form; cross-attention (K or V different from Q) fails loudly.  Gradients
-        reach Q and the six parameters through torch.cat in packed()."""
-        if (K is not None and K is not Q) or (V is not None and V is not Q):
-            raise NotImplementedError("libnrms_b200 compiles MultiHeadSelfAttention for K = V = Q (self-attention)")
+        built from Q's length, so it exists where the reference's broadcast defines it: Sk == Sq (the key mask), or
+        Sq == 1 (all keys kept iff length >= 1); any other Sq != Sk with a length raises NotImplementedError.
+        Gradients reach Q, K, V and the six parameters (through torch.cat in packed())."""
         from .... import ops
         from ....config import resolve_mode
+        K = Q if K is None else K
+        V = Q if V is None else V
+        mode = resolve_mode(None, getattr(self, "precision", None))
+        if K is Q and V is Q and Q.dim() == 3 and Q.shape[1] in (20, 50):
+            wqkv, bqkv = self.packed()
+            return ops.mhsa(Q.to(self.W_Q.weight.device), wqkv, bqkv, mode=mode, length=length)
+        ops.mha_check(Q, K, V, length)
+        dev = self.W_Q.weight.device
+        Qd = Q.to(dev)                                   # each distinct input moved once: aliases stay aliases
+        Kd = Qd if K is Q else K.to(dev)
+        Vd = Qd if V is Q else (Kd if V is K else V.to(dev))
         wqkv, bqkv = self.packed()
-        return ops.mhsa(Q.to(self.W_Q.weight.device), wqkv, bqkv,
-                        mode=resolve_mode(None, getattr(self, "precision", None)), length=length)
+        return ops.mha(Qd, Kd, Vd, wqkv, bqkv, mode=mode, length=length)

@@ -505,6 +505,112 @@ def mhsa(x, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
     return _MHSAFn.apply(x, wqkv, bqkv, mode, length, torch.is_grad_enabled())
 
 
+MHA_MAX_LEN = 64
+
+
+def mha_check(q, k, v, length):
+    """The shapes nrms_mha_* take (reference multihead_self.py:15-23,46-76); NotImplementedError names what is not
+    compiled or not defined by the reference."""
+    if q.dim() != 3 or k.dim() != 3 or v.dim() != 3 or not (q.shape[2] == k.shape[2] == v.shape[2] == D):
+        raise RuntimeError(f"compiled for [B, S, {D}] inputs, got {tuple(q.shape)}, {tuple(k.shape)}, {tuple(v.shape)}")
+    if not (q.shape[0] == k.shape[0] == v.shape[0]):
+        raise RuntimeError(f"Q, K and V need the same batch, got {q.shape[0]}, {k.shape[0]}, {v.shape[0]}")
+    sq, sk = q.shape[1], k.shape[1]
+    if v.shape[1] != sk:
+        raise NotImplementedError(f"K and V must have the same number of rows (attn @ V), got {sk} and {v.shape[1]}")
+    if not (1 <= sq <= MHA_MAX_LEN and 1 <= sk <= MHA_MAX_LEN):
+        raise NotImplementedError(f"libnrms_b200 compiles 1..{MHA_MAX_LEN} queries and keys, got {sq} and {sk}")
+    if length is not None and sq != sk and sq != 1:
+        raise NotImplementedError(f"the reference's length mask [B, {sq}] does not broadcast over {sk} keys")
+
+
+def _mha_operands(q, k, v):
+    """The fp32 contiguous operands of Q, K and V: one converted copy per distinct tensor object, made before any
+    .float().contiguous(), and every role of one object gets that copy.  The library treats equal pointers as one
+    input (projected once, one summed gradient), so a distinct tensor whose copy shares storage with an earlier one's
+    (a view such as Q.detach() or h[:, :5] of a batch of one) gets its own clone; the roles are assigned only after
+    that, so no role keeps a pointer another object's copy was replaced from."""
+    copies = []                                   # (tensor object, its operand)
+    out = []
+    for t in (q, k, v):
+        for o, c in copies:
+            if t is o:
+                out.append(c)
+                break
+        else:
+            c = _f32c(t)
+            if any(c.data_ptr() == u.data_ptr() for _, u in copies):
+                c = c.clone()
+            copies.append((t, c))
+            out.append(c)
+    return out
+
+
+class _MHAFn(torch.autograd.Function):
+    """MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries and keys (reference multihead_self.py:15-23,
+    46-76) with its backward: nrms_mha_fwd / nrms_mha_bwd.  An input passed in two roles (`k is q`, `v is k`, ...)
+    reaches the library as one pointer, so it is projected once; its gradient (the sum over its roles) comes back
+    once, and None for the alias.  Grad and no-grad forwards run the same call, so they give the same bits."""
+
+    @staticmethod
+    def forward(ctx, q, k, v, wqkv, bqkv, mode, length, track_grad):
+        lib = _lib.load()
+        n, sq, _ = q.shape
+        sk = k.shape[1]
+        q_c, k_c, v_c = _mha_operands(q, k, v)
+        w_c, b_c = _f32c(wqkv), _f32c(bqkv)
+        len_c = None
+        if length is not None:
+            if length.numel() != n:
+                raise RuntimeError(f"length must hold one entry per sequence ({n}), got {tuple(length.shape)}")
+            len_c = length.to(device=q.device, dtype=torch.int32).contiguous().view(-1)
+        out = torch.empty((n, sq, D), dtype=torch.float32, device=q.device)
+        ws = _bytes(lib.nrms_mha_fwd_workspace_bytes(n, sq, sk), q.device)
+        check(lib.nrms_mha_fwd(ptr(q_c), ptr(k_c), ptr(v_c), n, sq, sk, ptr(len_c), ptr(w_c), ptr(b_c), ptr(out), ptr(ws),
+                               ws.numel(), mode, stream_ptr(q.device)), "nrms_mha_fwd")
+        if track_grad and any(ctx.needs_input_grad):
+            ctx.save_for_backward(q_c, k_c, v_c, w_c, len_c, ws)
+            ctx.meta = (mode, k is q, v is q, v is k)
+        return out
+
+    @staticmethod
+    def backward(ctx, d_ctx):
+        lib = _lib.load()
+        q, k, v, wqkv, lengths, fws = ctx.saved_tensors
+        mode, kq, vq, vk = ctx.meta
+        need = ctx.needs_input_grad
+        n, sq, _ = q.shape
+        sk = k.shape[1]
+        dev = d_ctx.device
+        d_ctx = d_ctx.contiguous().float()
+        need_q = need[0] or (kq and need[1]) or (vq and need[2])
+        need_k = not kq and (need[1] or (vk and need[2]))
+        need_v = not vq and not vk and need[2]
+        d_q = torch.empty_like(q) if need_q else None
+        d_k = torch.empty_like(k) if need_k else None
+        d_v = torch.empty_like(v) if need_v else None
+        d_xk = d_q if kq else d_k
+        d_xv = d_q if vq else (d_xk if vk else d_v)
+        d_w = torch.zeros((3 * D, D), dtype=torch.float32, device=dev)
+        d_b = torch.zeros((3 * D,), dtype=torch.float32, device=dev)
+        ws = _bytes(lib.nrms_mha_bwd_workspace_bytes(n, sq, sk, mode), dev)
+        check(lib.nrms_mha_bwd(ptr(d_ctx), ptr(q), ptr(k), ptr(v), n, sq, sk, ptr(lengths), ptr(wqkv), ptr(fws), ptr(d_q),
+                               ptr(d_xk), ptr(d_xv), ptr(d_w), ptr(d_b), ptr(ws), ws.numel(), mode, stream_ptr(dev)),
+              "nrms_mha_bwd")
+        return (d_q, d_k, d_v, d_w if need[3] else None, d_b if need[4] else None, None, None, None)
+
+
+def mha(q, k, v, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
+    """MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries and keys, autograd-connected (forward and
+    backward in libnrms_b200).  K = None means K = Q and V = None means V = Q, as in the reference; pass the same tensor
+    object for an input used in two roles so that it is projected once."""
+    k = q if k is None else k
+    v = q if v is None else v
+    mha_check(q, k, v, length)
+    _require_cuda(q, k, v, wqkv, bqkv)
+    return _MHAFn.apply(q, k, v, wqkv, bqkv, mode, length, torch.is_grad_enabled())
+
+
 class _AdditiveFn(torch.autograd.Function):
     """AdditiveAttention.forward (reference src/model/general/attention/additive.py:27-53) with its backward, for
     candidate sizes 20 / 50 and 2..4 (the final attention of model/Exp1)."""
