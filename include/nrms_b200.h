@@ -19,7 +19,8 @@
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
  *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
  *   nrms_mha_fwd/bwd            MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries / keys  (same lines)
- *   nrms_element_encoder_fwd/bwd, nrms_add_position_fwd/bwd, nrms_additive_fwd/bwd at 2..4 candidates
+ *   nrms_additive_fwd/bwd       AdditiveAttention.forward at 1..64 candidates  src/model/general/attention/additive.py:27-53
+ *   nrms_element_encoder_fwd/bwd, nrms_add_position_fwd/bwd
  *                               model/Exp1                                  src/model/Exp1/news_encoder.py:37-111,
  *                                                                           src/model/Exp1/user_encoder.py:15-31
  *
@@ -31,7 +32,8 @@
  *   - Return value: 0 = ok, nonzero = error (NRMS_E_*); text via nrms_last_error()
  *     (thread-local).  No exception crosses the ABI.  There is no CPU fallback.
  *   - Model dimensions are compile-time: D=300, H=15 (d_k=d_v=20), query dim 200
- *     (src/config.py:14-45); sequence length S is 20 (titles) or 50 (click history).
+ *     (src/config.py:14-45).  Text length L is 20 (titles) or 50 (abstracts); the user encoder's history length S
+ *     (config.num_clicked_news_a_user) is any 1..64, with fused kernels at 20 and 50.
  *   - Packed weights: wqkv = rows [W_Q; W_K; W_V] -> [900,300] (nn.Linear "out,in" layout),
  *     bqkv [900], wa [200,300], ba [200], qa [200].
  */
@@ -81,7 +83,8 @@ int64_t nrms_launch_count(void);
  *  2^(s - max) / (Z + 1e-8 * 2^-max) from a bound on the scores, 0 / 1 force one form (tests).
  * "train_attn_mma" (default 1): tensor-mode training attention of the news encoder, over titles (L = 20) and 50-token
  *  texts (L = 50), on mma.sync TF32 tiles (attn_mma.cu); 0 = the CUDA-core kernels of the FP32 mode.  The user
- *  encoder's S = 50 training attention stays on the CUDA-core kernel either way.
+ *  encoder's S = 50 training attention stays on the CUDA-core kernel either way; its other history lengths (not 20)
+ *  run the attention of nrms_mha_* in the call's mode.
  * "k1f_debug": component-removal timing masks of K1f (garbage results; profiles/k1f_probe.py). */
 int nrms_set_option(const char* key, int value);
 /* "time_k1" = 1 brackets every fused K1 launch with CUDA events on the launching stream (clears the previous
@@ -141,7 +144,11 @@ int nrms_news_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_t
 
 /* User encoder forward.  Input rows are either dense x [n_users, S, 300] (rows == NULL, n_rows ignored) or
  * gathered from a table: x = table [n_rows,300], rows int32 [n_users, S] with values in [0, n_rows)
- * (evaluate.py:220-224; the PADDED_NEWS zero vector is a zero row of the table). */
+ * (evaluate.py:220-224; the PADDED_NEWS zero vector is a zero row of the table).
+ * S = 1..64 for every user-encoder entry point (forward, backward, LayerNorm and fp16-table forms); S outside that range
+ * returns NRMS_E_UNSUPPORTED before any CUDA call.  S = 20 and 50 run the compiled kernels (in tensor-mode inference the
+ * fused K1 / K2 paths); other lengths run the projection GEMM, the run-time-length attention of nrms_mha_* and the
+ * additive block, chunked in inference. */
 int nrms_user_encoder_fwd(const float* x, int64_t n_rows, const int32_t* rows, int64_t n_users, int S,
                           const float* wqkv, const float* bqkv,
                           const float* wa, const float* ba, const float* qa,
@@ -152,15 +159,16 @@ int nrms_user_encoder_fwd(const float* x, int64_t n_rows, const int32_t* rows, i
 /* Tensor-mode, inference-only form of the indexed user encoder whose table is already held as fp16 rows: table16 =
  * [n_rows + 1][320] halfs in nrms_pack_rows_f16's layout (300 values, 1.0 in column 300, zero tail; last row all zero).
  * This is what evaluate keeps between its stages (src/evaluate.py:193-233): the news stage packs its vectors once, the
- * all-gather moves 640-byte rows, and both the user encoder and nrms_score_csr_f16 read the same copy. */
+ * all-gather moves 640-byte rows, and both the user encoder and nrms_score_csr_f16 read the same copy.  At S other than
+ * 20 and 50 the gathered rows are widened to fp32 and run through the tensor-mode encoder a chunk of users at a time. */
 size_t nrms_user_encoder_table16_workspace_bytes(int64_t n_users, int S, int64_t n_rows);
 int nrms_user_encoder_table16_fwd(const void* table16, int64_t n_rows, const int32_t* rows, int64_t n_users, int S,
                                   const float* wqkv, const float* bqkv,
                                   const float* wa, const float* ba, const float* qa,
                                   float* out, void* workspace, size_t workspace_bytes, void* stream);
 
-/* User encoder backward (dense input only).  d_x [n_users,S,300] is OVERWRITTEN; weight
- * gradients are accumulated (+=). */
+/* User encoder backward (dense input only, S = 1..64 as the forward that wrote the stash).  d_x [n_users,S,300] is
+ * OVERWRITTEN; weight gradients are accumulated (+=). */
 int nrms_user_encoder_bwd(const float* d_out, int64_t n_users, int S,
                           const float* wqkv, const float* wa, const float* qa,
                           const void* stash,
@@ -220,9 +228,9 @@ int nrms_mha_bwd(const float* d_ctx, const float* xq, const float* xk, const flo
                  float* d_xv, float* d_wqkv, float* d_bqkv, void* workspace, size_t workspace_bytes, int mode,
                  void* stream);
 
-/* AdditiveAttention backward for the standalone block.  nrms_additive_fwd accepts S = 20, 50 and 2..4 (the final attention
- * over the 2..4 element vectors of model/Exp1, src/model/Exp1/news_encoder.py:104-110; that form always runs on the CUDA
- * cores).  fwd_workspace = the workspace the forward call filled (tanh activations | softmax weights).  d_c [n_seq,S,300]
+/* AdditiveAttention backward for the standalone block.  nrms_additive_fwd accepts 1 <= S <= 64 (2..4: the final attention
+ * over the element vectors of model/Exp1, src/model/Exp1/news_encoder.py:104-110).  S < 20 runs its linear map on the
+ * CUDA cores in either mode.  fwd_workspace = the workspace the forward call filled (tanh activations | softmax weights).  d_c [n_seq,S,300]
  * is OVERWRITTEN; d_wa [200,300], d_ba [200], d_qa [200] are accumulated into. */
 size_t nrms_additive_bwd_workspace_bytes(int64_t n_seq, int S, int mode);
 int nrms_additive_bwd(const float* d_out, const float* c, int64_t n_seq, int S, const float* wa, const float* qa,

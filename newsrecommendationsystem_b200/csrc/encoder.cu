@@ -117,9 +117,10 @@ static int gemm_nt_bias(const float* A, int64_t lda, const float* B, int64_t ldb
   return NRMS_OK;
 }
 
-// additive pooling kernels at every compiled sequence length: 20 (titles), 50 (history / abstracts) and 2..4 (the
-// final attention over the element vectors of model/Exp1, reference src/model/Exp1/news_encoder.py:106-110)
-static bool additive_len_ok(int S) { return S == 20 || S == 50 || (S >= 2 && S <= 4); }
+// additive pooling kernels: compiled for 20 (titles), 50 (history / abstracts) and 2..4 (the final attention over the
+// element vectors of model/Exp1, reference src/model/Exp1/news_encoder.py:106-110); every other length up to 64 (user
+// histories of another num_clicked_news_a_user, standalone blocks) takes the run-time-length kernels
+static bool additive_len_ok(int S) { return S >= 1 && S <= ADD_MAXS; }
 static cudaError_t launch_additive_fwd(const float* cin, float* t, const float* qa, float* wv, float* out, int64_t n_seq,
                                        int S, cudaStream_t st) {
   const unsigned gx = (unsigned)(n_seq < (int64_t)num_sms() * 8 ? n_seq : (int64_t)num_sms() * 8);
@@ -128,7 +129,8 @@ static cudaError_t launch_additive_fwd(const float* cin, float* t, const float* 
     case 50: additive_fwd_kernel<50><<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq); break;
     case 2: additive_fwd_kernel<2><<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq); break;
     case 3: additive_fwd_kernel<3><<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq); break;
-    default: additive_fwd_kernel<4><<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq); break;
+    case 4: additive_fwd_kernel<4><<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq); break;
+    default: additive_fwd_rt_kernel<<<gx, 256, 0, st>>>(cin, t, qa, wv, out, n_seq, S); break;
   }
   count_launch();
   return cudaGetLastError();
@@ -141,7 +143,8 @@ static cudaError_t launch_additive_bwd(const float* d_out, const float* cin, con
     case 50: additive_bwd_kernel<50><<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq); break;
     case 2: additive_bwd_kernel<2><<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq); break;
     case 3: additive_bwd_kernel<3><<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq); break;
-    default: additive_bwd_kernel<4><<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq); break;
+    case 4: additive_bwd_kernel<4><<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq); break;
+    default: additive_bwd_rt_kernel<<<nb, 256, 0, st>>>(d_out, cin, t, wv, qa, d_c, d_u, partial, n_seq, S); break;
   }
   count_launch();
   return cudaGetLastError();
@@ -168,7 +171,15 @@ static int encoder_core_fwd(const Stash& s, int64_t n_seq, int S, const float* w
     if (int rc2 = attn_mma50_fwd(s.qkv, s.c, n_seq, p2, seed, off2, st)) return rc2;
     e = cudaSuccess;
   } else if (S == 20) e = launch_attention_fwd<20, 15>(s.qkv, s.c, n_seq, p2, seed, off2, st);
-  else e = launch_attention_fwd<50, 5>(s.qkv, s.c, n_seq, p2, seed, off2, st);
+  else if (S == 50) e = launch_attention_fwd<50, 5>(s.qkv, s.c, n_seq, p2, seed, off2, st);
+  else {
+    // user histories of any other length (1..64, no dropout): the run-time-length attention of attn_cross.cu over the
+    // stash's q|k|v rows, in the call's mode
+    NRMS_CHECK_ARG(p2 == 0.f, NRMS_E_INVALID, "no dropout at sequence length %d (user encoder only)", S);
+    const MhaOperands op{s.qkv, s.qkv + D, s.qkv + 2 * D, D3, D3, D3};
+    if (int rc2 = mha_attn_fwd(op, s.c, n_seq, S, S, nullptr, mode, st)) return rc2;
+    e = cudaSuccess;
+  }
   if (e != cudaSuccess) return cuda_fail(e, "attention_fwd");
   const float* cin = s.c;
   if (ln) {
@@ -320,14 +331,30 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
     dqkv_t_written = true;
     e = cudaSuccess;
   } else if (S == 20) e = launch_attention_bwd<20, NRMS_ATTN_BWD_HC20>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
-  else e = launch_attention_bwd<50, 5>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
+  else if (S == 50) e = launch_attention_bwd<50, 5>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
+  else {
+    // other history lengths (user encoder only, no dropout): dq | dk | dv into dQKV with the pitch of the stash
+    NRMS_CHECK_ARG(p2 == 0.f, NRMS_E_INVALID, "no dropout at sequence length %d (user encoder only)", S);
+    const MhaOperands op{s.qkv, s.qkv + D, s.qkv + 2 * D, D3, D3, D3};
+    if (int rc2 = mha_attn_bwd(op, w.d_c, w.d_qkv, w.d_qkv + D, w.d_qkv + 2 * D, n_seq, S, S, nullptr, mode, st)) return rc2;
+    e = cudaSuccess;
+  }
   if (e != cudaSuccess) return cuda_fail(e, "attention_bwd");
   const QkvBwdWs qw{w.d_qkv, w.partial, w.t1, w.t2, w.wt, w.ldr};
   return qkv_proj_bwd(qw, s.x, wqkv, rows, d_x, d_wqkv, d_bqkv, tc, dqkv_t_written, st);
 }
 
+// news encoder and nrms_mhsa_*: the compiled title / abstract lengths
 static int check_common(int S, int mode) {
   NRMS_CHECK_ARG(S == 20 || S == 50, NRMS_E_UNSUPPORTED, "sequence length %d unsupported (compiled: 20, 50)", S);
+  NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
+  return NRMS_OK;
+}
+
+// user encoder: any history length up to 64 (20 and 50 keep their compiled kernels)
+constexpr int USER_MAXS = 64;
+static int check_user(int S, int mode) {
+  NRMS_CHECK_ARG(S >= 1 && S <= USER_MAXS, NRMS_E_UNSUPPORTED, "history length %d unsupported (1..%d)", S, USER_MAXS);
   NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
   return NRMS_OK;
 }
@@ -542,8 +569,8 @@ static int user_encoder_fwd_impl(const float* x, int64_t n_rows, const int32_t* 
                                  float* out, void* stash, void* workspace, size_t workspace_bytes, int mode,
                                  void* stream, const LnArgs* ln) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (int rc = check_user(S, mode)) return rc;     // the length first: outside 1..64 is NRMS_E_UNSUPPORTED
   if (int rc = check_ln(ln, false)) return rc;
-  if (int rc = check_common(S, mode)) return rc;
   NRMS_CHECK_ARG(n_users >= 0, NRMS_E_INVALID, "bad sizes");
   if (n_users == 0) return NRMS_OK;
   NRMS_CHECK_ARG(x && wqkv && bqkv && wa && ba && qa && out, NRMS_E_INVALID, "null pointer");
@@ -599,26 +626,50 @@ int nrms_user_encoder_ln_fwd(const float* x, int64_t n_rows, const int32_t* rows
                                workspace_bytes, mode, stream, &ln);
 }
 
+// S = 20 / 50: the fused kernels over the fp16 table; other lengths: chunks of fp32 stash rows widened from it
+static int64_t table16_chunk_seq(int64_t n_users, int S) {
+  const int64_t chunk_seq = INFER_CHUNK_ROWS / S;
+  return n_users < chunk_seq ? n_users : chunk_seq;
+}
+
 size_t nrms_user_encoder_table16_workspace_bytes(int64_t n_users, int S, int64_t n_rows) {
-  if (n_users <= 0 || S <= 0 || n_rows <= 0) return 0;
+  if (n_users <= 0 || S <= 0 || S > USER_MAXS || n_rows <= 0) return 0;
   size_t fused = tc_fused_workspace_bytes(n_users, S, n_rows, true);
-  return fused == (size_t)-1 ? 0 : fused + 256;
+  if (fused != (size_t)-1) return fused + 256;
+  return carve_stash(nullptr, table16_chunk_seq(n_users, S) * S).bytes + 256;
 }
 
 int nrms_user_encoder_table16_fwd(const void* table16, int64_t n_rows, const int32_t* rows_idx, int64_t n_users, int S,
                                   const float* wqkv, const float* bqkv, const float* wa, const float* ba, const float* qa,
                                   float* out, void* workspace, size_t workspace_bytes, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (int rc = check_common(S, NRMS_MODE_TF32)) return rc;
+  if (int rc = check_user(S, NRMS_MODE_TF32)) return rc;
   NRMS_CHECK_ARG(n_users >= 0 && n_rows > 0, NRMS_E_INVALID, "bad sizes");
   if (n_users == 0) return NRMS_OK;
   NRMS_CHECK_ARG(table16 && rows_idx && wqkv && bqkv && wa && ba && qa && out, NRMS_E_INVALID, "null pointer");
   NRMS_CHECK_ARG(aligned16(table16) && aligned16(wqkv) && aligned16(bqkv) && aligned16(wa) && aligned16(ba) && aligned16(out),
                  NRMS_E_INVALID, "pointers must be 16-byte aligned");
-  NRMS_CHECK_ARG(tc_fused_workspace_bytes(n_users, S, n_rows, true) != (size_t)-1, NRMS_E_UNSUPPORTED,
-                 "sequence length not compiled");
-  return tc_encoder_fused(nullptr, table16, n_rows, rows_idx, 2, n_users, S, wqkv, bqkv, wa, ba, qa, out, workspace,
-                          workspace_bytes, st);
+  if (tc_fused_workspace_bytes(n_users, S, n_rows, true) != (size_t)-1)
+    return tc_encoder_fused(nullptr, table16, n_rows, rows_idx, 2, n_users, S, wqkv, bqkv, wa, ba, qa, out, workspace,
+                            workspace_bytes, st);
+  // other lengths: the tensor-mode core over fp32 rows widened from the fp16 table, chunk by chunk
+  const int64_t chunk_seq = INFER_CHUNK_ROWS / S;
+  const size_t need = carve_stash(nullptr, table16_chunk_seq(n_users, S) * S).bytes;
+  NRMS_CHECK_ARG(workspace && aligned16(workspace) && workspace_bytes >= need, NRMS_E_WORKSPACE,
+                 "workspace too small: need %zu bytes", need);
+  for (int64_t s0 = 0; s0 < n_users; s0 += chunk_seq) {
+    const int64_t n = (n_users - s0 < chunk_seq) ? (n_users - s0) : chunk_seq;
+    Stash s = carve_stash(workspace, n * S);
+    const int64_t rows = n * S;
+    int64_t gb = (rows + 7) / 8;
+    if (gb > (int64_t)num_sms() * 16) gb = (int64_t)num_sms() * 16;
+    gather_rows_f16_kernel<<<(unsigned)gb, 256, 0, st>>>(reinterpret_cast<const __half*>(table16), rows_idx + s0 * S, rows,
+                                                         s.x);
+    NRMS_LAUNCH_CHECK("gather_rows_f16");
+    if (int rc = encoder_core_fwd(s, n, S, wqkv, bqkv, wa, ba, qa, out + s0 * D, 0.f, 0, 0, 0, NRMS_MODE_TF32, st))
+      return rc;
+  }
+  return NRMS_OK;
 }
 
 static int user_encoder_bwd_impl(const float* d_out, int64_t n_users, int S, const float* wqkv, const float* wa,
@@ -626,8 +677,8 @@ static int user_encoder_bwd_impl(const float* d_out, int64_t n_users, int S, con
                                  float* d_wa, float* d_ba, float* d_qa, void* workspace, size_t workspace_bytes,
                                  int mode, void* stream, const LnArgs* ln) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (int rc = check_user(S, mode)) return rc;     // the length first: outside 1..64 is NRMS_E_UNSUPPORTED
   if (int rc = check_ln(ln, true)) return rc;
-  if (int rc = check_common(S, mode)) return rc;
   if (n_users == 0) return NRMS_OK;
   NRMS_CHECK_ARG(n_users > 0, NRMS_E_INVALID, "bad sizes");
   NRMS_CHECK_ARG(d_out && wqkv && wa && qa && stash && d_x && d_wqkv && d_bqkv && d_wa && d_ba && d_qa, NRMS_E_INVALID,
@@ -947,7 +998,7 @@ int nrms_mha_bwd(const float* d_ctx, const float* xq, const float* xk, const flo
 int nrms_additive_fwd(const float* c, int64_t n_seq, int S, const float* wa, const float* ba, const float* qa,
                       float* out, void* workspace, size_t workspace_bytes, int mode, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  NRMS_CHECK_ARG(additive_len_ok(S), NRMS_E_UNSUPPORTED, "candidate size %d unsupported (compiled: 2, 3, 4, 20, 50)", S);
+  NRMS_CHECK_ARG(additive_len_ok(S), NRMS_E_UNSUPPORTED, "candidate size %d unsupported (1..64)", S);
   NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
   NRMS_CHECK_ARG(n_seq >= 0, NRMS_E_INVALID, "bad sizes");
   if (n_seq == 0) return NRMS_OK;
@@ -981,7 +1032,7 @@ int nrms_additive_bwd(const float* d_out, const float* c, int64_t n_seq, int S, 
                       const void* fwd_workspace, float* d_c, float* d_wa, float* d_ba, float* d_qa, void* workspace,
                       size_t workspace_bytes, int mode, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  NRMS_CHECK_ARG(additive_len_ok(S), NRMS_E_UNSUPPORTED, "candidate size %d unsupported (compiled: 2, 3, 4, 20, 50)", S);
+  NRMS_CHECK_ARG(additive_len_ok(S), NRMS_E_UNSUPPORTED, "candidate size %d unsupported (1..64)", S);
   NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
   NRMS_CHECK_ARG(n_seq >= 0, NRMS_E_INVALID, "bad sizes");
   if (n_seq == 0) return NRMS_OK;

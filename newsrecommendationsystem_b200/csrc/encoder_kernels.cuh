@@ -4,6 +4,7 @@
 // file:line map): scores = QK^T / sqrt(20); e = exp(scores) (no max subtraction);
 // attn = e / (sum e + 1e-8); ctx = attn V; pooling = stable softmax over tanh(linear(c)) . q.
 #pragma once
+#include <cuda_fp16.h>
 #include "common.cuh"
 
 namespace nrms {
@@ -58,6 +59,27 @@ gather_rows_kernel(const float* __restrict__ src, const IdxT* __restrict__ rows,
     const float4* s = reinterpret_cast<const float4*>(src) + (int64_t)rows[r] * width4;
     float4* d = reinterpret_cast<float4*>(dst) + r * width4;
     for (int l = lane; l < width4; l += 32) d[l] = __ldg(s + l);
+  }
+}
+
+// the same gather from an fp16 table in pack_rows_f16's layout ([*, 320] halfs, values in columns 0..299): each row's 300
+// values widened to an fp32 row of dst [n, 300].  One warp per row, four halfs (8 bytes) per lane and step.
+static __global__ void __launch_bounds__(256)
+gather_rows_f16_kernel(const __half* __restrict__ src, const int32_t* __restrict__ rows, int64_t n,
+                       float* __restrict__ dst) {
+  constexpr int SRC_LD = 320;
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t r = warp; r < n; r += nwarps) {
+    const uint2* s = reinterpret_cast<const uint2*>(src + (int64_t)rows[r] * SRC_LD);
+    float4* d = reinterpret_cast<float4*>(dst) + r * DV4;
+    for (int l = lane; l < DV4; l += 32) {
+      const uint2 u = __ldg(s + l);
+      const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
+      const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+      d[l] = make_float4(a.x, a.y, b.x, b.y);
+    }
   }
 }
 
@@ -368,6 +390,106 @@ additive_bwd_kernel(const float* __restrict__ d_out, const float* __restrict__ c
   __shared__ float dwv[S];
   __shared__ float dsv[S];
   __shared__ float wv[S];
+  __shared__ __align__(16) float go[D];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  float dqa_acc = 0.f, dba_acc = 0.f;
+  const float qv = (tid < QD) ? qa[tid] : 0.f;
+  for (int64_t seq = blockIdx.x; seq < n_seq; seq += gridDim.x) {
+    for (int d = tid; d < D; d += 256) go[d] = d_out[seq * D + d];
+    if (tid < S) wv[tid] = w[seq * S + tid];
+    __syncthreads();
+    for (int i = warp; i < S; i += 8) {
+      const float* cp = c + (seq * S + i) * D;
+      float part = 0.f;
+      for (int d = lane; d < D; d += 32) part = fmaf(go[d], cp[d], part);
+      part = warp_sum(part);
+      if (lane == 0) dwv[i] = part;
+    }
+    __syncthreads();
+    if (warp == 0) {
+      float dot = 0.f;
+      for (int i = lane; i < S; i += 32) dot = fmaf(wv[i], dwv[i], dot);
+      dot = warp_sum(dot);
+      for (int i = lane; i < S; i += 32) dsv[i] = wv[i] * (dwv[i] - dot);
+    }
+    __syncthreads();
+    if (tid < QD) {
+      for (int i = 0; i < S; ++i) {
+        const int64_t row = seq * S + i;
+        const float tv = t[row * QD + tid];
+        const float ds = dsv[i];
+        const float du = ds * qv * (1.f - tv * tv);
+        d_u[row * QD + tid] = du;
+        dba_acc += du;
+        dqa_acc = fmaf(ds, tv, dqa_acc);
+      }
+    }
+    for (int f = tid; f < S * DV4; f += 256) {
+      const int i = f / DV4, l = f % DV4;
+      const float wi = wv[i];
+      float4 g = *reinterpret_cast<const float4*>(go + 4 * l);
+      *reinterpret_cast<float4*>(d_c + (seq * S + i) * D + 4 * l) = make_float4(wi * g.x, wi * g.y, wi * g.z, wi * g.w);
+    }
+    __syncthreads();
+  }
+  if (tid < QD) {
+    partial_dqa[(int64_t)blockIdx.x * QD + tid] = dqa_acc;
+    partial_dqa[(int64_t)(gridDim.x + blockIdx.x) * QD + tid] = dba_acc;
+  }
+}
+
+// The two additive kernels above with the sequence length passed at run time, 1 <= S <= ADD_MAXS: the user encoder at
+// any history length and the standalone block at any candidate count.  The compiled lengths keep their templates.
+constexpr int ADD_MAXS = 64;
+
+static __global__ void __launch_bounds__(256)
+additive_fwd_rt_kernel(const float* __restrict__ c, float* __restrict__ t, const float* __restrict__ qa,
+                       float* __restrict__ w, float* __restrict__ out, int64_t n_seq, int S) {
+  __shared__ float sc[ADD_MAXS];
+  __shared__ float wv[ADD_MAXS];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int64_t seq = blockIdx.x; seq < n_seq; seq += gridDim.x) {
+    for (int i = warp; i < S; i += 8) {
+      float* trow = t + (seq * S + i) * QD;
+      float part = 0.f;
+      for (int q = lane; q < QD; q += 32) {
+        float v = tanhf(trow[q]);
+        trow[q] = v;
+        part = fmaf(v, __ldg(qa + q), part);
+      }
+      part = warp_sum(part);
+      if (lane == 0) sc[i] = part;
+    }
+    __syncthreads();
+    if (warp == 0) {
+      float m = -INFINITY;
+      for (int i = lane; i < S; i += 32) m = fmaxf(m, sc[i]);
+      m = warp_max(m);
+      float sum = 0.f;
+      for (int i = lane; i < S; i += 32) { float e = expf(sc[i] - m); wv[i] = e; sum += e; }
+      sum = warp_sum(sum);
+      for (int i = lane; i < S; i += 32) { float x = wv[i] / sum; wv[i] = x; w[seq * S + i] = x; }
+    }
+    __syncthreads();
+    for (int d = tid; d < D; d += 256) {
+      const float* cp = c + seq * S * D + d;
+      float acc = 0.f;
+#pragma unroll 5
+      for (int i = 0; i < S; ++i) acc = fmaf(wv[i], cp[(int64_t)i * D], acc);
+      out[seq * D + d] = acc;
+    }
+    __syncthreads();
+  }
+}
+
+static __global__ void __launch_bounds__(256)
+additive_bwd_rt_kernel(const float* __restrict__ d_out, const float* __restrict__ c, const float* __restrict__ t,
+                       const float* __restrict__ w, const float* __restrict__ qa,
+                       float* __restrict__ d_c, float* __restrict__ d_u, float* __restrict__ partial_dqa,
+                       int64_t n_seq, int S) {
+  __shared__ float dwv[ADD_MAXS];
+  __shared__ float dsv[ADD_MAXS];
+  __shared__ float wv[ADD_MAXS];
   __shared__ __align__(16) float go[D];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float dqa_acc = 0.f, dba_acc = 0.f;

@@ -7,11 +7,11 @@ The reference keeps pandas frames and dicts of per-news tensors and assembles ev
                           abstract_entities`; list columns are Python-list literals)
       -> NewsTable: ids, `title` int64 [N, 20] (+ `abstract` [N, 50], `category` / `subcategory` [N] on request)
   behaviors_parsed.tsv   (data_preprocess.py:77-81: header `user clicked_news candidate_news clicked`)
-      -> TrainRows: `cand_rows` int64 [B, 1+K], `hist_rows` int64 [B, 50] -- news-row indices for
+      -> TrainRows: `cand_rows` int64 [B, 1+K], `hist_rows` int64 [B, num_clicked] -- news-row indices for
          `TrainStep.step_rows` (first 50 clicks, LEFT-padded, dataset.py:69-83; the pad index is row N of
          `NewsTable.token_table_with_pad()`, an all-zero title = the reference's `padding` entry, dataset.py:45-60)
   behaviors.tsv          (raw MIND, no header: impression_id user time clicked_news impressions)
-      -> the arguments of `evaluate.EvalHost`: `hist_rows` [I, 50] (-1 = PADDED_NEWS), CSR candidates and labels
+      -> the arguments of `evaluate.EvalHost`: `hist_rows` [I, num_clicked] (-1 = PADDED_NEWS), CSR candidates and labels
          (`"N123-1"` split on '-', evaluate.py:252,261-263; first 50 clicks, left-padded, :117-124)
 
 Duplicate news ids: the first row wins (evaluate.py:197-201) -- `NewsTable.row_of`.

@@ -5,7 +5,7 @@ launches one bmm + .tolist() per impression.  Here the same semantics run on int
 
   stage A  news table  [N_news+1, 300]; last row = PADDED_NEWS zeros (evaluate.py:203-204);
            duplicate news ids resolve to their FIRST row (evaluate.py:197-201)
-  stage B  user vectors from int32 history rows [I, 50] (first 50 clicks, LEFT padded,
+  stage B  user vectors from int32 history rows [I, S] (first S = num_clicked_news_a_user clicks, LEFT padded,
            evaluate.py:111-124), gathered inside the library
   stage C  CSR scoring (evaluate.py:245-260), `max_count` keeps the reference's off-by-one
            (:247-249 processes max_count-1 impressions)
@@ -82,7 +82,7 @@ class EvalHost:
     """Evaluate inputs preprocessed on the host into the library's index formats, in pinned
     memory (when CUDA is available) so `EvalInputs.from_host` is a handful of async H2D copies.
 
-    news_tokens  int64 [N_news, L]        hist_rows  int32 [I, 50]  (pad -> N_news, the zero row)
+    news_tokens  int64 [N_news, L]        hist_rows  int32 [I, S]   (pad -> N_news, the zero row)
     cand_rows    int32 [sumC]             cand_offsets int64 [I+1]   labels int8 [sumC]
     """
 
@@ -373,7 +373,9 @@ def evaluate(model, directory, num_workers=0, max_count=None):
     import sys
     from . import data
     news = data.load_news_parsed(os.path.join(directory, "news_parsed.tsv"))
-    ev = data.load_behaviors(os.path.join(directory, "behaviors.tsv"), news)
+    # the history length the model was built for (a model without a config: the reference's default, 50)
+    num_clicked = int(getattr(getattr(model, "config", None), "num_clicked_news_a_user", 50))
+    ev = data.load_behaviors(os.path.join(directory, "behaviors.tsv"), news, num_clicked=num_clicked)
     device = next(model.parameters()).device if hasattr(model, "parameters") else "cpu"
     inputs = EvalInputs(news.title, ev.hist_rows, ev.cand_offsets, ev.cand_rows, ev.labels, news_ids=news.ids, device=device)
     if max_count is not None and max_count >= sys.maxsize:

@@ -34,7 +34,7 @@ class UserEncoder(nn.Module):
                                 mode=resolve_mode(self.config, self.precision), ln=self._ln())
 
     def forward_indexed(self, table, rows):
-        """Inference: history rows gathered from the news-vector table (int32 [B, 50]).  `table` is the fp32 [n, 300]
+        """Inference: history rows gathered from the news-vector table (int32 [B, S], S = num_clicked_news_a_user, 1..64).  `table` is the fp32 [n, 300]
         table, or (tensor mode, no LayerNorm) its fp16 copy [n + 1, 320] from `ops.pack_rows_f16`."""
         if table.dtype == torch.float16:
             from ... import _lib

@@ -20,7 +20,7 @@ class AdditiveAttention(nn.Module):
 
     def forward(self, candidate_vector):
         """candidate_vector: batch_size, candidate_size, candidate_vector_dim -> batch_size, candidate_vector_dim.
-        Standalone use (candidate_size 20, 50, or 2..4 as in model/Exp1's final attention), forward and backward in
+        Standalone use (candidate_size 1..64; 2..4 is model/Exp1's final attention), forward and backward in
         libnrms_b200; inside the NRMS encoders this block is fused into the encoder kernels."""
         from .... import ops
         from ....config import resolve_mode

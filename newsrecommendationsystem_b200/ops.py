@@ -613,7 +613,8 @@ def mha(q, k, v, wqkv, bqkv, mode=_lib.MODE_TF32, length=None):
 
 class _AdditiveFn(torch.autograd.Function):
     """AdditiveAttention.forward (reference src/model/general/attention/additive.py:27-53) with its backward, for
-    candidate sizes 20 / 50 and 2..4 (the final attention of model/Exp1)."""
+    candidate sizes 1..64 (20 / 50: encoder lengths, 2..4: the final attention of model/Exp1; below 20 the linear map
+    runs on the CUDA cores in either mode)."""
 
     @staticmethod
     def forward(ctx, c, wa, ba, qa, mode, track_grad):

@@ -78,7 +78,7 @@ class Recommender:
         return self.recommend(clicked, impressions)
 
     def history_rows(self, clicked_news):
-        """First 50 clicks, LEFT-padded with PADDED_NEWS (src/recommend.py:117-124 = evaluate.py:117-124)."""
+        """First num_clicked_news_a_user clicks, LEFT-padded with PADDED_NEWS (src/recommend.py:117-124 = evaluate.py:117-124)."""
         rows = [self.row_of[x] for x in list(clicked_news)[:self.n_hist]]
         return [self.pad_row] * (self.n_hist - len(rows)) + rows
 
@@ -115,10 +115,13 @@ class Recommender:
         the returned tensors are views that the next call overwrites.  The host waits only when the previous call's
         index copy has not run yet, before it rewrites the pinned staging buffer; otherwise nothing syncs.
         Order: score descending, equal scores by ascending candidate position, NaN scores last (np.argsort(-y) on a
-        stable sort), on both sides of the 4,096-candidate limit."""
+        stable sort), on both sides of the 4,096-candidate limit.  The cluster kernel is compiled for 50 history rows;
+        other num_clicked_news_a_user take the indexed user encoder (FP32 mode) and a device sort, with fresh tensors."""
         from ._lib import check, ptr
         n_c = len(cand_rows)
         dev = self.table.device
+        if self.n_hist != 50:
+            return self._recommend_rows_any_length(hist_rows, cand_rows)
         if n_c > 4096:
             ue = self.model.user_encoder
             a = ue.additive_attention
@@ -143,10 +146,26 @@ class Recommender:
                                             C.c_void_p(stream.cuda_stream)), "nrms_recommend_user")
         return st["order"][:n_c], st["scores"][:n_c], st["user"]
 
+    def _recommend_rows_any_length(self, hist_rows, cand_rows):
+        """recommend_rows at a history length the cluster kernel is not compiled for (num_clicked_news_a_user != 50):
+        the indexed user encoder in FP32 mode -- the arithmetic of the S = 50 latency path, which is FP32 too -- then
+        score_csr over one impression and a stable descending sort (NaN last), as the > 4,096-candidate branch."""
+        from . import _lib
+        ue = self.model.user_encoder
+        dev = self.table.device
+        hist = torch.as_tensor(hist_rows, dtype=torch.int32).to(dev).view(1, -1)
+        if hist.shape[1] != self.n_hist:
+            raise RuntimeError(f"hist_rows must hold {self.n_hist} rows, got {hist.shape[1]}")
+        cand = torch.as_tensor(cand_rows, dtype=torch.int32).to(dev).view(-1)
+        user = ops.user_encoder_indexed(self.table, hist, *ue._weights(), mode=_lib.MODE_FP32, ln=ue._ln())
+        offsets = torch.tensor([0, cand.numel()], dtype=torch.int64, device=dev)
+        scores = ops.score_csr(self.table, cand, offsets, user)
+        return torch.argsort(-scores, stable=True).int(), scores, user[0]
+
     @torch.no_grad()
     def top_k_rows(self, hist_rows, k, exclude_clicked=True):
         """The k best news of the whole table for each user, not only for candidates the caller already has.
-        hist_rows: int32 [U, 50] in `history_rows` form (pads = the table's last row), host or device.  Returns (rows int32
+        hist_rows: int32 [U, num_clicked_news_a_user] in `history_rows` form (pads = the table's last row), host or device.  Returns (rows int32
         [U, k], scores fp32 [U, k], user_vec fp32 [U, 300]) on the device, no sync: rows by descending score (equal scores
         by ascending row), the clicked rows left out when exclude_clicked; tail entries are row -1, score -inf.
         Arithmetic follows the user encoder's precision: tensor mode scores against an fp16 copy of the table, packed on
