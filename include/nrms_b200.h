@@ -16,6 +16,8 @@
  *   nrms_adam_step              torch.optim.Adam(lr=1e-4).step()   src/train.py:127-128,233 (AdamW: decoupled=1)
  *   nrms_rank_metrics           calculate_single_user_metric + nanmean  src/evaluate.py:24-42,160-168,270-272
  *   nrms_news_encoder_rows_fwd/bwd  NewsEncoder over an index-only minibatch    src/dataset.py:17-85, src/train.py:118-124
+ *   nrms_text_encoder_fwd/bwd   NewsEncoder.forward / Exp1 TextEncoder at any text length 1..64
+ *                               src/model/NRMS/news_encoder.py:27-48, src/model/Exp1/news_encoder.py:10-34
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
  *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
  *   nrms_mha_fwd/bwd            MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries / keys  (same lines)
@@ -32,7 +34,8 @@
  *   - Return value: 0 = ok, nonzero = error (NRMS_E_*); text via nrms_last_error()
  *     (thread-local).  No exception crosses the ABI.  There is no CPU fallback.
  *   - Model dimensions are compile-time: D=300, H=15 (d_k=d_v=20), query dim 200
- *     (src/config.py:14-45).  Text length L is 20 (titles) or 50 (abstracts); the user encoder's history length S
+ *     (src/config.py:14-45).  Text length L is 20 (titles) or 50 (abstracts) in nrms_news_encoder_*, and any 1..64
+ *     (config.num_words_title / num_words_abstract) in nrms_text_encoder_*; the user encoder's history length S
  *     (config.num_clicked_news_a_user) is any 1..64, with fused kernels at 20 and 50.
  *   - Packed weights: wqkv = rows [W_Q; W_K; W_V] -> [900,300] (nn.Linear "out,in" layout),
  *     bqkv [900], wa [200,300], ba [200], qa [200].
@@ -254,6 +257,37 @@ int nrms_news_encoder_rows_bwd(const float* d_out, const int64_t* token_table, i
                                float* d_bqkv, float* d_ln_gamma, float* d_ln_beta, float* d_wa, float* d_ba, float* d_qa,
                                void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset,
                                int mode, void* stream);
+
+/* ---- text encoder at any length 1..64 --------------------------------------------------------
+ * The news encoder (src/model/NRMS/news_encoder.py:27-48; Exp1's TextEncoder, src/model/Exp1/news_encoder.py:10-34) at
+ * any title / abstract length L = 1..64: the reference pads and truncates every text to BaseConfig.num_words_title /
+ * num_words_abstract (src/data_preprocess.py:115,132-139), so L is a setting.  One pair for every form:
+ *   - news_rows NULL: dense tokens int64 [n_token_rows, L], text t = row t (n_token_rows >= n_texts);
+ *     news_rows non-NULL: index-only minibatch (as nrms_news_encoder_rows_*), text t = row news_rows[t] of the
+ *     [n_token_rows, L] table -- training only (stash required);
+ *   - ln_gamma / ln_beta both NULL (reference NRMS) or both given (config-5 LayerNorm); the backward takes ln_gamma and
+ *     d_ln_gamma / d_ln_beta;
+ *   - stash non-NULL: training (nrms_encoder_stash_bytes / nrms_encoder_ln_stash_bytes); NULL: inference, with
+ *     workspace = nrms_encoder_fwd_workspace_bytes(n_texts, L, mode, 0, num_words).  The backward's workspace is
+ *     nrms_encoder_bwd_workspace_bytes(n_texts, L, mode).
+ * Both dropout sites (:38-45) draw the Philox stream of nrms_news_encoder_fwd: element e of the [rows, 300] activation
+ * keeps counter e / 4 + offset, so a text's masks depend only on its row, and a chunked inference pass equals a single
+ * one.  L outside 1..64 returns NRMS_E_UNSUPPORTED before any pointer check and before any CUDA call; then each form is
+ * checked as its nrms_news_encoder_* counterpart.  L = 20 and 50 run exactly what nrms_news_encoder_* run; other lengths
+ * run the attention of nrms_mha_* with dropout #2 applied inside it, and the run-time-length additive kernels (inference
+ * takes the chunked path: the fused inference kernels are compiled for 20 and 50 only).  Gradients are ACCUMULATED as in
+ * nrms_news_encoder_bwd. */
+int nrms_text_encoder_fwd(const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows, int64_t n_texts, int L,
+                          const float* emb, int64_t num_words, const float* wqkv, const float* bqkv,
+                          const float* ln_gamma, const float* ln_beta, const float* wa, const float* ba, const float* qa,
+                          float* out, void* stash, void* workspace, size_t workspace_bytes, float dropout_p,
+                          uint64_t seed, uint64_t offset, int mode, void* stream);
+int nrms_text_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows,
+                          int64_t n_texts, int L, int64_t num_words, const float* wqkv, const float* ln_gamma,
+                          const float* wa, const float* qa, const void* stash, float* d_emb, float* d_wqkv,
+                          float* d_bqkv, float* d_ln_gamma, float* d_ln_beta, float* d_wa, float* d_ba, float* d_qa,
+                          void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset,
+                          int mode, void* stream);
 
 /* ---- model/Exp1 blocks (SURVEY 8 f3) ------------------------------------------------------
  * ElementEncoder.forward = relu(linear(embedding(element)))  (src/model/Exp1/news_encoder.py:37-44):

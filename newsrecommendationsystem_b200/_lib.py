@@ -62,6 +62,10 @@ SIGNATURES = {
                                           _vp, _f32, _u64, _u64, _i32, _vp]),
     "nrms_news_encoder_rows_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                           _vp, _vp, _vp, _vp, _vp, _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
+    "nrms_text_encoder_fwd": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                     _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
+    "nrms_text_encoder_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                     _vp, _vp, _vp, _vp, _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
     "nrms_element_encoder_table_bytes": (_sz, [_i64]),
     "nrms_element_encoder_fwd": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "nrms_element_encoder_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -23,6 +23,12 @@
 // FP32 mode (attn_cross_fwd/bwd_kernel): CUDA-core kernels in the style of attention_fwd/bwd_kernel<S, HC>
 // (encoder_kernels.cuh) with run-time lengths: thread = (head, query), K and V in shared memory, the same arithmetic
 // (reference-exact up to summation order).
+// DROPOUT (the news encoder's dropout #2 at text lengths other than 20 and 50, reference
+// src/model/NRMS/news_encoder.py:43-45; self-attention only, ctx pitch 300): the forward multiplies the context by the
+// mask where it stores it, the backward multiplies d_ctx by the same mask where it loads it.  The mask of element
+// (seq * sq + i) * 300 + col is dropout_mask4(.., DROPOUT_STREAM_CTX, p, 1 / (1 - p), seed, offset), the stream the
+// compiled 20- and 50-token kernels draw: one Philox evaluation covers four aligned columns, and heads start at multiples
+// of 20 columns, so a group never straddles two heads.  Without it the kernels are those of the standalone block.
 #include "common.cuh"
 #include "tc_api.cuh"
 
@@ -36,6 +42,13 @@ constexpr float SQRT_DH = 4.47213595499957939f;
 constexpr float SCALE_LOG2E = 1.4426950408889634f / SQRT_DH;     // exp(s / sqrt 20) = 2^(s * log2(e) / sqrt 20)
 constexpr float INV_SQRT_DH = 1.f / SQRT_DH;
 constexpr float ATTN_EPS = 1e-8f;
+constexpr uint32_t DROPOUT_STREAM_CTX = 2;     // encoder_kernels.cuh
+
+// dropout #2 of the call (read only by the DROPOUT instantiations)
+struct Drop {
+  float p, scale;
+  uint64_t seed, offset;
+};
 
 typedef float Row[NT][4];        // accumulators of 16 rows x 64 columns
 typedef float Out[3][4];         // accumulators of 16 rows x 24 columns (the head dimension)
@@ -165,6 +178,18 @@ __device__ __forceinline__ void fetch_round(float* tile, int n, int lane) {
     *q = make_float4(tf32_round(x.x), tf32_round(x.y), tf32_round(x.z), tf32_round(x.w));
   }
 }
+// fetch_round of the d_ctx tile with the dropout-2 mask applied before the rounding: row j of the tile is row row0 + j
+// of the call, its columns start at column `col` of the 300
+__device__ __forceinline__ void fetch_round_masked(float* tile, int n, int lane, int64_t row0, int col, const Drop& dr) {
+  for (int f = lane; f < n * (DH / 4); f += 32) {
+    const int j = f / (DH / 4), d4 = f % (DH / 4);
+    float4* q = reinterpret_cast<float4*>(tile + j * ST + d4 * 4);
+    const float4 x = *q;
+    const float4 m = dropout_mask4((uint64_t)(row0 + j) * D + col + d4 * 4, DROPOUT_STREAM_CTX, dr.p, dr.scale, dr.seed,
+                                   dr.offset);
+    *q = make_float4(tf32_round(x.x * m.x), tf32_round(x.y * m.y), tf32_round(x.z * m.z), tf32_round(x.w * m.w));
+  }
+}
 
 // keys of sequence `seq` that the mask keeps (see the file header)
 __device__ __forceinline__ int key_limit(const int32_t* __restrict__ lengths, int64_t seq, int sq, int sk) {
@@ -174,10 +199,11 @@ __device__ __forceinline__ int key_limit(const int32_t* __restrict__ lengths, in
   return l < 0 ? 0 : (l < sk ? l : sk);
 }
 
+template <bool DROPOUT>
 __global__ void __launch_bounds__(32)
 mha_fwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict__ k, int64_t ldk,
                const float* __restrict__ v, int64_t ldv, float* __restrict__ ctx, int64_t n_seq, int sq, int sk,
-               const int32_t* __restrict__ lengths) {
+               const int32_t* __restrict__ lengths, Drop dr) {
   extern __shared__ __align__(16) float smem[];
   const int lane = threadIdx.x, g = lane >> 2, t = lane & 3;
   const int rq = round16(sq), rk = round16(sk);
@@ -209,17 +235,34 @@ mha_fwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict
       Out o;
       zero(o);
       gemm_frag_n<false>(o, a, V, nkb, g, t);
+      if (DROPOUT) {
+        // a lane pair (t, t ^ 1) holds two columns of one aligned group of four in two rows: the even lane draws row
+        // g's group, the odd lane row g + 8's, and each hands its partner the half it needs (as attn_mma.cu's amma50)
+        const int odd = t & 1;
+#pragma unroll
+        for (int nt = 0; nt < 3; ++nt) {
+          const float4 m = dropout_mask4((uint64_t)(seq * sq + m0 + g + 8 * odd) * D + col + nt * 8 + (t >> 1) * 4,
+                                         DROPOUT_STREAM_CTX, dr.p, dr.scale, dr.seed, dr.offset);
+          const float r0 = __shfl_xor_sync(0xffffffffu, odd ? m.x : m.z, 1);
+          const float r1 = __shfl_xor_sync(0xffffffffu, odd ? m.y : m.w, 1);
+          o[nt][0] *= odd ? r0 : m.x;
+          o[nt][1] *= odd ? r1 : m.y;
+          o[nt][2] *= odd ? m.z : r0;
+          o[nt][3] *= odd ? m.w : r1;
+        }
+      }
       store_rows(ctx + seq * sq * D + col, D, o, m0, sq, g, t);
     }
   }
 }
 
 // dq / dk / dv are written with the pitches of q / k / v (the projection layout the weight contractions read)
+template <bool DROPOUT>
 __global__ void __launch_bounds__(32)
 mha_bwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict__ k, int64_t ldk,
                const float* __restrict__ v, int64_t ldv, const float* __restrict__ d_ctx, float* __restrict__ dq,
                float* __restrict__ dk, float* __restrict__ dv, int64_t n_seq, int sq, int sk,
-               const int32_t* __restrict__ lengths) {
+               const int32_t* __restrict__ lengths, Drop dr) {
   extern __shared__ __align__(16) float smem[];
   const int lane = threadIdx.x, g = lane >> 2, t = lane & 3;
   const int rq = round16(sq), rk = round16(sk);
@@ -241,7 +284,8 @@ mha_bwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict
     fetch_issue(V, v + seq * sk * ldv + col, ldv, sk, lane);
     cp_async_wait_all();
     fetch_round(Q, sq, lane);
-    fetch_round(G, sq, lane);
+    if (DROPOUT) fetch_round_masked(G, sq, lane, seq * sq, col, dr);
+    else fetch_round(G, sq, lane);
     fetch_round(K, sk, lane);
     fetch_round(V, sk, lane);
     __syncwarp();
@@ -322,11 +366,11 @@ constexpr int MHA_HC_FWD = 5;    // heads per CTA: K and V of 5 heads at 64 keys
 constexpr int MHA_HC_BWD = 3;    // Q, dO, K, V and the two [3*Sq][Sk+1] score planes: 161 KB at 64 x 64
 
 // CTA = (sequence, chunk of HC heads); thread = (head, query i)
-template <int HC>
+template <int HC, bool DROPOUT>
 __global__ void __launch_bounds__(HC * MHA_MAXS)
 attn_cross_fwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict__ k, int64_t ldk,
                       const float* __restrict__ v, int64_t ldv, float* __restrict__ ctx, int64_t n_seq, int sq, int sk,
-                      const int32_t* __restrict__ lengths) {
+                      const int32_t* __restrict__ lengths, amha::Drop dr) {
   constexpr int W = HC * DH, W4 = W / 4;
   extern __shared__ __align__(16) float smem[];
   float* Ks = smem;            // [sk][W]
@@ -380,19 +424,27 @@ attn_cross_fwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __r
     const float inv = 1.f / (Z + amha::ATTN_EPS);
     float4* op = reinterpret_cast<float4*>(ctx + (seq * sq + i) * D + cw + hl * DH);
 #pragma unroll
-    for (int c = 0; c < DH / 4; ++c) op[c] = make_float4(acc[4 * c] * inv, acc[4 * c + 1] * inv, acc[4 * c + 2] * inv, acc[4 * c + 3] * inv);
+    for (int c = 0; c < DH / 4; ++c) {
+      float4 o = make_float4(acc[4 * c] * inv, acc[4 * c + 1] * inv, acc[4 * c + 2] * inv, acc[4 * c + 3] * inv);
+      if (DROPOUT) {
+        const float4 m = dropout_mask4((uint64_t)(seq * sq + i) * D + cw + hl * DH + 4 * c, amha::DROPOUT_STREAM_CTX, dr.p,
+                                       dr.scale, dr.seed, dr.offset);
+        o.x *= m.x; o.y *= m.y; o.z *= m.z; o.w *= m.w;
+      }
+      op[c] = o;
+    }
   }
 }
 
 // Phase 1: thread (h, query i) computes row i of the scores (e_ij, da_ij = g_i . v_j), its 1 / (Z + eps) and delta, then
 // dQ_i, leaving attn_ij and ds_ij in shared memory (zero for masked keys).  Phase 2: thread (h, key j) reads column j
 // and accumulates dK_j and dV_j.  Score planes have a pitch of sk + 1 words.
-template <int HC>
+template <int HC, bool DROPOUT>
 __global__ void __launch_bounds__(HC * MHA_MAXS)
 attn_cross_bwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __restrict__ k, int64_t ldk,
                       const float* __restrict__ v, int64_t ldv, const float* __restrict__ d_ctx, float* __restrict__ dq,
                       float* __restrict__ dk, float* __restrict__ dv, int64_t n_seq, int sq, int sk,
-                      const int32_t* __restrict__ lengths) {
+                      const int32_t* __restrict__ lengths, amha::Drop dr) {
   constexpr int W = HC * DH, W4 = W / 4;
   const int sp1 = sk + 1;
   extern __shared__ __align__(16) float smem[];
@@ -414,6 +466,14 @@ attn_cross_bwd_kernel(const float* __restrict__ q, int64_t ldq, const float* __r
         const int which = f / nq, r = f % nq, j = r / W4, c4 = r % W4;
         src = (which ? d_ctx + (seq * sq + j) * D : q + (seq * sq + j) * ldq) + cw + c4 * 4;
         dst = (which ? Gs : Qs) + j * W + c4 * 4;
+        if (DROPOUT && which) {      // d_ctx through the dropout-2 mask
+          float4 x = *reinterpret_cast<const float4*>(src);
+          const float4 m = dropout_mask4((uint64_t)(seq * sq + j) * D + cw + c4 * 4, amha::DROPOUT_STREAM_CTX, dr.p,
+                                         dr.scale, dr.seed, dr.offset);
+          x.x *= m.x; x.y *= m.y; x.z *= m.z; x.w *= m.w;
+          *reinterpret_cast<float4*>(dst) = x;
+          continue;
+        }
       } else {
         const int f2 = f - 2 * nq, nk = sk * W4;
         const int which = f2 / nk, r = f2 % nk, j = r / W4, c4 = r % W4;
@@ -512,44 +572,77 @@ static unsigned mha_grid_x(int64_t n_seq, int per_sm) {
 }
 
 int mha_attn_fwd(const MhaOperands& in, float* ctx, int64_t n_seq, int sq, int sk, const int32_t* lengths, int mode,
-                 cudaStream_t st) {
+                 cudaStream_t st, float p, uint64_t seed, uint64_t offset) {
   if (n_seq == 0) return NRMS_OK;
+  const amha::Drop dr{p, p > 0.f ? 1.f / (1.f - p) : 1.f, seed, offset};
   if (mode == NRMS_MODE_TF32) {
     const size_t smem = (size_t)(amha::round16(sq) + 2 * amha::round16(sk)) * amha::ST * sizeof(float);
-    amha::mha_fwd_kernel<<<dim3(mha_grid_x(n_seq, 16), H), 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx,
-                                                                            n_seq, sq, sk, lengths);
+    const dim3 grid(mha_grid_x(n_seq, 16), H);
+    if (p > 0.f)
+      amha::mha_fwd_kernel<true><<<grid, 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx, n_seq, sq, sk,
+                                                         lengths, dr);
+    else
+      amha::mha_fwd_kernel<false><<<grid, 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx, n_seq, sq, sk,
+                                                          lengths, dr);
     NRMS_LAUNCH_CHECK("mha_fwd");
     return NRMS_OK;
   }
   constexpr int HC = MHA_HC_FWD;
-  static bool configured[64] = {false};
-  if (cudaError_t e = set_max_dynamic_smem(attn_cross_fwd_kernel<HC>, 2 * MHA_MAXS * HC * DH * (int)sizeof(float), configured))
-    return cuda_fail(e, "attn_cross_fwd attr");
   const size_t smem = (size_t)2 * sk * HC * DH * sizeof(float);
-  attn_cross_fwd_kernel<HC><<<dim3(mha_grid_x(n_seq, 8), H / HC), (sq * HC + 31) / 32 * 32, smem, st>>>(
-      in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx, n_seq, sq, sk, lengths);
+  const dim3 grid(mha_grid_x(n_seq, 8), H / HC);
+  const int threads = (sq * HC + 31) / 32 * 32;
+  const int max_smem = 2 * MHA_MAXS * HC * DH * (int)sizeof(float);
+  if (p > 0.f) {
+    static bool configured[64] = {false};
+    if (cudaError_t e = set_max_dynamic_smem(attn_cross_fwd_kernel<HC, true>, max_smem, configured))
+      return cuda_fail(e, "attn_cross_fwd attr");
+    attn_cross_fwd_kernel<HC, true><<<grid, threads, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx, n_seq, sq,
+                                                                 sk, lengths, dr);
+  } else {
+    static bool configured[64] = {false};
+    if (cudaError_t e = set_max_dynamic_smem(attn_cross_fwd_kernel<HC, false>, max_smem, configured))
+      return cuda_fail(e, "attn_cross_fwd attr");
+    attn_cross_fwd_kernel<HC, false><<<grid, threads, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, ctx, n_seq, sq,
+                                                                  sk, lengths, dr);
+  }
   NRMS_LAUNCH_CHECK("attn_cross_fwd");
   return NRMS_OK;
 }
 
 int mha_attn_bwd(const MhaOperands& in, const float* d_ctx, float* dq, float* dk, float* dv, int64_t n_seq, int sq, int sk,
-                 const int32_t* lengths, int mode, cudaStream_t st) {
+                 const int32_t* lengths, int mode, cudaStream_t st, float p, uint64_t seed, uint64_t offset) {
   if (n_seq == 0) return NRMS_OK;
+  const amha::Drop dr{p, p > 0.f ? 1.f / (1.f - p) : 1.f, seed, offset};
   if (mode == NRMS_MODE_TF32) {
     const size_t smem = ((size_t)(2 * amha::round16(sq) + 2 * amha::round16(sk)) * amha::ST + 2 * amha::ZS) * sizeof(float);
-    amha::mha_bwd_kernel<<<dim3(mha_grid_x(n_seq, 16), H), 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx,
-                                                                            dq, dk, dv, n_seq, sq, sk, lengths);
+    const dim3 grid(mha_grid_x(n_seq, 16), H);
+    if (p > 0.f)
+      amha::mha_bwd_kernel<true><<<grid, 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx, dq, dk, dv, n_seq,
+                                                         sq, sk, lengths, dr);
+    else
+      amha::mha_bwd_kernel<false><<<grid, 32, smem, st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx, dq, dk, dv,
+                                                          n_seq, sq, sk, lengths, dr);
     NRMS_LAUNCH_CHECK("mha_bwd");
     return NRMS_OK;
   }
   constexpr int HC = MHA_HC_BWD;
   auto bytes = [](int a, int b) { return (size_t)(2 * (a + b) * HC * DH + 2 * HC * a * (b + 1)) * sizeof(float); };
-  static bool configured[64] = {false};
-  if (cudaError_t e = set_max_dynamic_smem(attn_cross_bwd_kernel<HC>, (int)bytes(MHA_MAXS, MHA_MAXS), configured))
-    return cuda_fail(e, "attn_cross_bwd attr");
   const int rows = sq > sk ? sq : sk;
-  attn_cross_bwd_kernel<HC><<<dim3(mha_grid_x(n_seq, 4), H / HC), (rows * HC + 31) / 32 * 32, bytes(sq, sk), st>>>(
-      in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx, dq, dk, dv, n_seq, sq, sk, lengths);
+  const dim3 grid(mha_grid_x(n_seq, 4), H / HC);
+  const int threads = (rows * HC + 31) / 32 * 32;
+  if (p > 0.f) {
+    static bool configured[64] = {false};
+    if (cudaError_t e = set_max_dynamic_smem(attn_cross_bwd_kernel<HC, true>, (int)bytes(MHA_MAXS, MHA_MAXS), configured))
+      return cuda_fail(e, "attn_cross_bwd attr");
+    attn_cross_bwd_kernel<HC, true><<<grid, threads, bytes(sq, sk), st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx,
+                                                                          dq, dk, dv, n_seq, sq, sk, lengths, dr);
+  } else {
+    static bool configured[64] = {false};
+    if (cudaError_t e = set_max_dynamic_smem(attn_cross_bwd_kernel<HC, false>, (int)bytes(MHA_MAXS, MHA_MAXS), configured))
+      return cuda_fail(e, "attn_cross_bwd attr");
+    attn_cross_bwd_kernel<HC, false><<<grid, threads, bytes(sq, sk), st>>>(in.q, in.ldq, in.k, in.ldk, in.v, in.ldv, d_ctx,
+                                                                           dq, dk, dv, n_seq, sq, sk, lengths, dr);
+  }
   NRMS_LAUNCH_CHECK("attn_cross_bwd");
   return NRMS_OK;
 }

@@ -173,11 +173,10 @@ static int encoder_core_fwd(const Stash& s, int64_t n_seq, int S, const float* w
   } else if (S == 20) e = launch_attention_fwd<20, 15>(s.qkv, s.c, n_seq, p2, seed, off2, st);
   else if (S == 50) e = launch_attention_fwd<50, 5>(s.qkv, s.c, n_seq, p2, seed, off2, st);
   else {
-    // user histories of any other length (1..64, no dropout): the run-time-length attention of attn_cross.cu over the
-    // stash's q|k|v rows, in the call's mode
-    NRMS_CHECK_ARG(p2 == 0.f, NRMS_E_INVALID, "no dropout at sequence length %d (user encoder only)", S);
+    // every other length (1..64: user histories, texts of nrms_text_encoder_*): the run-time-length attention of
+    // attn_cross.cu over the stash's q|k|v rows, in the call's mode, with dropout #2 when p2 > 0
     const MhaOperands op{s.qkv, s.qkv + D, s.qkv + 2 * D, D3, D3, D3};
-    if (int rc2 = mha_attn_fwd(op, s.c, n_seq, S, S, nullptr, mode, st)) return rc2;
+    if (int rc2 = mha_attn_fwd(op, s.c, n_seq, S, S, nullptr, mode, st, p2, seed, off2)) return rc2;
     e = cudaSuccess;
   }
   if (e != cudaSuccess) return cuda_fail(e, "attention_fwd");
@@ -333,10 +332,11 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
   } else if (S == 20) e = launch_attention_bwd<20, NRMS_ATTN_BWD_HC20>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
   else if (S == 50) e = launch_attention_bwd<50, 5>(s.qkv, w.d_c, w.d_qkv, n_seq, p2, seed, offset, st);
   else {
-    // other history lengths (user encoder only, no dropout): dq | dk | dv into dQKV with the pitch of the stash
-    NRMS_CHECK_ARG(p2 == 0.f, NRMS_E_INVALID, "no dropout at sequence length %d (user encoder only)", S);
+    // every other length: dq | dk | dv into dQKV with the pitch of the stash
     const MhaOperands op{s.qkv, s.qkv + D, s.qkv + 2 * D, D3, D3, D3};
-    if (int rc2 = mha_attn_bwd(op, w.d_c, w.d_qkv, w.d_qkv + D, w.d_qkv + 2 * D, n_seq, S, S, nullptr, mode, st)) return rc2;
+    if (int rc2 = mha_attn_bwd(op, w.d_c, w.d_qkv, w.d_qkv + D, w.d_qkv + 2 * D, n_seq, S, S, nullptr, mode, st, p2, seed,
+                               offset))
+      return rc2;
     e = cudaSuccess;
   }
   if (e != cudaSuccess) return cuda_fail(e, "attention_bwd");
@@ -344,9 +344,17 @@ static int encoder_core_bwd(const Stash& s, const BwdWs& w, const float* d_out, 
   return qkv_proj_bwd(qw, s.x, wqkv, rows, d_x, d_wqkv, d_bqkv, tc, dqkv_t_written, st);
 }
 
-// news encoder and nrms_mhsa_*: the compiled title / abstract lengths
+// nrms_news_encoder_* and nrms_mhsa_*: the compiled title / abstract lengths
 static int check_common(int S, int mode) {
   NRMS_CHECK_ARG(S == 20 || S == 50, NRMS_E_UNSUPPORTED, "sequence length %d unsupported (compiled: 20, 50)", S);
+  NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
+  return NRMS_OK;
+}
+
+// nrms_text_encoder_*: any title / abstract length up to 64 (20 and 50 keep their compiled kernels)
+constexpr int TEXT_MAXS = 64;
+static int check_text(int L, int mode) {
+  NRMS_CHECK_ARG(L >= 1 && L <= TEXT_MAXS, NRMS_E_UNSUPPORTED, "text length %d unsupported (1..%d)", L, TEXT_MAXS);
   NRMS_CHECK_ARG(mode == NRMS_MODE_FP32 || mode == NRMS_MODE_TF32, NRMS_E_INVALID, "bad mode %d", mode);
   return NRMS_OK;
 }
@@ -400,14 +408,17 @@ static int check_ln(const LnArgs* ln, bool bwd) {
   return NRMS_OK;
 }
 
+// The length rule is the caller's: check_common (nrms_news_encoder_*) or check_text (nrms_text_encoder_*)
+typedef int (*LengthRule)(int L, int mode);
+
 static int news_encoder_fwd_impl(const int64_t* tokens, int64_t n_titles, int L, const float* emb, int64_t num_words,
                                  const float* wqkv, const float* bqkv, const float* wa, const float* ba, const float* qa,
                                  float* out, void* stash, void* workspace, size_t workspace_bytes, float dropout_p,
                                  uint64_t seed, uint64_t offset, int mode, void* stream, const LnArgs* ln,
-                                 const int64_t* news_rows = nullptr) {
+                                 LengthRule length_rule, const int64_t* news_rows = nullptr) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (int rc = check_ln(ln, false)) return rc;
-  if (int rc = check_common(L, mode)) return rc;
+  if (int rc = length_rule(L, mode)) return rc;
   NRMS_CHECK_ARG(news_rows == nullptr || stash != nullptr, NRMS_E_UNSUPPORTED,
                  "the index-only form (token table + news rows) is the training form: pass a stash");
   NRMS_CHECK_ARG(n_titles >= 0 && num_words > 0, NRMS_E_INVALID, "bad sizes");
@@ -460,7 +471,7 @@ int nrms_news_encoder_fwd(const int64_t* tokens, int64_t n_titles, int L, const 
                           float* out, void* stash, void* workspace, size_t workspace_bytes, float dropout_p,
                           uint64_t seed, uint64_t offset, int mode, void* stream) {
   return news_encoder_fwd_impl(tokens, n_titles, L, emb, num_words, wqkv, bqkv, wa, ba, qa, out, stash, workspace,
-                               workspace_bytes, dropout_p, seed, offset, mode, stream, nullptr);
+                               workspace_bytes, dropout_p, seed, offset, mode, stream, nullptr, check_common);
 }
 
 int nrms_news_encoder_i32_fwd(const int32_t* tokens, int64_t n_titles, int L, const float* emb, int64_t num_words,
@@ -485,17 +496,18 @@ int nrms_news_encoder_ln_fwd(const int64_t* tokens, int64_t n_titles, int L, con
                              void* stream) {
   const LnArgs ln{ln_gamma, ln_beta, nullptr, nullptr};
   return news_encoder_fwd_impl(tokens, n_titles, L, emb, num_words, wqkv, bqkv, wa, ba, qa, out, stash, workspace,
-                               workspace_bytes, dropout_p, seed, offset, mode, stream, &ln);
+                               workspace_bytes, dropout_p, seed, offset, mode, stream, &ln, check_common);
 }
 
 static int news_encoder_bwd_impl(const float* d_out, const int64_t* tokens, int64_t n_titles, int L, int64_t num_words,
                                  const float* wqkv, const float* wa, const float* qa, const void* stash, float* d_emb,
                                  float* d_wqkv, float* d_bqkv, float* d_wa, float* d_ba, float* d_qa, void* workspace,
                                  size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset, int mode,
-                                 void* stream, const LnArgs* ln, const int64_t* news_rows = nullptr) {
+                                 void* stream, const LnArgs* ln, LengthRule length_rule,
+                                 const int64_t* news_rows = nullptr) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (int rc = check_ln(ln, true)) return rc;
-  if (int rc = check_common(L, mode)) return rc;
+  if (int rc = length_rule(L, mode)) return rc;
   if (n_titles == 0) return NRMS_OK;
   NRMS_CHECK_ARG(n_titles > 0 && num_words > 0, NRMS_E_INVALID, "bad sizes");
   NRMS_CHECK_ARG(d_out && tokens && wqkv && wa && qa && stash && d_emb && d_wqkv && d_bqkv && d_wa && d_ba && d_qa,
@@ -525,7 +537,8 @@ int nrms_news_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_t
                           size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset, int mode,
                           void* stream) {
   return news_encoder_bwd_impl(d_out, tokens, n_titles, L, num_words, wqkv, wa, qa, stash, d_emb, d_wqkv, d_bqkv, d_wa,
-                               d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream, nullptr);
+                               d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream, nullptr,
+                               check_common);
 }
 
 int nrms_news_encoder_ln_bwd(const float* d_out, const int64_t* tokens, int64_t n_titles, int L, int64_t num_words,
@@ -536,7 +549,8 @@ int nrms_news_encoder_ln_bwd(const float* d_out, const int64_t* tokens, int64_t 
                              void* stream) {
   const LnArgs ln{ln_gamma, nullptr, d_ln_gamma, d_ln_beta};
   return news_encoder_bwd_impl(d_out, tokens, n_titles, L, num_words, wqkv, wa, qa, stash, d_emb, d_wqkv, d_bqkv, d_wa,
-                               d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream, &ln);
+                               d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream, &ln,
+                               check_common);
 }
 
 int nrms_news_encoder_rows_fwd(const int64_t* token_table, int64_t n_news, const int64_t* news_rows, int64_t n_titles,
@@ -548,7 +562,7 @@ int nrms_news_encoder_rows_fwd(const int64_t* token_table, int64_t n_news, const
   NRMS_CHECK_ARG((ln_gamma == nullptr) == (ln_beta == nullptr), NRMS_E_INVALID, "LayerNorm needs both weight and bias");
   const LnArgs ln{ln_gamma, ln_beta, nullptr, nullptr};
   return news_encoder_fwd_impl(token_table, n_titles, L, emb, num_words, wqkv, bqkv, wa, ba, qa, out, stash, nullptr, 0,
-                               dropout_p, seed, offset, mode, stream, ln_gamma ? &ln : nullptr, news_rows);
+                               dropout_p, seed, offset, mode, stream, ln_gamma ? &ln : nullptr, check_common, news_rows);
 }
 
 int nrms_news_encoder_rows_bwd(const float* d_out, const int64_t* token_table, int64_t n_news, const int64_t* news_rows,
@@ -561,7 +575,41 @@ int nrms_news_encoder_rows_bwd(const float* d_out, const int64_t* token_table, i
   const LnArgs ln{ln_gamma, nullptr, d_ln_gamma, d_ln_beta};
   return news_encoder_bwd_impl(d_out, token_table, n_titles, L, num_words, wqkv, wa, qa, stash, d_emb, d_wqkv, d_bqkv,
                                d_wa, d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream,
-                               ln_gamma ? &ln : nullptr, news_rows);
+                               ln_gamma ? &ln : nullptr, check_common, news_rows);
+}
+
+// Any text length 1..64, one pair for every form: dense tokens [n_texts, L] (news_rows NULL, n_token_rows >= n_texts)
+// or the index-only form (text t is row news_rows[t] of the [n_token_rows, L] table, training only), with or without the
+// LayerNorm, training (a stash) or inference.  The length is checked before anything else; then each form is checked as
+// in nrms_news_encoder_{,ln_,rows_}fwd / bwd, and 20 / 50 run what those run.
+int nrms_text_encoder_fwd(const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows, int64_t n_texts, int L,
+                          const float* emb, int64_t num_words, const float* wqkv, const float* bqkv,
+                          const float* ln_gamma, const float* ln_beta, const float* wa, const float* ba, const float* qa,
+                          float* out, void* stash, void* workspace, size_t workspace_bytes, float dropout_p,
+                          uint64_t seed, uint64_t offset, int mode, void* stream) {
+  if (int rc = check_text(L, mode)) return rc;
+  NRMS_CHECK_ARG(news_rows ? (n_token_rows > 0) : (n_token_rows >= n_texts), NRMS_E_INVALID,
+                 "bad token rows: %lld for %lld texts", (long long)n_token_rows, (long long)n_texts);
+  NRMS_CHECK_ARG((ln_gamma == nullptr) == (ln_beta == nullptr), NRMS_E_INVALID, "LayerNorm needs both weight and bias");
+  const LnArgs ln{ln_gamma, ln_beta, nullptr, nullptr};
+  return news_encoder_fwd_impl(tokens, n_texts, L, emb, num_words, wqkv, bqkv, wa, ba, qa, out, stash, workspace,
+                               workspace_bytes, dropout_p, seed, offset, mode, stream, ln_gamma ? &ln : nullptr,
+                               check_text, news_rows);
+}
+
+int nrms_text_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows,
+                          int64_t n_texts, int L, int64_t num_words, const float* wqkv, const float* ln_gamma,
+                          const float* wa, const float* qa, const void* stash, float* d_emb, float* d_wqkv,
+                          float* d_bqkv, float* d_ln_gamma, float* d_ln_beta, float* d_wa, float* d_ba, float* d_qa,
+                          void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset,
+                          int mode, void* stream) {
+  if (int rc = check_text(L, mode)) return rc;
+  NRMS_CHECK_ARG(news_rows ? (n_token_rows > 0) : (n_token_rows >= n_texts), NRMS_E_INVALID,
+                 "bad token rows: %lld for %lld texts", (long long)n_token_rows, (long long)n_texts);
+  const LnArgs ln{ln_gamma, nullptr, d_ln_gamma, d_ln_beta};
+  return news_encoder_bwd_impl(d_out, tokens, n_texts, L, num_words, wqkv, wa, qa, stash, d_emb, d_wqkv, d_bqkv, d_wa,
+                               d_ba, d_qa, workspace, workspace_bytes, dropout_p, seed, offset, mode, stream,
+                               ln_gamma ? &ln : nullptr, check_text, news_rows);
 }
 
 static int user_encoder_fwd_impl(const float* x, int64_t n_rows, const int32_t* rows_idx, int64_t n_users, int S,

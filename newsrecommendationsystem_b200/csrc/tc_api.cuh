@@ -53,15 +53,17 @@ int attn_mma50_bwd(const float* qkv, const float* d_ctx, float* d_qkv, float* d_
 // attn_cross.cu: attention of the standalone block at 1 <= sq, sk <= 64 (self- or cross-attention), both modes.  q rows
 // [n_seq*sq] and k / v rows [n_seq*sk] of 300 used columns each, at their own pitches; ctx / d_ctx [n_seq*sq, 300].
 // lengths (nullable, int32 [n_seq]): the reference's `length` (sq == sk: keys j < length; sq == 1 < sk: all keys iff
-// length >= 1).  The backward writes dq / dk / dv with the pitches of q / k / v.
+// length >= 1).  The backward writes dq / dk / dv with the pitches of q / k / v.  p > 0: the news encoder's dropout #2
+// on the context (self-attention, sq == sk, the row index of the call keys the mask; p == 0 launches the kernels without
+// dropout).
 struct MhaOperands {
   const float *q, *k, *v;
   int64_t ldq, ldk, ldv;
 };
 int mha_attn_fwd(const MhaOperands& in, float* ctx, int64_t n_seq, int sq, int sk, const int32_t* lengths, int mode,
-                 cudaStream_t st);
+                 cudaStream_t st, float p = 0.f, uint64_t seed = 0, uint64_t offset = 0);
 int mha_attn_bwd(const MhaOperands& in, const float* d_ctx, float* dq, float* dk, float* dv, int64_t n_seq, int sq, int sk,
-                 const int32_t* lengths, int mode, cudaStream_t st);
+                 const int32_t* lengths, int mode, cudaStream_t st, float p = 0.f, uint64_t seed = 0, uint64_t offset = 0);
 // K1f (k1f_attn_pool.cu): table attention + additive pooling in one kernel (the context rows stay on the SM)
 int k1f_qk_bound(const void* table16, int64_t n_rows, float* bound, cudaStream_t st);
 int k1f_run(int S, int idx_kind, const void* table16, int64_t n_table_rows, const void* rows, int64_t n_seq,

@@ -5,7 +5,8 @@ The reference keeps pandas frames and dicts of per-news tensors and assembles ev
 
   news_parsed.tsv        (data_preprocess.py: header `id category subcategory title abstract title_entities
                           abstract_entities`; list columns are Python-list literals)
-      -> NewsTable: ids, `title` int64 [N, 20] (+ `abstract` [N, 50], `category` / `subcategory` [N] on request)
+      -> NewsTable: ids, `title` int64 [N, num_words_title] (+ `abstract` [N, num_words_abstract], `category` /
+         `subcategory` [N] on request); the text widths are those the file was written with
   behaviors_parsed.tsv   (data_preprocess.py:77-81: header `user clicked_news candidate_news clicked`)
       -> TrainRows: `cand_rows` int64 [B, 1+K], `hist_rows` int64 [B, num_clicked] -- news-row indices for
          `TrainStep.step_rows` (first 50 clicks, LEFT-padded, dataset.py:69-83; the pad index is row N of

@@ -39,8 +39,9 @@ class Exp1(torch.nn.Module):
         return self.click_predictor(vec[:, :n_cand], user_vector)
 
     def forward_rows(self, news_table, cand_rows, hist_rows):
-        """Index-only minibatch: news_table {attribute: device column} with N + 1 rows (title [N+1, 20], abstract
-        [N+1, 50], category / subcategory [N+1]; row N is the pad, as NewsTable.token_table_with_pad builds it),
+        """Index-only minibatch: news_table {attribute: device column} with N + 1 rows (title [N+1, num_words_title],
+        abstract [N+1, num_words_abstract], category / subcategory [N+1]; row N is the pad, as
+        NewsTable.token_table_with_pad builds it),
         cand_rows [B, 1+K] and hist_rows [B, N_clicked] news-row indices -> logits [B, 1+K]."""
         B, n_cand = cand_rows.shape
         dev = next(iter(news_table.values())).device

@@ -11,18 +11,24 @@ from ... import ops
 from ...config import resolve_mode
 from ..general.attention.multihead_self import MultiHeadSelfAttention
 from ..general.attention.additive import AdditiveAttention
+from ..NRMS.news_encoder import check_text_width
 
 
 # Philox keys of the text encoders' dropout streams.  Both encoders start at offset 0 each step, so with one key element
 # i of a title and element i of an abstract would drop together; the abstract gets its own key (the title keeps the
 # key it always had, so title-only models draw the same masks as before).
 DROPOUT_SEEDS = {"title": 0x5EED, "abstract": 0xAB57AC7}
+# configured length of each text attribute: (config attribute, the reference's default)
+TEXT_LENGTHS = {"title": ("num_words_title", 20), "abstract": ("num_words_abstract", 50)}
 
 
 class TextEncoder(nn.Module):
     def __init__(self, word_embedding, word_embedding_dim, num_attention_heads, query_vector_dim, dropout_probability,
-                 dropout_seed=0x5EED):
+                 dropout_seed=0x5EED, num_words=None):
+        """num_words: (config attribute, value) of the text's configured length, e.g. ("num_words_abstract", 50); texts
+        of another width than that value, 20 and 50 are refused.  None: no width rule beyond the library's 1..64."""
         super().__init__()
+        self.num_words = num_words
         self.word_embedding = word_embedding
         self.dropout_probability = dropout_probability
         self.multihead_self_attention = MultiHeadSelfAttention(word_embedding_dim, num_attention_heads)
@@ -37,9 +43,12 @@ class TextEncoder(nn.Module):
         return (int(self.dropout_seed) + 0x9E3779B97F4A7C15 * rank) & 0xFFFFFFFFFFFFFFFF
 
     def forward(self, text, news_rows=None):
-        """text: integer [n, num_words_text] (20 = title, 50 = abstract; training and inference) -> fp32 [n, 300].
+        """text: integer [n, num_words_text] (num_words_title / num_words_abstract, any 1..64; training and inference)
+        -> fp32 [n, 300].
         With news_rows (int64 [m] on the device) `text` is the device-resident token column [N + 1, L] of the news table
         and the call encodes its rows news_rows, read through the indices inside the gather / scatter kernels."""
+        if self.num_words is not None:
+            check_text_width(text, self.num_words[1], self.num_words[0])
         dev = self.word_embedding.weight.device
         if not text.is_cuda and text.numel():
             lo, hi = int(text.min()), int(text.max())
@@ -94,7 +103,8 @@ class NewsEncoder(nn.Module):
         text_names = sorted(set(config.dataset_attributes['news']) & {'title', 'abstract'})
         self.text_encoders = nn.ModuleDict({
             name: TextEncoder(word_embedding, config.word_embedding_dim, config.num_attention_heads,
-                              config.query_vector_dim, config.dropout_probability, DROPOUT_SEEDS[name])
+                              config.query_vector_dim, config.dropout_probability, DROPOUT_SEEDS[name],
+                              num_words=(TEXT_LENGTHS[name][0], getattr(config, *TEXT_LENGTHS[name])))
             for name in text_names
         })
         category_embedding = nn.Embedding(config.num_categories, config.category_embedding_dim, padding_idx=0)

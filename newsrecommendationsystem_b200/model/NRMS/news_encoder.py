@@ -9,6 +9,15 @@ from ..general.attention.multihead_self import MultiHeadSelfAttention
 from ..general.attention.additive import AdditiveAttention
 
 
+def check_text_width(text, configured, attr):
+    """A text tensor is as wide as the configured length, or one of the compiled lengths; any other width is not a
+    tokenisation of this model's data (the reference pads and truncates every text to the configured length)."""
+    width = text.shape[-1] if text.dim() else 0
+    if width != configured and width not in ops.TEXT_LENGTHS_COMPILED:
+        raise RuntimeError(f"text of {width} tokens: this model is configured for {attr} = {configured} "
+                           f"(texts of {configured} tokens, or of {' or '.join(map(str, ops.TEXT_LENGTHS_COMPILED))})")
+
+
 class NewsEncoder(nn.Module):
     def __init__(self, config, pretrained_word_embedding):
         super().__init__()
@@ -42,8 +51,10 @@ class NewsEncoder(nn.Module):
 
     def encode_tokens(self, title, news_rows=None):
         """title: integer tensor [n, num_words_title] (any device) -> fp32 [n, 300].  With news_rows (int64 [m] on the
-        device) `title` is the device-resident token table and the call encodes its rows news_rows (SURVEY 8 f2)."""
+        device) `title` is the device-resident token table and the call encodes its rows news_rows (SURVEY 8 f2).
+        The width is config.num_words_title (any 1..64; the reference's default 20), or one of the compiled 20 and 50."""
         self._check_dims()
+        check_text_width(title, getattr(self.config, "num_words_title", 20), "num_words_title")
         dev = self.word_embedding.weight.device
         if not title.is_cuda and title.numel():
             # host input (the reference's DataLoader path): nn.Embedding would raise on an id outside the vocabulary; the

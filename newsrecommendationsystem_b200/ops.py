@@ -15,6 +15,9 @@ from . import _lib
 from ._lib import check, ptr, stream_ptr
 
 D, H, QD = 300, 15, 200
+# Text lengths with compiled news-encoder kernels (nrms_news_encoder_*: the reference's num_words_title = 20 and
+# num_words_abstract = 50).  Every other length 1..64 runs through nrms_text_encoder_*.
+TEXT_LENGTHS_COMPILED = (20, 50)
 # An embedding parameter marked `_nrms_grad_sink` (optim.FusedAdam marks the parameters it owns) has a .grad that is a
 # live view of the optimizer's flat gradient: the news encoder's backward accumulates the embedding gradient directly
 # into it instead of returning a fresh 85 MB tensor for autograd to add.  Every other embedding gets its gradient
@@ -65,6 +68,23 @@ class _NewsEncoderFn(torch.autograd.Function):
         stash = None
         if needs_grad or rows is not None:
             stash = _bytes((lib.nrms_encoder_ln_stash_bytes if ln else lib.nrms_encoder_stash_bytes)(n, L), dev)
+        ctx.rows = rows
+        if L not in TEXT_LENGTHS_COMPILED:
+            # any other length: one entry point for the dense and index-only, plain and LayerNorm forms
+            if ln:
+                _require_cuda(ln_w, ln_b)
+            lnw_c, lnb_c = (_f32c(ln_w), _f32c(ln_b)) if ln else (None, None)
+            ws = _bytes(lib.nrms_encoder_fwd_workspace_bytes(n, L, mode, 1 if stash is not None else 0, emb_c.shape[0]),
+                        dev)
+            check(lib.nrms_text_encoder_fwd(ptr(tokens), n_news, ptr(rows), n, L, ptr(emb_c), emb_c.shape[0],
+                                            ptr(wqkv_c), ptr(bqkv_c), ptr(lnw_c), ptr(lnb_c), ptr(wa_c), ptr(ba_c),
+                                            ptr(qa_c), ptr(out), ptr(stash), ptr(ws), ws.numel(), float(dropout_p),
+                                            int(seed), int(offset), mode, stream_ptr(dev)), "nrms_text_encoder_fwd")
+            if needs_grad:
+                ctx.save_for_backward(tokens, wqkv_c, wa_c, qa_c, stash, *([lnw_c] if ln else []))
+                ctx.meta = (n, L, emb_c.shape[0], float(dropout_p), int(seed), int(offset), mode, ln)
+                ctx.emb_param = emb if (emb.is_leaf and getattr(emb, "_nrms_grad_sink", False)) else None
+            return out
         if rows is not None:
             lnw_c, lnb_c = (_f32c(ln_w), _f32c(ln_b)) if ln else (None, None)
             check(lib.nrms_news_encoder_rows_fwd(ptr(tokens), n_news, ptr(rows), n, L, ptr(emb_c), emb_c.shape[0],
@@ -75,9 +95,7 @@ class _NewsEncoderFn(torch.autograd.Function):
                 ctx.save_for_backward(tokens, wqkv_c, wa_c, qa_c, stash, *([lnw_c] if ln else []))
                 ctx.meta = (n, L, emb_c.shape[0], float(dropout_p), int(seed), int(offset), mode, ln)
                 ctx.emb_param = emb if (emb.is_leaf and getattr(emb, "_nrms_grad_sink", False)) else None
-                ctx.rows = rows
             return out
-        ctx.rows = None
         ws_bytes = lib.nrms_encoder_fwd_workspace_bytes(n, L, mode, 1 if needs_grad else 0, emb_c.shape[0])
         ws = _bytes(ws_bytes, dev)
         if ln:
@@ -126,7 +144,13 @@ class _NewsEncoderFn(torch.autograd.Function):
             d_lnw = torch.zeros((D,), dtype=torch.float32, device=dev)
             d_lnb = torch.zeros((D,), dtype=torch.float32, device=dev)
         rows = getattr(ctx, "rows", None)
-        if rows is not None:
+        if L not in TEXT_LENGTHS_COMPILED:
+            check(lib.nrms_text_encoder_bwd(ptr(d_out), ptr(tokens), tokens.shape[0], ptr(rows), n, L, V, ptr(wqkv),
+                                            ptr(lnw) if ln else None, ptr(wa), ptr(qa), ptr(stash), ptr(d_emb),
+                                            ptr(d_wqkv), ptr(d_bqkv), ptr(d_lnw), ptr(d_lnb), ptr(d_wa), ptr(d_ba),
+                                            ptr(d_qa), ptr(ws), ws.numel(), p, seed, offset, mode, stream_ptr(dev)),
+                  "nrms_text_encoder_bwd")
+        elif rows is not None:
             check(lib.nrms_news_encoder_rows_bwd(ptr(d_out), ptr(tokens), tokens.shape[0], ptr(rows), n, L, V, ptr(wqkv),
                                                  ptr(lnw) if ln else None, ptr(wa), ptr(qa), ptr(stash), ptr(d_emb),
                                                  ptr(d_wqkv), ptr(d_bqkv), ptr(d_lnw), ptr(d_lnb), ptr(d_wa), ptr(d_ba),
@@ -310,13 +334,16 @@ def user_encoder_indexed(table, rows, wqkv, bqkv, wa, ba, qa, mode=_lib.MODE_TF3
 
 @torch.no_grad()
 def news_encoder_i32(tokens, emb, wqkv, bqkv, wa, ba, qa):
-    """Tensor-mode, inference-only news encoder over int32 token ids [n, L] (evaluate's pre-tokenised table)."""
+    """Tensor-mode, inference-only news encoder over int32 token ids [n, L] (evaluate's pre-tokenised table).  The
+    int32 kernels are compiled for L = 20 and 50; any other length widens the ids and runs news_encoder in tensor mode."""
     lib = _lib.load()
     _require_cuda(tokens, emb)
     if tokens.dtype != torch.int32:
         raise RuntimeError("news_encoder_i32 takes int32 token ids")
     tokens = tokens.contiguous()
     n, L = tokens.shape
+    if L not in TEXT_LENGTHS_COMPILED:
+        return news_encoder(tokens.long(), emb, wqkv, bqkv, wa, ba, qa, mode=_lib.MODE_TF32)
     dev = emb.device
     out = torch.empty((n, D), dtype=torch.float32, device=dev)
     args = [_f32c(t) for t in (emb, wqkv, bqkv, wa, ba, qa)]

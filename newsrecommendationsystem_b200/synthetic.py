@@ -6,8 +6,8 @@ Shapes follow the reference's data contracts:
   * impressions  history = first <=50 clicks, LEFT-padded (`evaluate.py:111-124`),
     candidates as CSR (offsets, rows, labels) replacing the "N123-1 N456-0" strings
     (`evaluate.py:251-263`)
-  * training batch  int64 [B, 1+K, 20] candidates (column 0 = the positive,
-    `data_preprocess.py:63-66`) and int64 [B, 50, 20] clicked titles, left-padded with
+  * training batch  int64 [B, 1+K, L] candidates (column 0 = the positive,
+    `data_preprocess.py:63-66`) and int64 [B, 50, L] clicked titles (L = the table's title width), left-padded with
     all-zero titles (`dataset.py:47,75-83`).
 """
 from __future__ import annotations
