@@ -18,6 +18,8 @@
  *   nrms_news_encoder_rows_fwd/bwd  NewsEncoder over an index-only minibatch    src/dataset.py:17-85, src/train.py:118-124
  *   nrms_text_encoder_fwd/bwd   NewsEncoder.forward / Exp1 TextEncoder at any text length 1..64
  *                               src/model/NRMS/news_encoder.py:27-48, src/model/Exp1/news_encoder.py:10-34
+ *   nrms_cnn_text_fwd/bwd       NAML TextEncoder.forward (CNN, ReLU, additive pooling) at text length 1..64
+ *                               src/model/NAML/news_encoder.py:9-40
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
  *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
  *   nrms_mha_fwd/bwd            MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries / keys  (same lines)
@@ -288,6 +290,36 @@ int nrms_text_encoder_bwd(const float* d_out, const int64_t* tokens, int64_t n_t
                           float* d_bqkv, float* d_ln_gamma, float* d_ln_beta, float* d_wa, float* d_ba, float* d_qa,
                           void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed, uint64_t offset,
                           int mode, void* stream);
+
+/* ---- NAML's CNN text encoder (src/model/NAML/news_encoder.py:9-40) ---------------------------------------
+ * TextEncoder.forward: x = dropout(word_embedding(text)); c = Conv2d(1, 300, (3, 300), padding=(1, 0))(x); a =
+ * dropout(relu(c)); out = AdditiveAttention(a) -- at any text length L = 1..64.  conv_w is CNN.weight [300, 1, 3, 300]
+ * viewed as [300, 900] (w*300 + d order), conv_b [300].  The conv's padding rows are zeros, not the embedding of token 0.
+ *   - news_rows NULL: dense tokens int64 [n_token_rows, L], text t = row t (n_token_rows >= n_texts); news_rows non-NULL:
+ *     text t = row news_rows[t] of the [n_token_rows, L] token column (the index-only minibatch), in either form below;
+ *   - stash non-NULL (nrms_cnn_text_stash_bytes): training; its layout, each field starting at a 256-byte boundary, is
+ *     X [rows, 300] (embedding rows after dropout #1) | H [rows, 300] (relu(conv), before dropout #2) | A [rows, 300]
+ *     (H after dropout #2) | T [rows, 200] | w [rows] (the additive block's tanh activations and weights), rows =
+ *     n_texts * L.  NULL: inference, a chunk of texts at a time inside the workspace.
+ *   - workspace: nrms_cnn_text_fwd_workspace_bytes(n_texts, L, mode, training) / nrms_cnn_text_bwd_workspace_bytes.
+ * Dropout: element (row, col) of site 1 (the embedded rows) is dropout_mask4(row * 300 + col, stream 1) and of site 2
+ * (relu(conv)) dropout_mask4(row * 300 + col, stream 2), row = text * L + i: the streams and counters of the NRMS encoder,
+ * so a text's masks depend only on its row and a chunked pass equals a single one.  The tensor mode runs the conv's three
+ * taps as one [rows, 300] x [300, 900] tcgen05 projection, followed by a shift-add epilogue (bias, ReLU, dropout #2).
+ * L outside 1..64 returns NRMS_E_UNSUPPORTED before any pointer check and before any CUDA call.  The backward ACCUMULATES
+ * into d_emb (row 0 = padding_idx untouched), d_conv_w [300, 900], d_conv_b, d_wa, d_ba, d_qa. */
+size_t nrms_cnn_text_stash_bytes(int64_t n_texts, int L);
+size_t nrms_cnn_text_fwd_workspace_bytes(int64_t n_texts, int L, int mode, int training);
+size_t nrms_cnn_text_bwd_workspace_bytes(int64_t n_texts, int L, int mode);
+int nrms_cnn_text_fwd(const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows, int64_t n_texts, int L,
+                      const float* emb, int64_t num_words, const float* conv_w, const float* conv_b, const float* wa,
+                      const float* ba, const float* qa, float* out, void* stash, void* workspace, size_t workspace_bytes,
+                      float dropout_p, uint64_t seed, uint64_t offset, int mode, void* stream);
+int nrms_cnn_text_bwd(const float* d_out, const int64_t* tokens, int64_t n_token_rows, const int64_t* news_rows,
+                      int64_t n_texts, int L, int64_t num_words, const float* conv_w, const float* wa, const float* qa,
+                      const void* stash, float* d_emb, float* d_conv_w, float* d_conv_b, float* d_wa, float* d_ba,
+                      float* d_qa, void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed,
+                      uint64_t offset, int mode, void* stream);
 
 /* ---- model/Exp1 blocks (SURVEY 8 f3) ------------------------------------------------------
  * ElementEncoder.forward = relu(linear(embedding(element)))  (src/model/Exp1/news_encoder.py:37-44):

@@ -66,6 +66,13 @@ SIGNATURES = {
                                      _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
     "nrms_text_encoder_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                      _vp, _vp, _vp, _vp, _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
+    "nrms_cnn_text_stash_bytes": (_sz, [_i64, _i32]),
+    "nrms_cnn_text_fwd_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32]),
+    "nrms_cnn_text_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "nrms_cnn_text_fwd": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                 _f32, _u64, _u64, _i32, _vp]),
+    "nrms_cnn_text_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                 _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
     "nrms_element_encoder_table_bytes": (_sz, [_i64]),
     "nrms_element_encoder_fwd": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "nrms_element_encoder_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

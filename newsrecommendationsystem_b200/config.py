@@ -54,6 +54,14 @@ class Exp1Config(BaseConfig):
     ensemble_factor = 1
 
 
+class NAMLConfig(BaseConfig):
+    """reference src/config.py (NAMLConfig): CNN text encoders over title and abstract, element encoders over category
+    and subcategory."""
+    dataset_attributes = {"news": ['category', 'subcategory', 'title', 'abstract'], "record": []}
+    num_filters = 300
+    window_size = 3
+
+
 def resolve_mode(config=None, override=None):
     from . import _lib
     name = override or getattr(config, "precision", None) or os.environ.get("NRMS_B200_PRECISION", "tf32")

@@ -372,6 +372,9 @@ def evaluate(model, directory, num_workers=0, max_count=None):
     import os
     import sys
     from . import data
+    from .model.NAML import NAML
+    if isinstance(model, NAML):
+        return _evaluate_columns(model, directory, max_count)
     news = data.load_news_parsed(os.path.join(directory, "news_parsed.tsv"))
     # the history length the model was built for (a model without a config: the reference's default, 50)
     num_clicked = int(getattr(getattr(model, "config", None), "num_clicked_news_a_user", 50))
@@ -381,4 +384,62 @@ def evaluate(model, directory, num_workers=0, max_count=None):
     if max_count is not None and max_count >= sys.maxsize:
         max_count = None
     return evaluate_tensors(model, inputs, max_count=max_count)
+
+
+@torch.no_grad()
+def _evaluate_columns(model, directory, max_count=None):
+    """evaluate() for a model whose news encoder reads several news columns (NAML): the columns of
+    `model.config.dataset_attributes['news']` go to the device once, `get_news_vector` encodes the table, the user vectors
+    come from `user_encoder.forward_indexed` over the fp32 table, then scoring and metrics as in evaluate_tensors (one
+    device, tensor-mode scoring on the fp16 copy of the table)."""
+    import os
+    from . import data
+    attrs = list(model.config.dataset_attributes["news"])
+    news = data.load_news_parsed(os.path.join(directory, "news_parsed.tsv"), attributes=attrs)
+    num_clicked = int(model.config.num_clicked_news_a_user)
+    ev = data.load_behaviors(os.path.join(directory, "behaviors.tsv"), news, num_clicked=num_clicked)
+    dev = next(model.parameters()).device
+    n = len(news)
+    host = EvalHost(news.columns[attrs[0]].reshape(n, -1), ev.hist_rows, ev.cand_offsets, ev.cand_rows, ev.labels,
+                    news_ids=news.ids)
+    cols = {a: torch.as_tensor(news.columns[a]).to(dev) for a in attrs}
+    return evaluate_columns(model, cols, host, max_count)
+
+
+@torch.no_grad()
+def evaluate_columns(model, cols, host, max_count=None):
+    """The device part of evaluate() for a multi-column model: cols {attribute: device column with one row per news},
+    host = the EvalHost of the impressions -> (AUC, MRR, nDCG@5, nDCG@10)."""
+    import sys
+    from .config import resolve_mode
+    from . import _lib
+    dev = next(model.parameters()).device
+    n = host.n_news
+    was_training = model.training
+    model.eval()
+    try:
+        table = torch.zeros((n + PAD_REPLICAS, ops.D), dtype=torch.float32, device=dev)
+        if n:
+            table[:n] = model.get_news_vector(cols)
+    finally:
+        model.train(was_training)
+    n_imp = host.n_impressions
+    if max_count is not None and max_count < sys.maxsize:
+        n_imp = max(0, min(n_imp, int(max_count) - 1))
+    if n_imp == 0:
+        return tuple(float("nan") for _ in range(4))
+    c1 = int(host.cand_offsets_host[n_imp])
+    hist = host.hist_rows[:n_imp].to(dev)
+    cand_rows, labels = host.cand_rows[:c1].to(dev), host.labels[:c1].to(dev)
+    offs = host.cand_offsets[:n_imp + 1].to(dev)
+    user_vec = model.user_encoder.forward_indexed(table, hist)
+    ue = model.user_encoder
+    if resolve_mode(ue.config, ue.precision) == _lib.MODE_TF32:
+        scores = ops.score_csr_f16(ops.pack_rows_f16(table), cand_rows, offs, user_vec)
+    else:
+        scores = ops.score_csr(table, cand_rows, offs, user_vec)
+    _, sums = ops.rank_metrics(scores, labels, offs)
+    s = sums.cpu().numpy()
+    with np.errstate(all="ignore"):
+        return tuple(float(x) for x in (s[:4] / s[4:]))
 

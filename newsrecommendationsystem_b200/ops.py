@@ -682,6 +682,79 @@ def additive_attention(c, wa, ba, qa, mode=_lib.MODE_TF32):
     return _AdditiveFn.apply(c, wa, ba, qa, mode, torch.is_grad_enabled())
 
 
+CNN_TEXT_MAX_LEN = 64
+
+
+class _CnnTextEncoderFn(torch.autograd.Function):
+    """NAML TextEncoder.forward (reference src/model/NAML/news_encoder.py:9-40): embedding, dropout, Conv2d(1, 300,
+    (3, 300), padding=(1, 0)), ReLU, dropout, additive pooling -- nrms_cnn_text_fwd / _bwd.  conv_w is CNN.weight viewed
+    as [300, 900].  The embedding gradient goes straight into an optimizer-owned gradient buffer when there is one, as
+    in _NewsEncoderFn."""
+
+    @staticmethod
+    def forward(ctx, tokens, emb, conv_w, conv_b, wa, ba, qa, dropout_p, seed, offset, mode, track_grad, news_rows):
+        lib = _lib.load()
+        _require_cuda(tokens, emb, conv_w, conv_b, wa, ba, qa, news_rows)
+        tokens = tokens.contiguous()
+        if tokens.dtype != torch.int64:
+            tokens = tokens.long()
+        rows = None if news_rows is None else news_rows.contiguous().long().view(-1)
+        n_tok_rows, L = tokens.shape
+        n = n_tok_rows if rows is None else rows.numel()
+        dev = emb.device
+        emb_c, w_c, b_c, wa_c, ba_c, qa_c = map(_f32c, (emb, conv_w, conv_b, wa, ba, qa))
+        out = torch.empty((n, D), dtype=torch.float32, device=dev)
+        needs_grad = track_grad and any(ctx.needs_input_grad)
+        stash = _bytes(lib.nrms_cnn_text_stash_bytes(n, L), dev) if needs_grad else None
+        ws = _bytes(lib.nrms_cnn_text_fwd_workspace_bytes(n, L, mode, 1 if needs_grad else 0), dev)
+        check(lib.nrms_cnn_text_fwd(ptr(tokens), n_tok_rows, ptr(rows), n, L, ptr(emb_c), emb_c.shape[0], ptr(w_c),
+                                    ptr(b_c), ptr(wa_c), ptr(ba_c), ptr(qa_c), ptr(out), ptr(stash), ptr(ws), ws.numel(),
+                                    float(dropout_p), int(seed), int(offset), mode, stream_ptr(dev)), "nrms_cnn_text_fwd")
+        if needs_grad:
+            ctx.save_for_backward(tokens, rows, w_c, wa_c, qa_c, stash)
+            ctx.meta = (n, L, emb_c.shape[0], float(dropout_p), int(seed), int(offset), mode)
+            ctx.emb_param = emb if (emb.is_leaf and getattr(emb, "_nrms_grad_sink", False)) else None
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        lib = _lib.load()
+        n, L, V, p, seed, offset, mode = ctx.meta
+        tokens, rows, conv_w, wa, qa, stash = ctx.saved_tensors
+        dev = d_out.device
+        d_out = d_out.contiguous().float()
+        sink = getattr(ctx, "emb_param", None)
+        g = sink.grad if sink is not None else None
+        in_place = (g is not None and g.dtype == torch.float32 and g.is_contiguous() and tuple(g.shape) == (V, D)
+                    and g.device == dev)
+        d_emb = g if in_place else torch.zeros((V, D), dtype=torch.float32, device=dev)
+        d_w = torch.zeros((D, 3 * D), dtype=torch.float32, device=dev)
+        d_b = torch.zeros((D,), dtype=torch.float32, device=dev)
+        d_wa = torch.zeros((QD, D), dtype=torch.float32, device=dev)
+        d_ba = torch.zeros((QD,), dtype=torch.float32, device=dev)
+        d_qa = torch.zeros((QD,), dtype=torch.float32, device=dev)
+        ws = _bytes(lib.nrms_cnn_text_bwd_workspace_bytes(n, L, mode), dev)
+        check(lib.nrms_cnn_text_bwd(ptr(d_out), ptr(tokens), tokens.shape[0], ptr(rows), n, L, V, ptr(conv_w), ptr(wa),
+                                    ptr(qa), ptr(stash), ptr(d_emb), ptr(d_w), ptr(d_b), ptr(d_wa), ptr(d_ba), ptr(d_qa),
+                                    ptr(ws), ws.numel(), p, seed, offset, mode, stream_ptr(dev)), "nrms_cnn_text_bwd")
+        return (None, (None if in_place else d_emb), d_w, d_b, d_wa, d_ba, d_qa, None, None, None, None, None, None)
+
+
+def cnn_text_encoder(tokens, emb, conv_w, conv_b, wa, ba, qa, dropout_p=0.0, seed=0, offset=0, mode=_lib.MODE_TF32,
+                     news_rows=None):
+    """NAML's CNN text encoder, autograd-connected.  tokens: integer [n, L] (L = 1..64), emb [num_words, 300], conv_w
+    [300, 900] (CNN.weight [300, 1, 3, 300] viewed flat), conv_b [300], wa [200, 300], ba / qa [200] -> fp32 [n, 300].
+    news_rows (int64 [m], device): `tokens` is a device-resident token column and text t of the call is its row
+    news_rows[t], read through the index inside the gather / scatter kernels."""
+    L = tokens.shape[-1]
+    if tokens.dim() != 2 or not 1 <= L <= CNN_TEXT_MAX_LEN:
+        raise RuntimeError(f"cnn_text_encoder takes [n, L] tokens with L in 1..{CNN_TEXT_MAX_LEN}, got {tuple(tokens.shape)}")
+    if tuple(conv_w.shape) != (D, 3 * D):
+        raise RuntimeError(f"conv_w must be CNN.weight viewed as [{D}, {3 * D}], got {tuple(conv_w.shape)}")
+    return _CnnTextEncoderFn.apply(tokens, emb, conv_w, conv_b, wa, ba, qa, dropout_p, seed, offset, mode,
+                                   torch.is_grad_enabled(), news_rows)
+
+
 class _ElementEncoderFn(torch.autograd.Function):
     """ElementEncoder.forward = relu(linear(embedding(element)))  (reference src/model/Exp1/news_encoder.py:37-44)."""
 
