@@ -12,6 +12,7 @@
  *               AdditiveAttention.forward        src/model/general/attention/additive.py:27-53)
  *   nrms_score_fwd/bwd          DotProductClickPredictor.forward  src/model/general/click_predictor/dot_product.py:8-19
  *   nrms_score_csr              the per-impression get_prediction loop   src/evaluate.py:245-260
+ *   nrms_score_csr_width        the same loop at width 900 (LSTUR)
  *   nrms_ce_loss_fwd_bwd        CrossEntropyLoss(y_pred, zeros)    src/train.py:126,205-206
  *   nrms_adam_step              torch.optim.Adam(lr=1e-4).step()   src/train.py:127-128,233 (AdamW: decoupled=1)
  *   nrms_rank_metrics           calculate_single_user_metric + nanmean  src/evaluate.py:24-42,160-168,270-272
@@ -20,6 +21,9 @@
  *                               src/model/NRMS/news_encoder.py:27-48, src/model/Exp1/news_encoder.py:10-34
  *   nrms_cnn_text_fwd/bwd       NAML TextEncoder.forward (CNN, ReLU, additive pooling) at text length 1..64
  *                               src/model/NAML/news_encoder.py:9-40
+ *   nrms_gru_fwd/bwd            LSTUR UserEncoder.forward: nn.GRU over pack_padded_sequence  src/model/LSTUR/user_encoder.py
+ *   nrms_rows_fwd/bwd           nn.Embedding rows (LSTUR category / user embedding; the user rows under F.dropout2d)
+ *                               src/model/LSTUR/news_encoder.py, src/model/LSTUR/__init__.py
  *   nrms_recommend_user         the single-user path of the demo            src/recommend.py:245-341
  *   nrms_mhsa_fwd/bwd, nrms_mhsa_masked_fwd  MultiHeadSelfAttention.forward(Q, length=...)  multihead_self.py:46-76
  *   nrms_mha_fwd/bwd            MultiHeadSelfAttention.forward(Q, K, V, length) at 1..64 queries / keys  (same lines)
@@ -321,6 +325,46 @@ int nrms_cnn_text_bwd(const float* d_out, const int64_t* tokens, int64_t n_token
                       float* d_qa, void* workspace, size_t workspace_bytes, float dropout_p, uint64_t seed,
                       uint64_t offset, int mode, void* stream);
 
+/* ---- LSTUR (src/model/LSTUR) -------------------------------------------------------------------------------------
+ * nrms_gru_fwd: h_out [n_seq, H] = the last hidden state of a one-layer nn.GRU(I, H) (torch's gate order r | z | n in
+ * the rows of w_ih [3H, I], w_hh [3H, H], b_ih / b_hh [3H]) run over steps t < lengths[s] of sequence s, from h0
+ * (NULL: zeros) -- what the reference gets from gru(pack_padded_sequence(x, lengths, batch_first=True)).  A length of 0
+ * runs no step (h_out = h0); the reference's caller turns 0 into 1 before the call.
+ *   - (I, H) must be (900, 900) or (900, 450); anything else returns NRMS_E_UNSUPPORTED before any other check.
+ *   - lengths_host: int32 [n_seq] in HOST memory, each in 0..T.  The sequences are sorted by length on the host, so
+ *     step t runs over the sequences still going (sum(lengths) rows of work in all).
+ *   - x_rows NULL: x is dense [n_seq * T, I] (n_x_rows = n_seq * T), step t of sequence s reads row s*T + t.
+ *     x_rows non-NULL (int64 [n_seq * T], device): x is a table [n_x_rows, I] and step t of sequence s reads its row
+ *     x_rows[s*T + t]; the input projection runs once over the table rows.  Inference only.  Every x_rows entry must
+ *     lie in [0, n_x_rows); the caller guarantees it (the kernels do not check it).
+ *   - stash non-NULL (nrms_gru_stash_bytes): training, dense x only; it keeps the sorted order, h_{t-1} and r | z | n |
+ *     W_hn h_{t-1} + b_hn of every step.  workspace: nrms_gru_fwd_workspace_bytes(n_seq, T, n_x_rows, I, H).
+ *   - mode: NRMS_MODE_FP32 (CUDA cores) or NRMS_MODE_TF32 (tcgen05 GEMMs with TF32 operands, fp32 accumulation; the
+ *     carried hidden state stays fp32).
+ * nrms_gru_bwd: from d_out [n_seq, H] and the forward's stash, WRITES d_x [n_seq * T, I] (nullable; zero at steps past a
+ * length) and d_h0 [n_seq, H] (nullable), and ACCUMULATES into d_w_ih, d_w_hh, d_b_ih, d_b_hh.  workspace:
+ * nrms_gru_bwd_workspace_bytes(n_seq, T, I, H, mode). */
+size_t nrms_gru_stash_bytes(int64_t n_seq, int T, int I, int H);
+size_t nrms_gru_fwd_workspace_bytes(int64_t n_seq, int T, int64_t n_x_rows, int I, int H);
+size_t nrms_gru_bwd_workspace_bytes(int64_t n_seq, int T, int I, int H, int mode);
+int nrms_gru_fwd(const float* x, int64_t n_x_rows, const int64_t* x_rows, int64_t n_seq, int T, int I, int H,
+                 const int32_t* lengths_host, const float* h0, const float* w_ih, const float* w_hh, const float* b_ih,
+                 const float* b_hh, float* h_out, void* stash, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream);
+int nrms_gru_bwd(const float* d_out, const float* x, int64_t n_seq, int T, int I, int H, const int32_t* lengths_host,
+                 const float* w_ih, const float* w_hh, const void* stash, float* d_x, float* d_h0, float* d_w_ih,
+                 float* d_w_hh, float* d_b_ih, float* d_b_hh, void* workspace, size_t workspace_bytes, int mode,
+                 void* stream);
+/* nrms_rows_fwd: out[i, :width] (row pitch ld_out) = src[r(i), :width] * m(i), r(i) = idx[i] (int64, device) or i when
+ * idx is NULL (a strided row copy), src rows of pitch ld_src.  m(i) is a whole-row dropout mask: 0 with probability
+ * dropout_p, else 1 / (1 - dropout_p), from Philox counter (i + offset, stream 3) keyed by seed (lane x) -- F.dropout2d
+ * over a [1, n, width] input.  Any width (450 and 900 are not multiples of 4).
+ * nrms_rows_bwd: d_src[idx[i], :width] += d_out[i, :width] * m(i), skipping rows with idx[i] == padding_idx (-1: none). */
+int nrms_rows_fwd(const float* src, int64_t n_src_rows, int64_t ld_src, const int64_t* idx, int64_t n, int width,
+                  float* out, int64_t ld_out, float dropout_p, uint64_t seed, uint64_t offset, void* stream);
+int nrms_rows_bwd(const float* d_out, int64_t ld_dout, const int64_t* idx, int64_t n, int width, float* d_src,
+                  int64_t ld_dsrc, int64_t padding_idx, float dropout_p, uint64_t seed, uint64_t offset, void* stream);
+
 /* ---- model/Exp1 blocks (SURVEY 8 f3) ------------------------------------------------------
  * ElementEncoder.forward = relu(linear(embedding(element)))  (src/model/Exp1/news_encoder.py:37-44):
  * idx int64 [n] in [0, num_categories), emb [num_categories, 100], w [300, 100], b [300] -> out [n, 300].
@@ -394,6 +438,10 @@ int nrms_score_bwd(const float* d_scores, const float* cand, const float* user,
  * scores[k] = table[cand_rows[k], :] . user_vec[i, :]   (X = 300). */
 int nrms_score_csr(const float* table, const int32_t* cand_rows, const int64_t* offsets,
                    const float* user_vec, int64_t n_impressions, float* scores, void* stream);
+/* nrms_score_csr at width 300 or 900 (LSTUR's news and user vectors): table [*, width], user_vec [n_impressions, width],
+ * the same CSR layout and arithmetic.  Any other width returns NRMS_E_UNSUPPORTED; nrms_score_csr is width 300. */
+int nrms_score_csr_width(const float* table, const int32_t* cand_rows, const int64_t* offsets, const float* user_vec,
+                         int64_t n_impressions, int width, float* scores, void* stream);
 /* Tensor-mode scoring: the candidate rows are read from an fp16 copy of the table (half the bytes per candidate, fp32
  * accumulation).  nrms_pack_rows_f16 writes that copy: dst16 = (n_rows + 1) * 640 bytes, rows of 320 halfs. */
 int nrms_pack_rows_f16(const float* src, int64_t n_rows, void* dst16, void* stream);

@@ -5,9 +5,10 @@ hand-written sm_100a library `libnrms_b200.so` through the C-ABI in `include/nrm
 Importing the package does not load CUDA; the first op call does, and raises if the library
 is missing (there is no CPU fallback).
 """
-from .config import NRMSConfig, NRMSLNConfig, Exp1Config, NAMLConfig, BaseConfig  # noqa: F401
+from .config import NRMSConfig, NRMSLNConfig, Exp1Config, NAMLConfig, LSTURConfig, BaseConfig  # noqa: F401
 
-__all__ = ["NRMSConfig", "NRMSLNConfig", "Exp1Config", "NAMLConfig", "BaseConfig", "NRMS", "Exp1", "NAML", "NewsEncoder",
+__all__ = ["NRMSConfig", "NRMSLNConfig", "Exp1Config", "NAMLConfig", "LSTURConfig", "BaseConfig", "NRMS", "Exp1", "NAML",
+           "LSTUR", "NewsEncoder",
            "UserEncoder", "DotProductClickPredictor"]
 
 
@@ -21,6 +22,9 @@ def __getattr__(name):
     if name == "NAML":
         from .model.NAML import NAML
         return NAML
+    if name == "LSTUR":
+        from .model.LSTUR import LSTUR
+        return LSTUR
     if name == "NewsEncoder":
         from .model.NRMS.news_encoder import NewsEncoder
         return NewsEncoder

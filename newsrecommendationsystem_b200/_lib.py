@@ -73,6 +73,15 @@ SIGNATURES = {
                                  _f32, _u64, _u64, _i32, _vp]),
     "nrms_cnn_text_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                  _vp, _sz, _f32, _u64, _u64, _i32, _vp]),
+    "nrms_gru_stash_bytes": (_sz, [_i64, _i32, _i32, _i32]),
+    "nrms_gru_fwd_workspace_bytes": (_sz, [_i64, _i32, _i64, _i32, _i32]),
+    "nrms_gru_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32, _i32]),
+    "nrms_gru_fwd": (_i32, [_vp, _i64, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                            _i32, _vp]),
+    "nrms_gru_bwd": (_i32, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                            _i32, _vp]),
+    "nrms_rows_fwd": (_i32, [_vp, _i64, _i64, _vp, _i64, _i32, _vp, _i64, _f32, _u64, _u64, _vp]),
+    "nrms_rows_bwd": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp, _i64, _i64, _f32, _u64, _u64, _vp]),
     "nrms_element_encoder_table_bytes": (_sz, [_i64]),
     "nrms_element_encoder_fwd": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "nrms_element_encoder_bwd": (_i32, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -87,6 +96,7 @@ SIGNATURES = {
     "nrms_score_fwd": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _vp]),
     "nrms_score_bwd": (_i32, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     "nrms_score_csr": (_i32, [_vp, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "nrms_score_csr_width": (_i32, [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp]),
     "nrms_pack_rows_f16": (_i32, [_vp, _i64, _vp, _vp]),
     "nrms_score_csr_f16": (_i32, [_vp, _vp, _vp, _vp, _i64, _vp, _vp]),
     "nrms_ce_loss_fwd_bwd": (_i32, [_vp, _i64, _i32, _f32, _vp, _vp, _vp]),

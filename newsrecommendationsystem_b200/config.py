@@ -62,6 +62,17 @@ class NAMLConfig(BaseConfig):
     window_size = 3
 
 
+class LSTURConfig(BaseConfig):
+    """reference src/config.py (LSTURConfig): NAML's CNN title encoder plus raw category rows, and a GRU user encoder
+    started from (ini) or concatenated with (con) a learned per-user embedding."""
+    dataset_attributes = {"news": ['category', 'subcategory', 'title'], "record": ['user', 'clicked_news_length']}
+    num_filters = 300
+    window_size = 3
+    long_short_term_method = 'ini'
+    # See paper for more detail
+    masking_probability = 0.5
+
+
 def resolve_mode(config=None, override=None):
     from . import _lib
     name = override or getattr(config, "precision", None) or os.environ.get("NRMS_B200_PRECISION", "tf32")

@@ -10,7 +10,7 @@ OUT = os.path.join(PKG, "libnrms_b200.so")
 OBJ = os.path.join(HERE, "_obj")
 SOURCES = ["encoder.cu", "misc.cu", "pack.cu", "tc_gemm.cu", "fused_host.cu", "tc_fused3.cu", "tc_fused7.cu", "k1g_table_attn.cu",
            "k1f_attn_pool.cu", "exp1.cu", "recommend.cu", "attn_mma.cu", "topk.cu",
-           "attn_cross.cu", "cnn_text.cu"]
+           "attn_cross.cu", "cnn_text.cu", "gru.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

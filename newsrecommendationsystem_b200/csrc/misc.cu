@@ -65,40 +65,48 @@ score_bwd_kernel(const float* __restrict__ d_scores, const float* __restrict__ c
 }
 
 // ---- evaluate scoring on CSR impressions: warp per impression, 8 lanes per candidate --------
-// The user vector lives in registers (10 float4 per lane); each 8-lane group streams one
-// 1200-byte news-vector row with coalesced float4 loads and reduces with 3 shuffles.
+// Rows of DVEC float4 (300 wide: DVEC = 75; LSTUR's 900-wide vectors: 225).  Up to 80 float4 per row, the user vector
+// lives in registers (10 float4 per lane) and each 8-lane group streams one row with coalesced float4 loads and reduces
+// with 3 shuffles.  Wider rows are walked in chunks of 80 float4, the user chunk reloaded next to the row chunk.
+template <int DVEC>
 __global__ void __launch_bounds__(256)
 score_csr_kernel(const float* __restrict__ table, const int32_t* __restrict__ cand_rows,
                  const int64_t* __restrict__ offsets, const float* __restrict__ user_vec, int64_t n_imp,
                  float* __restrict__ scores) {
+  constexpr int NCH = (DVEC + 79) / 80;
   const int lane = threadIdx.x & 31;
   const int g = lane & 7, grp = lane >> 3;
   const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
   for (int64_t imp = warp; imp < n_imp; imp += nwarps) {
-    const float4* up = reinterpret_cast<const float4*>(user_vec + imp * D);
+    const float4* up = reinterpret_cast<const float4*>(user_vec + imp * 4 * DVEC);
     float4 u[10];
+    if (NCH == 1) {
 #pragma unroll
-    for (int k = 0; k < 10; ++k) {
-      const int idx = g + 8 * k;
-      u[k] = (idx < DV4) ? __ldg(up + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int k = 0; k < 10; ++k) {
+        const int idx = g + 8 * k;
+        u[k] = (idx < DVEC) ? __ldg(up + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
     }
     const int64_t beg = offsets[imp], end = offsets[imp + 1];
     for (int64_t c0 = beg; c0 < end; c0 += 4) {
       const int64_t c = c0 + grp;
       float acc = 0.f;
       if (c < end) {
-        const float4* rp = reinterpret_cast<const float4*>(table + (int64_t)cand_rows[c] * D);
-        float4 v[10];
+        const float4* rp = reinterpret_cast<const float4*>(table + (int64_t)cand_rows[c] * 4 * DVEC);
+        for (int ch = 0; ch < NCH; ++ch) {
+          float4 v[10];
 #pragma unroll
-        for (int k = 0; k < 10; ++k) {
-          const int idx = g + 8 * k;
-          v[k] = (idx < DV4) ? __ldg(rp + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
+          for (int k = 0; k < 10; ++k) {
+            const int idx = ch * 80 + g + 8 * k;
+            v[k] = (idx < DVEC) ? __ldg(rp + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
+            if (NCH > 1) u[k] = (idx < DVEC) ? __ldg(up + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
+          }
 #pragma unroll
-        for (int k = 0; k < 10; ++k) {
-          acc = fmaf(v[k].x, u[k].x, acc); acc = fmaf(v[k].y, u[k].y, acc);
-          acc = fmaf(v[k].z, u[k].z, acc); acc = fmaf(v[k].w, u[k].w, acc);
+          for (int k = 0; k < 10; ++k) {
+            acc = fmaf(v[k].x, u[k].x, acc); acc = fmaf(v[k].y, u[k].y, acc);
+            acc = fmaf(v[k].z, u[k].z, acc); acc = fmaf(v[k].w, u[k].w, acc);
+          }
         }
       }
       acc += __shfl_xor_sync(0xffffffffu, acc, 4);
@@ -378,18 +386,27 @@ int nrms_score_bwd(const float* d_scores, const float* cand, const float* user, 
   return NRMS_OK;
 }
 
-int nrms_score_csr(const float* table, const int32_t* cand_rows, const int64_t* offsets, const float* user_vec,
-                   int64_t n_impressions, float* scores, void* stream) {
+int nrms_score_csr_width(const float* table, const int32_t* cand_rows, const int64_t* offsets, const float* user_vec,
+                         int64_t n_impressions, int width, float* scores, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  NRMS_CHECK_ARG(width == D || width == 3 * D, NRMS_E_UNSUPPORTED, "score width %d unsupported (300 or 900)", width);
   NRMS_CHECK_ARG(n_impressions >= 0, NRMS_E_INVALID, "bad sizes");
   if (n_impressions == 0) return NRMS_OK;
   NRMS_CHECK_ARG(table && cand_rows && offsets && user_vec && scores && aligned16(table) && aligned16(user_vec),
                  NRMS_E_INVALID, "null/misaligned pointer");
   int64_t gb = (n_impressions + 7) / 8;
   if (gb > (int64_t)num_sms() * 8) gb = (int64_t)num_sms() * 8;
-  score_csr_kernel<<<(unsigned)gb, 256, 0, st>>>(table, cand_rows, offsets, user_vec, n_impressions, scores);
+  if (width == D)
+    score_csr_kernel<DV4><<<(unsigned)gb, 256, 0, st>>>(table, cand_rows, offsets, user_vec, n_impressions, scores);
+  else
+    score_csr_kernel<3 * DV4><<<(unsigned)gb, 256, 0, st>>>(table, cand_rows, offsets, user_vec, n_impressions, scores);
   NRMS_LAUNCH_CHECK("score_csr");
   return NRMS_OK;
+}
+
+int nrms_score_csr(const float* table, const int32_t* cand_rows, const int64_t* offsets, const float* user_vec,
+                   int64_t n_impressions, float* scores, void* stream) {
+  return nrms_score_csr_width(table, cand_rows, offsets, user_vec, n_impressions, D, scores, stream);
 }
 
 int nrms_pack_rows_f16(const float* src, int64_t n_rows, void* dst16, void* stream) {

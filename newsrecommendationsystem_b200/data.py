@@ -21,6 +21,7 @@ from __future__ import annotations
 
 import csv
 import json
+import os
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -82,13 +83,15 @@ class TrainRows:
     hist_rows: np.ndarray              # int64 [B, num_clicked]
     clicked: np.ndarray                # int8  [B, 1+K]  (the 0/1 labels of the candidates; NRMS trains with label 0)
     users: list
+    user: np.ndarray = None            # int64 [B], the integer `user` column (LSTUR's user-embedding row)
+    clicked_news_length: np.ndarray = None   # int64 [B], len(first num_clicked clicks) (LSTUR's GRU length)
 
 
 def load_behaviors_parsed(path, news: NewsTable, num_clicked=50) -> TrainRows:
     """`behaviors_parsed.tsv` -> index-only training samples (what `BaseDataset.__getitem__` builds per sample,
     dataset.py:62-85): candidate rows, the FIRST `num_clicked` clicked rows left-padded with the pad row (index N)."""
     pad = len(news)
-    cand, hist, clicked, users = [], [], [], []
+    cand, hist, clicked, users, lengths = [], [], [], [], []
     with open(path, newline="") as f:
         reader = csv.DictReader(f, delimiter="\t", quoting=csv.QUOTE_NONE)
         for row in reader:
@@ -98,12 +101,14 @@ def load_behaviors_parsed(path, news: NewsTable, num_clicked=50) -> TrainRows:
             hist.append([pad] * (num_clicked - len(h)) + h)
             clicked.append([int(x) for x in row["clicked"].split()])
             users.append(row["user"])
+            lengths.append(len(h))
     width = {len(c) for c in cand}
     if len(width) > 1:
         raise ValueError(f"{path}: samples with different numbers of candidates {sorted(width)}")
     return TrainRows(np.asarray(cand, dtype=np.int64).reshape(len(cand), -1),
                      np.asarray(hist, dtype=np.int64).reshape(len(hist), num_clicked),
-                     np.asarray(clicked, dtype=np.int8).reshape(len(clicked), -1), users)
+                     np.asarray(clicked, dtype=np.int8).reshape(len(clicked), -1), users,
+                     np.asarray([int(u) for u in users], dtype=np.int64), np.asarray(lengths, dtype=np.int64))
 
 
 @dataclass
@@ -114,17 +119,18 @@ class EvalRows:
     labels: np.ndarray                 # int8  [sum C]
     impression_ids: list
     clicked_news_strings: list         # the reference's user key (evaluate.py:218,256)
+    users: list = None                 # the raw `user` column (LSTUR maps it through user2int.tsv)
 
 
 def load_behaviors(path, news: NewsTable, num_clicked=50, max_count=None) -> EvalRows:
     """Raw `behaviors.tsv` -> the impression tables of `evaluate.EvalHost` (evaluate.py:111-124, 127-157, 245-265).
     `max_count`: the reference stops BEFORE the max_count-th impression (`count == max_count: break`, :247-249)."""
-    hist, offs, rows, labels, imp_ids, keys = [], [0], [], [], [], []
+    hist, offs, rows, labels, imp_ids, keys, users = [], [0], [], [], [], [], []
     with open(path, newline="") as f:
         for n, rec in enumerate(csv.reader(f, delimiter="\t", quoting=csv.QUOTE_NONE), 1):
             if max_count is not None and n == max_count:
                 break
-            impression_id, _user, _time, clicked_news, impressions = rec[:5]
+            impression_id, user, _time, clicked_news, impressions = rec[:5]
             clicked_news = clicked_news if clicked_news else " "          # fillna(' ') of the reference
             h = [news.row_of[x] for x in clicked_news.split()[:num_clicked]]
             hist.append([-1] * (num_clicked - len(h)) + h)
@@ -135,5 +141,18 @@ def load_behaviors(path, news: NewsTable, num_clicked=50, max_count=None) -> Eva
             offs.append(len(rows))
             imp_ids.append(impression_id)
             keys.append(clicked_news)
+            users.append(user)
     return EvalRows(np.asarray(hist, dtype=np.int64).reshape(len(hist), num_clicked), np.asarray(offs, dtype=np.int64),
-                    np.asarray(rows, dtype=np.int64), np.asarray(labels, dtype=np.int8), imp_ids, keys)
+                    np.asarray(rows, dtype=np.int64), np.asarray(labels, dtype=np.int8), imp_ids, keys, users)
+
+
+def load_user2int(path) -> dict:
+    """`user2int.tsv` (header `user\tint`, written by the reference's preprocessing) -> {user string: integer id}.  A
+    missing file raises FileNotFoundError naming the path."""
+    if not os.path.exists(path):
+        raise FileNotFoundError(f"user2int file not found: {path}")
+    out = {}
+    with open(path, newline="") as f:
+        for row in csv.DictReader(f, delimiter="\t", quoting=csv.QUOTE_NONE):
+            out[row["user"]] = int(row["int"])
+    return out

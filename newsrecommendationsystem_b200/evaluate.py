@@ -363,16 +363,22 @@ def evaluate_tensors(model, inputs: EvalInputs, max_count=None, return_details=F
     return means
 
 
-def evaluate(model, directory, num_workers=0, max_count=None):
+def evaluate(model, directory, num_workers=0, max_count=None, user2int_path=None):
     """The reference's entry point (src/evaluate.py:171-272), same signature and return value: evaluate `model` on
     `directory` (which holds `behaviors.tsv` and `news_parsed.tsv`) -> (AUC, MRR, nDCG@5, nDCG@10).  The files are read once
     into integer tables (`data.py`); everything after that is the device-resident pipeline above.  `num_workers` (the
     reference's metric process pool) is accepted and unused: the metrics run on the GPU.  `max_count` as in the reference
-    (`sys.maxsize` or None = all impressions)."""
+    (`sys.maxsize` or None = all impressions).  `user2int_path` (LSTUR models only): the reference's
+    `data/train/user2int.tsv`, by default `<directory>/../train/user2int.tsv`."""
     import os
     import sys
     from . import data
     from .model.NAML import NAML
+    from .model.LSTUR import LSTUR
+    if isinstance(model, LSTUR):
+        if user2int_path is None:
+            user2int_path = os.path.join(directory, "..", "train", "user2int.tsv")
+        return _evaluate_lstur(model, directory, user2int_path, max_count)
     if isinstance(model, NAML):
         return _evaluate_columns(model, directory, max_count)
     news = data.load_news_parsed(os.path.join(directory, "news_parsed.tsv"))
@@ -443,3 +449,87 @@ def evaluate_columns(model, cols, host, max_count=None):
     with np.errstate(all="ignore"):
         return tuple(float(x) for x in (s[:4] / s[4:]))
 
+
+
+def lstur_user_keys(ev, user2int, num_clicked=50):
+    """The reference's LSTUR user walk (evaluate.py's UserDataset + user2vector): one user vector per distinct
+    clicked-news string, computed from the FIRST row of the file with that string (first wins; so users with the same
+    history share a vector, and every empty history ' ' shares one).  -> (key_of_impression int64 [I], first_row
+    int64 [U] (row of `ev` each key is taken from), user ids int64 [U] (user2int, 0 if missing), lengths int64 [U]
+    (len of the first num_clicked clicks; the user encoder reads 0 as 1))."""
+    key_index, key_of, first_rows = {}, np.empty(len(ev.clicked_news_strings), dtype=np.int64), []
+    for i, k in enumerate(ev.clicked_news_strings):
+        if k not in key_index:
+            key_index[k] = len(first_rows)
+            first_rows.append(i)
+        key_of[i] = key_index[k]
+    rows = np.asarray(first_rows, dtype=np.int64)
+    users = np.asarray([user2int.get(ev.users[i], 0) for i in rows], dtype=np.int64)
+    lengths = np.asarray([min(len(ev.clicked_news_strings[i].split()), num_clicked) for i in rows], dtype=np.int64)
+    return key_of, rows, users, lengths
+
+
+@torch.no_grad()
+def _evaluate_lstur(model, directory, user2int_path, max_count=None):
+    """evaluate() for LSTUR: the 900-wide news table (PADDED_NEWS = a zero row) from get_news_vector, one user vector per
+    distinct clicked-news string from the table-projected GRU (`user_encoder.forward_indexed`: the GRU's input projection
+    runs once over the news table), scoring at width 900 and the device metrics."""
+    import os
+    import sys
+    from . import data
+    user2int = data.load_user2int(user2int_path)
+    attrs = list(model.config.dataset_attributes["news"])
+    news = data.load_news_parsed(os.path.join(directory, "news_parsed.tsv"), attributes=attrs)
+    num_clicked = int(model.config.num_clicked_news_a_user)
+    ev = data.load_behaviors(os.path.join(directory, "behaviors.tsv"), news, num_clicked=num_clicked)
+    n_imp = len(ev.impression_ids)
+    if max_count is not None and max_count < sys.maxsize:
+        n_imp = max(0, min(n_imp, int(max_count) - 1))
+    if n_imp == 0:
+        return tuple(float("nan") for _ in range(4))
+    dev = next(model.parameters()).device
+    cols = {a: torch.as_tensor(news.columns[a]).to(dev) for a in attrs}
+    c1 = int(ev.cand_offsets[n_imp])
+    user_vec = lstur_user_vectors(model, cols, ev, user2int, n_imp)
+    table = user_vec.table
+    cand_rows = torch.as_tensor(ev.cand_rows[:c1], dtype=torch.int32).to(dev)
+    labels = torch.as_tensor(ev.labels[:c1]).to(dev)
+    offs = torch.as_tensor(ev.cand_offsets[:n_imp + 1]).to(dev)
+    scores = ops.score_csr(table, cand_rows, offs, user_vec.per_impression)
+    _, sums = ops.rank_metrics(scores, labels, offs)
+    s = sums.cpu().numpy()
+    with np.errstate(all="ignore"):
+        return tuple(float(x) for x in (s[:4] / s[4:]))
+
+
+class LsturUserVectors:
+    def __init__(self, table, per_key, per_impression, key_of, users, lengths):
+        self.table, self.per_key, self.per_impression = table, per_key, per_impression
+        self.key_of, self.users, self.lengths = key_of, users, lengths
+
+
+@torch.no_grad()
+def lstur_user_vectors(model, cols, ev, user2int, n_imp=None):
+    """The device part of LSTUR's evaluate up to scoring: cols {attribute: device column with one row per news}, ev the
+    EvalRows of the impressions -> LsturUserVectors (table [N + 1, 900] with the zero PADDED_NEWS row N, the vectors of the
+    distinct histories and of the first n_imp impressions)."""
+    n_imp = len(ev.impression_ids) if n_imp is None else n_imp
+    dev = next(model.parameters()).device
+    n = len(next(iter(cols.values())))
+    was_training = model.training
+    model.eval()
+    try:
+        table = torch.zeros((n + 1, 3 * ops.D), dtype=torch.float32, device=dev)
+        if n:
+            table[:n] = model.get_news_vector(cols)
+        key_of, rows, users, lengths = lstur_user_keys(ev, user2int, int(model.config.num_clicked_news_a_user))
+        key_of = key_of[:n_imp]
+        hist = ev.hist_rows[rows]
+        hist = np.where(hist < 0, n, hist)
+        user_rows = model._user(torch.from_numpy(users), False)
+        per_key = model.user_encoder.forward_indexed(user_rows, torch.from_numpy(lengths), table,
+                                                     torch.from_numpy(hist))
+    finally:
+        model.train(was_training)
+    per_imp = ops.embedding_rows(torch.from_numpy(key_of).to(dev), per_key, padding_idx=None)
+    return LsturUserVectors(table, per_key, per_imp, key_of, users, lengths)

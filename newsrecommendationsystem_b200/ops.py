@@ -386,12 +386,17 @@ def cross_entropy_label0(logits):
 
 @torch.no_grad()
 def score_csr(table, cand_rows, offsets, user_vec):
+    """Dot products of each impression's candidate rows of `table` with its user vector; rows 300 or 900 wide."""
     lib = _lib.load()
     _require_cuda(table, cand_rows, offsets, user_vec)
     n_imp = offsets.numel() - 1
     scores = torch.empty((cand_rows.numel(),), dtype=torch.float32, device=table.device)
-    check(lib.nrms_score_csr(ptr(table), ptr(cand_rows), ptr(offsets), ptr(user_vec), n_imp, ptr(scores),
-                             stream_ptr(table.device)), "nrms_score_csr")
+    if table.shape[-1] == D:
+        check(lib.nrms_score_csr(ptr(table), ptr(cand_rows), ptr(offsets), ptr(user_vec), n_imp, ptr(scores),
+                                 stream_ptr(table.device)), "nrms_score_csr")
+    else:
+        check(lib.nrms_score_csr_width(ptr(table), ptr(cand_rows), ptr(offsets), ptr(user_vec), n_imp,
+                                       table.shape[-1], ptr(scores), stream_ptr(table.device)), "nrms_score_csr_width")
     return scores
 
 
@@ -948,3 +953,196 @@ def additive_forward(c, wa, ba, qa, mode=_lib.MODE_TF32):
     check(lib.nrms_additive_fwd(ptr(c_c), n, S, ptr(wa_c), ptr(ba_c), ptr(qa_c), ptr(out), ptr(ws), ws.numel(), mode,
                                 stream_ptr(c.device)), "nrms_additive_fwd")
     return out
+
+
+GRU_SHAPES = ((900, 900), (900, 450))
+
+
+def _host_lengths(lengths, n_seq, T):
+    """int32 host copy of the per-sequence lengths (nrms_gru_* take them in host memory), checked against 0..T."""
+    if lengths.is_cuda:
+        raise RuntimeError("gru lengths must be a host tensor: the steps are scheduled on the host")
+    lh = lengths.detach().reshape(-1).to(torch.int32).contiguous()
+    if lh.numel() != n_seq:
+        raise RuntimeError(f"gru takes one length per sequence: {lh.numel()} for {n_seq}")
+    if lh.numel() and (int(lh.min()) < 0 or int(lh.max()) > T):
+        raise RuntimeError(f"gru lengths must lie in 0..{T}, got [{int(lh.min())}, {int(lh.max())}]")
+    return lh
+
+
+class _GRUFn(torch.autograd.Function):
+    """The last hidden state of nn.GRU over pack_padded_sequence(x, lengths, batch_first=True) from h0 (reference
+    src/model/LSTUR/user_encoder.py) -- nrms_gru_fwd / _bwd."""
+
+    @staticmethod
+    def forward(ctx, x, lengths, h0, w_ih, w_hh, b_ih, b_hh, mode, track_grad):
+        lib = _lib.load()
+        _require_cuda(x, h0, w_ih, w_hh, b_ih, b_hh)
+        n_seq, T, I = x.shape
+        Hd = w_hh.shape[1]
+        lh = _host_lengths(lengths, n_seq, T)
+        dev = x.device
+        x_c, w_ih_c, w_hh_c, b_ih_c, b_hh_c = map(_f32c, (x, w_ih, w_hh, b_ih, b_hh))
+        h0_c = None if h0 is None else _f32c(h0)
+        out = torch.empty((n_seq, Hd), dtype=torch.float32, device=dev)
+        needs_grad = track_grad and any(ctx.needs_input_grad)
+        stash = _bytes(lib.nrms_gru_stash_bytes(n_seq, T, I, Hd), dev) if needs_grad else None
+        ws = _bytes(lib.nrms_gru_fwd_workspace_bytes(n_seq, T, n_seq * T, I, Hd), dev)
+        check(lib.nrms_gru_fwd(ptr(x_c), n_seq * T, None, n_seq, T, I, Hd, C.c_void_p(lh.data_ptr()), ptr(h0_c),
+                               ptr(w_ih_c), ptr(w_hh_c), ptr(b_ih_c), ptr(b_hh_c), ptr(out), ptr(stash), ptr(ws),
+                               ws.numel(), mode, stream_ptr(dev)), "nrms_gru_fwd")
+        if needs_grad:
+            ctx.save_for_backward(x_c, w_ih_c, w_hh_c, stash)
+            ctx.lengths = lh
+            ctx.meta = (n_seq, T, I, Hd, mode, h0 is not None)
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        lib = _lib.load()
+        n_seq, T, I, Hd, mode, has_h0 = ctx.meta
+        x, w_ih, w_hh, stash = ctx.saved_tensors
+        dev = d_out.device
+        d_out = d_out.contiguous().float()
+        d_x = torch.empty((n_seq, T, I), dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        d_h0 = torch.empty((n_seq, Hd), dtype=torch.float32, device=dev) if has_h0 and ctx.needs_input_grad[2] else None
+        d_w_ih = torch.zeros((3 * Hd, I), dtype=torch.float32, device=dev)
+        d_w_hh = torch.zeros((3 * Hd, Hd), dtype=torch.float32, device=dev)
+        d_b_ih = torch.zeros((3 * Hd,), dtype=torch.float32, device=dev)
+        d_b_hh = torch.zeros((3 * Hd,), dtype=torch.float32, device=dev)
+        ws = _bytes(lib.nrms_gru_bwd_workspace_bytes(n_seq, T, I, Hd, mode), dev)
+        check(lib.nrms_gru_bwd(ptr(d_out), ptr(x), n_seq, T, I, Hd, C.c_void_p(ctx.lengths.data_ptr()), ptr(w_ih),
+                               ptr(w_hh), ptr(stash), ptr(d_x), ptr(d_h0), ptr(d_w_ih), ptr(d_w_hh), ptr(d_b_ih),
+                               ptr(d_b_hh), ptr(ws), ws.numel(), mode, stream_ptr(dev)), "nrms_gru_bwd")
+        return d_x, None, d_h0, d_w_ih, d_w_hh, d_b_ih, d_b_hh, None, None
+
+
+def _gru_check(I, w_ih, w_hh):
+    Hd = w_hh.shape[-1]
+    if (I, Hd) not in GRU_SHAPES or tuple(w_ih.shape) != (3 * Hd, I) or tuple(w_hh.shape) != (3 * Hd, Hd):
+        raise RuntimeError(f"gru is compiled for (input, hidden) in {GRU_SHAPES}, got w_ih {tuple(w_ih.shape)}, "
+                           f"w_hh {tuple(w_hh.shape)}")
+
+
+def gru(x, lengths, h0, w_ih, w_hh, b_ih, b_hh, mode=_lib.MODE_TF32):
+    """Last hidden state of a one-layer nn.GRU (weight_ih_l0 = w_ih [3H, I], ...) over steps t < lengths[s] of
+    x [n_seq, T, I], started from h0 [n_seq, H] (None: zeros), autograd-connected.  lengths: integer [n_seq] on the
+    HOST, each in 0..T (0 runs no step).  (I, H) = (900, 900) or (900, 450)."""
+    if x.dim() != 3:
+        raise RuntimeError(f"gru takes x [n_seq, T, I], got {tuple(x.shape)}")
+    _gru_check(x.shape[2], w_ih, w_hh)
+    return _GRUFn.apply(x, lengths, h0, w_ih, w_hh, b_ih, b_hh, mode, torch.is_grad_enabled())
+
+
+@torch.no_grad()
+def gru_indexed(table, rows, lengths, h0, w_ih, w_hh, b_ih, b_hh, mode=_lib.MODE_TF32):
+    """Inference form of gru: step t of sequence s reads row rows[s, t] of the table [n_rows, I] (device).  The input
+    projection runs once over the table rows, not once per history row.  rows on the host are range-checked against
+    the table before they go to the device; rows already on the device must lie in [0, n_rows)."""
+    if not rows.is_cuda:
+        if rows.numel() and (int(rows.min()) < 0 or int(rows.max()) >= table.shape[0]):
+            raise IndexError(f"gru_indexed rows must lie in [0, {table.shape[0]}), got [{int(rows.min())}, "
+                             f"{int(rows.max())}]")
+        rows = rows.to(table.device)
+    _require_cuda(table, rows, h0, w_ih, w_hh, b_ih, b_hh)
+    lib = _lib.load()
+    n_seq, T = rows.shape
+    I = table.shape[1]
+    _gru_check(I, w_ih, w_hh)
+    Hd = w_hh.shape[1]
+    if rows.numel() and table.shape[0] == 0:
+        raise RuntimeError("gru_indexed: empty table")
+    lh = _host_lengths(lengths, n_seq, T)
+    dev = table.device
+    tab, w_ih_c, w_hh_c, b_ih_c, b_hh_c = map(_f32c, (table, w_ih, w_hh, b_ih, b_hh))
+    h0_c = None if h0 is None else _f32c(h0)
+    r = rows.contiguous().long().view(-1)
+    out = torch.empty((n_seq, Hd), dtype=torch.float32, device=dev)
+    ws = _bytes(lib.nrms_gru_fwd_workspace_bytes(n_seq, T, tab.shape[0], I, Hd), dev)
+    check(lib.nrms_gru_fwd(ptr(tab), tab.shape[0], ptr(r), n_seq, T, I, Hd, C.c_void_p(lh.data_ptr()), ptr(h0_c),
+                           ptr(w_ih_c), ptr(w_hh_c), ptr(b_ih_c), ptr(b_hh_c), ptr(out), None, ptr(ws), ws.numel(),
+                           mode, stream_ptr(dev)), "nrms_gru_fwd")
+    return out
+
+
+class _RowsFn(torch.autograd.Function):
+    """weight[idx] (nn.Embedding / F.embedding), optionally under a whole-row dropout mask -- F.dropout2d of
+    embedding(idx).unsqueeze(0) zeroes whole rows (reference src/model/LSTUR/__init__.py) -- nrms_rows_fwd / _bwd."""
+
+    @staticmethod
+    def forward(ctx, idx, weight, padding_idx, p, seed, offset):
+        lib = _lib.load()
+        _require_cuda(idx, weight)
+        i = idx.contiguous().long().view(-1)
+        w = _f32c(weight)
+        n, width = i.numel(), w.shape[1]
+        out = torch.empty((n, width), dtype=torch.float32, device=w.device)
+        check(lib.nrms_rows_fwd(ptr(w), w.shape[0], width, ptr(i), n, width, ptr(out), width, float(p), int(seed),
+                                int(offset), stream_ptr(w.device)), "nrms_rows_fwd")
+        ctx.save_for_backward(i)
+        ctx.meta = (tuple(w.shape), padding_idx, float(p), int(seed), int(offset))
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        lib = _lib.load()
+        (i,) = ctx.saved_tensors
+        shape, padding_idx, p, seed, offset = ctx.meta
+        d_out = d_out.contiguous().float()
+        d_w = torch.zeros(shape, dtype=torch.float32, device=d_out.device)
+        check(lib.nrms_rows_bwd(ptr(d_out), shape[1], ptr(i), i.numel(), shape[1], ptr(d_w), shape[1],
+                                -1 if padding_idx is None else int(padding_idx), p, seed, offset,
+                                stream_ptr(d_out.device)), "nrms_rows_bwd")
+        return None, d_w, None, None, None, None
+
+
+def embedding_rows(idx, weight, padding_idx=0, dropout_p=0.0, seed=0, offset=0):
+    """weight[idx] -> fp32 [idx.numel(), width], autograd-connected (padding_idx rows get no gradient).  dropout_p > 0:
+    each output row is zeroed with probability p and the others scaled by 1 / (1 - p), from the Philox stream of the
+    (seed, offset) pair (row i: counter i + offset)."""
+    return _RowsFn.apply(idx, weight, padding_idx, dropout_p, seed, offset)
+
+
+def _copy_rows(src, ld_src, dst, ld_dst, n, width, lib, dev):
+    check(lib.nrms_rows_fwd(ptr(src), n, ld_src, None, n, width, ptr(dst), ld_dst, 0.0, 0, 0, stream_ptr(dev)),
+          "nrms_rows_fwd")
+
+
+class _ConcatRowsFn(torch.autograd.Function):
+    """torch.cat(parts, dim=1) of 2-D fp32 row blocks through strided row copies (nrms_rows_fwd with no index)."""
+
+    @staticmethod
+    def forward(ctx, *parts):
+        lib = _lib.load()
+        _require_cuda(*parts)
+        n = parts[0].shape[0]
+        widths = [p.shape[1] for p in parts]
+        dev = parts[0].device
+        out = torch.empty((n, sum(widths)), dtype=torch.float32, device=dev)
+        col = 0
+        for p, w in zip(parts, widths):
+            pc = _f32c(p)
+            _copy_rows(pc, w, out[:, col:], out.shape[1], n, w, lib, dev)
+            col += w
+        ctx.widths = widths
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        lib = _lib.load()
+        d_out = d_out.contiguous().float()
+        n, dev = d_out.shape[0], d_out.device
+        grads, col = [], 0
+        for w in ctx.widths:
+            g = torch.empty((n, w), dtype=torch.float32, device=dev)
+            _copy_rows(d_out[:, col:], d_out.shape[1], g, w, n, w, lib, dev)
+            grads.append(g)
+            col += w
+        return tuple(grads)
+
+
+def concat_rows(*parts):
+    """torch.cat(parts, dim=1) of [n, w_k] row blocks, autograd-connected, with the copies in libnrms_b200."""
+    if len({p.shape[0] for p in parts}) != 1 or any(p.dim() != 2 for p in parts):
+        raise RuntimeError(f"concat_rows takes [n, w] blocks of one n, got {[tuple(p.shape) for p in parts]}")
+    return _ConcatRowsFn.apply(*parts)

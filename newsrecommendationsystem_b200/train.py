@@ -40,12 +40,13 @@ class TrainStep:
         self.steps += 1
         return loss.detach()
 
-    def step_rows(self, token_table, cand_rows, hist_rows):
+    def step_rows(self, token_table, cand_rows, hist_rows, user=None, clicked_news_length=None):
         """Index-only minibatch (SURVEY 8 f2): `token_table` is the pre-tokenised news table int64 [N_news, L]
         resident on the GPU, `cand_rows` [B, 1+K] and `hist_rows` [B, N] are news-row indices -- 55 x B x 8 bytes of
         H2D per step instead of the 55 token tensors the reference DataLoader ships (dataset.py:17-85,
         train.py:118-124).  The token rows are read through the indices inside the embedding gather / gradient scatter
-        kernels (nrms_news_encoder_rows_fwd/bwd): no gathered token tensor is materialised."""
+        kernels (nrms_news_encoder_rows_fwd/bwd): no gathered token tensor is materialised.  user / clicked_news_length:
+        the minibatch's `user` and `clicked_news_length` columns, passed on to a model that reads them (LSTUR)."""
         if self.cosine_total_steps:
             self.optimizer.param_groups[0]["lr"] = cosine_lr(self.base_lr, self.steps, self.cosine_total_steps)
         # a model with several news attributes (Exp1) takes a dict of device columns with one row per news
@@ -55,7 +56,10 @@ class TrainStep:
             hi = max(int(cand_rows.max()), int(hist_rows.max()))
             if lo < 0 or hi >= n_rows:
                 raise IndexError(f"news rows must lie in [0, {n_rows}), got [{lo}, {hi}]")
-        logits = self.model.forward_rows(token_table, cand_rows, hist_rows)
+        if user is not None or clicked_news_length is not None:
+            logits = self.model.forward_rows(token_table, cand_rows, hist_rows, user, clicked_news_length)
+        else:
+            logits = self.model.forward_rows(token_table, cand_rows, hist_rows)
         loss = ops.cross_entropy_label0(logits)
         self.optimizer.zero_grad()
         loss.backward()
@@ -64,13 +68,18 @@ class TrainStep:
         self.steps += 1
         return loss.detach()
 
-    def step(self, candidate_news, clicked_news):
+    def step(self, candidate_news, clicked_news, user=None, clicked_news_length=None):
         """Reference minibatch format: lists of {"title": LongTensor[B, L]} (src/train.py:202-203), or of every
-        attribute the model reads ({"title", "abstract", "category", ...}) for a model without forward_tokens (Exp1)."""
+        attribute the model reads ({"title", "abstract", "category", ...}) for a model without forward_tokens (Exp1).
+        user / clicked_news_length: the minibatch's columns of those names, for LSTUR, which the reference calls as
+        model(minibatch["user"], minibatch["clicked_news_length"], candidate_news, clicked_news)."""
         if not hasattr(self.model, "forward_tokens"):
             if self.cosine_total_steps:
                 self.optimizer.param_groups[0]["lr"] = cosine_lr(self.base_lr, self.steps, self.cosine_total_steps)
-            logits = self.model(candidate_news, clicked_news)
+            if user is not None or clicked_news_length is not None:
+                logits = self.model(user, clicked_news_length, candidate_news, clicked_news)
+            else:
+                logits = self.model(candidate_news, clicked_news)
             loss = ops.cross_entropy_label0(logits)
             self.optimizer.zero_grad()
             loss.backward()
